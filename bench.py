@@ -9,7 +9,11 @@ metric through the C ABI with HOST buffers: upload (H2D) + score + consensus set
 least-squares refine inside the timed region.  Multi-GPU: points replicated, hypotheses
 partitioned (weak scaling: H per GPU fixed), one all-reduce(MAX) on the packed (count,index) key.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy (float64), so that two builds
+can be compared output for output: inputs and step seeds depend only on the arguments (with --impl reference the sample is
+--cpu-sample-hyps hypotheses, else DUMP_CPU_SAMPLE_HYPS instead of one sized from a timed probe).
 """
 import argparse
 import json
@@ -63,7 +67,27 @@ def parse():
     ap.add_argument("--no-configs", action="store_true", help="skip the secondary configurations (BASELINE.json configs[2..4], per-model scoring table)")
     ap.add_argument("--comm", default="native", choices=["native", "hooks"],
                     help="N > 1: collectives issued by the library itself (ncclAllReduce / ncclAllGather, lsqr_ctx_init_nccl) or torch.distributed hooks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64, rank 0)")
     return ap.parse_args()
+
+
+DUMP_MAX_BYTES = 64 << 20         # all arrays of one dump together
+DUMP_CPU_SAMPLE_HYPS = 1024       # reference arm with --dump-outputs and no --cpu-sample-hyps: a fixed sample, not a timed probe
+
+
+def dump_outputs(out_dir, arrays):
+    """One float64 .npy per output of the last timed step, DUMP_MAX_BYTES in all: an array longer than its share is replaced
+    by a fixed, seeded sample of its entries, stored with the sampled indices as <name>_index."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_MAX_BYTES // 8 // (2 * len(arrays))      # values per array, room left for its index
+    for name, a in arrays.items():
+        a = np.atleast_1d(np.asarray(a, dtype=np.float64))
+        if a.size > cap:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))
+            a = a.reshape(-1)[idx]
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -164,7 +188,7 @@ def cpu_reference_run(model, data, delta, n_hyps, threads=0):
     counts, _ = orc.score_subsets(m, delta, data, subs, nthreads=threads, want_params=False)
     dt = time.perf_counter() - t0
     return {"kind": "reference" if kind == "ref" else "port", "cores": threads,
-            "seconds": dt, "evals": float(n_hyps) * data.shape[0], "best": int(counts.max())}
+            "seconds": dt, "evals": float(n_hyps) * data.shape[0], "best": int(counts.max()), "counts": counts}
 
 
 def cpu_sample_size(model, data, delta, target_s, threads):
@@ -238,7 +262,12 @@ def run_reference_arm(args):
     cores = host_cores()
     # each step is a bounded sample of the workload; the whole run (warm-up + steps + compute()) stays under ~2 minutes
     target_s = min(5.0, max(0.5, 60.0 / max(args.steps + args.warmup / 4.0, 1.0)))
-    n_hyps = args.cpu_sample_hyps or cpu_sample_size(args.model, data, delta, target_s, cores)
+    if args.cpu_sample_hyps:
+        n_hyps = args.cpu_sample_hyps
+    elif args.dump_outputs:     # the dumped counts must not depend on this host's speed
+        n_hyps = DUMP_CPU_SAMPLE_HYPS
+    else:
+        n_hyps = cpu_sample_size(args.model, data, delta, target_s, cores)
     for _ in range(args.warmup):
         cpu_reference_run(args.model, data, delta, max(n_hyps // 4, cores), cores)
     times, info = [], None
@@ -247,6 +276,8 @@ def run_reference_arm(args):
         info = cpu_reference_run(args.model, data, delta, n_hyps, cores)
         times.append(info["seconds"])
     total = time.perf_counter() - t_all
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"counts": info["counts"], "best_count": info["best"]})
     value = info["evals"] * args.steps / sum(times)
     comp = None if args.no_e2e else reference_compute_ms(args.model, data, delta)
     comp_configs = None if (args.no_e2e or args.no_configs) else reference_compute_configs()
@@ -521,6 +552,8 @@ def main():
             cons_ms.append(r["consensus_ms"])
         ev1.record()
         barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {k: r[k] for k in ("best_index", "best_count", "n_valid", "best_subset", "best_params")})
     elapsed_ms = ev0.elapsed_time(ev1)
     launches = eng.kernel_launches - launches0
     t = torch.tensor([elapsed_ms], dtype=torch.float64, device="cuda")

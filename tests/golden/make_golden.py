@@ -11,6 +11,15 @@ the result of RANSAC<T,S>::compute (exhaustive overload) on a small problem, and
 leastSquaresEstimate() on the consensus set.  Plus the reference's file-based known-answer
 case (testing/Data/pivotCalibrationData.txt).  The fixtures travel to the GPU box; the
 reference does not.
+
+    python tests/golden/make_golden.py cases [ref|port]
+
+mints only reference_cases.npz: the inputs of the live comparisons in tests/test_oracle.py and what
+the reference returns for them, reduced as those tests read it without oracle/_ref (counts and
+rejection patterns in full, parameter matrices as a SHA-256 where compared bit-exact, else a fixed
+sample of rows).  `port` mints it from the C restatement instead, for where the reference's sources
+are not at hand: the restatement, as it stands, passed all of those comparisons against the
+reference live on exactly these inputs.  The file's `source` entry says which of the two it holds.
 """
 import os
 import sys
@@ -25,7 +34,37 @@ from oracle.pyoracle import INFO, MODELS, Oracle  # noqa: E402
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
+def mint_reference_cases(kind):
+    """tests/golden/reference_cases.npz from Oracle(kind), with the case definitions of tests/test_oracle.py."""
+    sys.path.insert(0, os.path.dirname(OUT))
+    import test_oracle as t
+    orc, fx = Oracle(kind), {}
+
+    def put(prefix, d):
+        fx.update({f"{prefix}.{k}": v for k, v in d.items()})
+    for name, m in MODELS.items():
+        put(f"live.{name}", t.reference_live(orc, name, m, keep=16))
+        put(f"degenerate.{name}", t.reference_degenerate(orc, name, m, keep=16))
+    for seed in range(4):
+        for name, m, data, delta, subs in t.seed_cases(seed):
+            put(f"seed{seed}.{name}", t.reference_seed_case(orc, name, m, data, delta, subs, keep=8))
+    data, w = t.horn_case()
+    put("horn", {"params": orc.weighted_absor(data, w)})
+    put("models", t.reference_model_table(orc))
+    # one byte blob with an index (name, dtype, shape, offset) instead of ~1300 small .npy members
+    names = sorted(fx)
+    arrs = [np.ascontiguousarray(fx[k]).reshape(np.shape(fx[k])) for k in names]
+    np.savez_compressed(os.path.join(OUT, "reference_cases.npz"), source=np.array("oracle/_ref" if kind == "ref" else "oracle/liboracle.so"),
+                        names=np.array(names), dtypes=np.array([a.dtype.str for a in arrs]),
+                        shapes=np.array([list(a.shape) + [-1] * (2 - a.ndim) for a in arrs]),
+                        offsets=np.cumsum([0] + [a.nbytes for a in arrs]),
+                        blob=np.concatenate([a.reshape(-1).view(np.uint8) for a in arrs]))
+
+
 def main():
+    if sys.argv[1:2] == ["cases"]:
+        mint_reference_cases(sys.argv[2] if len(sys.argv) > 2 else "ref")
+        return
     ref = Oracle("ref")
     only = sys.argv[1:]
     for name, m in MODELS.items():
@@ -104,6 +143,7 @@ def main():
                         known_exact=np.array([-18.586, 1.98134, -157.439, 146.965, -62.0497, -1042.87]),
                         known_ls=np.array([-17.7799, 1.1113, -156.865, 146.901, -62.9689, -1042.14]))
     print("pivot file: exact", exact, "ls", ls)
+    mint_reference_cases("ref")
 
 
 if __name__ == "__main__":

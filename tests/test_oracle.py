@@ -1,7 +1,10 @@
 """Pins the CPU oracle (oracle/lsqr_oracle.c, the plain-C restatement) before anything trusts it:
 against the reference's own golden values, against fixtures minted by the reference itself
-(tests/golden/make_golden.py), and -- when oracle/_ref is present -- against the reference live.
+(tests/golden/make_golden.py), and against the reference live -- or, without oracle/_ref, what it returned for the same inputs.
 No GPU involved."""
+import functools
+import hashlib
+
 import numpy as np
 import pytest
 
@@ -94,31 +97,88 @@ def test_config1_plane23(port):
         assert c[0] == g["all_counts"][r] and np.array_equal(p[0], g["all_params"][r])
 
 
-# ---- the reference live -----------------------------------------------------------------
+# ---- the reference live, or what it returned -------------------------------------------
+# With oracle/_ref present these tests compare the restatement with the reference on every row.  Without it they compare with
+# tests/golden/reference_cases.npz (tests/golden/make_golden.py): the same inputs, the reference's counts and rejection
+# pattern in full, its parameter vectors as a SHA-256 where the comparison is bit-exact and as a fixed sample of rows where it
+# has a tolerance.
+def _digest(p):
+    """SHA-256 of a parameter matrix as array_equal(nan_to_num(.)) sees it (NaN -> 0, -0.0 -> 0.0)."""
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(np.nan_to_num(p) + 0.0).tobytes()).digest(), dtype=np.uint8)
+
+
+def reduce_answer(counts, params, exact, rows=None, keep=None):
+    """What a comparison needs of the reference's answer.  rows: candidate rows for the value comparison (default all);
+    keep=None keeps every candidate (live), keep=K a fixed sample of K of them and, where exact, the digest instead (stored)."""
+    out = {"counts": counts.astype(np.uint32), "nan": np.isnan(params)}
+    if keep is not None and exact:
+        out["sha"] = _digest(params)
+        return out
+    idx = np.flatnonzero(np.ones(len(params), bool) if rows is None else rows)
+    if keep is not None and len(idx) > keep:
+        idx = np.sort(np.random.default_rng(0).choice(idx, keep, replace=False))
+    out["idx"], out["rows"] = idx, params[idx]
+    return out
+
+
+def assert_params(p1, want, tol):
+    if "sha" in want:
+        assert np.array_equal(_digest(p1), want["sha"])
+    elif tol is None:
+        assert np.array_equal(np.nan_to_num(p1[want["idx"]]), np.nan_to_num(want["rows"]))
+    else:
+        assert np.allclose(np.nan_to_num(p1[want["idx"]]), np.nan_to_num(want["rows"]), rtol=tol, atol=tol)
+
+
+def reference_answer(ref, prefix, live):
+    """live(ref) when oracle/_ref is present, else the stored entries <prefix>.*"""
+    if ref is not None:
+        return live(ref)
+    return {k[len(prefix) + 1:]: v for k, v in stored_cases().items() if k.startswith(prefix + ".")}
+
+
+@functools.lru_cache(maxsize=1)
+def stored_cases():
+    """tests/golden/reference_cases.npz unpacked: one byte blob, entry i at offsets[i]:offsets[i + 1] with dtypes[i], shapes[i]."""
+    g = golden("reference_cases")
+    blob, off = g["blob"], g["offsets"]
+    return {str(k): np.frombuffer(blob[off[i]:off[i + 1]].tobytes(), dtype=np.dtype(str(g["dtypes"][i]))).reshape([d for d in g["shapes"][i] if d >= 0])
+            for i, k in enumerate(g["names"])}
+
+
+def live_case(name, m):
+    n, k = 400, INFO[m][2]
+    data, _ = synth.GENERATORS[name](n, seed=4242 + m)
+    return data, synth.DELTAS[name], synth.random_subsets(n, k, 1500, seed=99 + m)
+
+
+def reference_live(orc, name, m, keep=None):
+    data, delta, subs = live_case(name, m)
+    c, p = orc.score_subsets(m, delta, data, subs)
+    return reduce_answer(c, p, pinv_tol(name) is None, keep=keep)
+
+
 @pytest.mark.parametrize("name,m", ALL)
 def test_port_matches_reference_live(port, ref, name, m):
-    D, P, k = INFO[m]
-    n = 400
-    data, _ = synth.GENERATORS[name](n, seed=4242 + m)
-    delta = synth.DELTAS[name]
-    subs = synth.random_subsets(n, k, 1500, seed=99 + m)
+    want = reference_answer(ref, f"live.{name}", lambda r: reference_live(r, name, m))
+    data, delta, subs = live_case(name, m)
     c1, p1 = port.score_subsets(m, delta, data, subs)
-    c2, p2 = ref.score_subsets(m, delta, data, subs)
-    assert np.array_equal(c1, c2)
-    assert np.array_equal(np.isnan(p1), np.isnan(p2))
-    if pinv_tol(name):
-        assert np.allclose(np.nan_to_num(p1), np.nan_to_num(p2), rtol=pinv_tol(name), atol=pinv_tol(name))
-    else:
-        assert np.array_equal(np.nan_to_num(p1), np.nan_to_num(p2))
+    assert np.array_equal(c1, want["counts"])
+    assert np.array_equal(np.isnan(p1), want["nan"])
+    assert_params(p1, want, pinv_tol(name))
+
+
+def horn_case():
+    data, _ = synth.absolute_orientation(500, seed=77, outlier_frac=0.0)
+    return data, np.random.default_rng(5).uniform(0.1, 3.0, 500)
 
 
 def test_weighted_horn_port_matches_reference(port, ref):
     """AbsoluteOrientationParametersEstimator::weightedLeastSquaresEstimate (.cxx:208-297): restatement vs the
     reference itself; unit weights reproduce the unweighted Horn solve; zero weights remove pairs."""
-    data, true = synth.absolute_orientation(500, seed=77, outlier_frac=0.0)
-    rng = np.random.default_rng(5)
-    w = rng.uniform(0.1, 3.0, 500)
-    a, b = port.weighted_absor(data, w), ref.weighted_absor(data, w)
+    data, w = horn_case()
+    b = reference_answer(ref, "horn", lambda r: {"params": r.weighted_absor(data, w)})["params"]
+    a = port.weighted_absor(data, w)
     assert len(a) == 7 and same_up_to_sign(a, b, SIGN_IDX["absor"], 1e-10)
     assert same_up_to_sign(port.weighted_absor(data, np.ones(500)), port.least_squares(MODELS["absor"], 2.0, data), SIGN_IDX["absor"], 1e-9)
     bad = data.copy()
@@ -162,41 +222,84 @@ def test_choose_unrank_and_stop_rule(port):
     assert port.num_tries(0.999, 100, 100, 3, 161700) == 0
 
 
+def reference_model_table(orc):
+    """(D, P, k) of every model id and of the first unknown id (-1s for None)."""
+    return {"info": np.array([orc.model_info(m) or (-1, -1, -1) for m in range(35)])}
+
+
 def test_model_tables_agree_everywhere(port, ref):
     """One id space: the Python tables of the oracle and of the engine binding, the C restatement and the reference harness
     describe every model with the same (doubles per datum, parameters, minimal subset)."""
     from lsqrrecipes_b200 import api
+    table = reference_answer(ref, "models", reference_model_table)["info"]
     assert MODELS == api.MODELS and len(MODELS) == 34
     for name, m in MODELS.items():
-        assert INFO[m] == api.MODEL_INFO[m] == port.model_info(m) == ref.model_info(m), name
-    assert port.model_info(34) is None and ref.model_info(34) is None and port.model_info(-1) is None
+        assert INFO[m] == api.MODEL_INFO[m] == port.model_info(m) == tuple(int(x) for x in table[m]), name
+    assert port.model_info(34) is None and tuple(table[34]) == (-1, -1, -1) and port.model_info(-1) is None
+
+
+def degenerate_case(name, m):
+    data = synth.degenerate_pool(name, seed=31 + m)
+    return data, synth.DELTAS[name], synth.random_subsets(len(data), INFO[m][2], 600, seed=7 + m)
+
+
+def reference_degenerate(orc, name, m, keep=None):
+    """Values are compared (pinv_tol models) for the hypotheses that explain more than their own subset; for the dense
+    systems only where the n x n system is well conditioned; for the calibration systems not at all (rejection pattern only)."""
+    data, delta, subs = degenerate_case(name, m)
+    k = INFO[m][2]
+    c, p = orc.score_subsets(m, delta, data, subs)
+    if pinv_tol(name) is None:
+        return reduce_answer(c, p, True, keep=keep)
+    ok = ~np.isnan(p[:, 0]) & (c > k)
+    if name.startswith("dense"):
+        ok &= np.array([np.linalg.cond(data[s][:, :k]) < 1e6 for s in subs])
+    if name in ("usxw", "uscp"):
+        ok[:] = False
+    return reduce_answer(c, p, False, rows=ok, keep=keep)
 
 
 @pytest.mark.parametrize("name,m", ALL)
 def test_port_matches_reference_on_degenerate_subsets(port, ref, name, m):
     """Minimal subsets with repeated, collinear, scaled and all-zero records: the restatement rejects exactly the subsets the
     reference rejects (empty parameter vector, RANSAC.hxx:87-88) and agrees on the rest."""
-    D, P, k = INFO[m]
-    data = synth.degenerate_pool(name, seed=31 + m)
-    subs = synth.random_subsets(len(data), k, 600, seed=7 + m)
-    delta = synth.DELTAS[name]
+    want = reference_answer(ref, f"degenerate.{name}", lambda r: reference_degenerate(r, name, m))
+    data, delta, subs = degenerate_case(name, m)
     c1, p1 = port.score_subsets(m, delta, data, subs)
-    c2, p2 = ref.score_subsets(m, delta, data, subs)
-    bad1, bad2 = np.isnan(p1[:, 0]), np.isnan(p2[:, 0])
+    bad1, bad2 = np.isnan(p1[:, 0]), want["nan"][:, 0]
     assert bad2.any() and not bad2.all(), "the pool must mix degenerate and valid subsets"
     assert np.array_equal(bad1, bad2), "same subsets rejected"
     if pinv_tol(name):
         # the reference's absolute rank test (singular values <= 2.2e-16) accepts numerically singular systems, whose "solution" is
-        # amplified rounding noise in either SVD: values are compared for the hypotheses that explain more than their own subset
-        ok = ~bad2 & (c2 > k)
-        if name.startswith("dense"):        # ... and whose n x n system is well conditioned
-            ok &= np.array([np.linalg.cond(data[s][:, :k]) < 1e6 for s in subs])
-        if name not in ("usxw", "uscp"):    # (the calibration systems of such pools are ill-conditioned throughout: rejection pattern only)
-            assert ok.any()
-            assert np.allclose(p1[ok], p2[ok], rtol=1e-6, atol=1e-6)
+        # amplified rounding noise in either SVD: values are compared for the rows reference_degenerate selects
+        if name not in ("usxw", "uscp"):
+            assert len(want["idx"])
+            assert_params(p1, want, 1e-6)
     else:
-        assert np.array_equal(np.nan_to_num(p1), np.nan_to_num(p2))
-        assert np.array_equal(c1, c2)
+        assert_params(p1, want, None)
+        assert np.array_equal(c1, want["counts"])
+
+
+def seed_cases(seed):
+    """(name, m, data, delta, subsets) of every model on fresh data with a threshold drawn per seed."""
+    rng = np.random.default_rng(1000 + seed)
+    for name, m in ALL:
+        k, n = INFO[m][2], 160
+        data, _ = synth.GENERATORS[name](n, seed=5000 + 37 * seed + m)
+        delta = synth.DELTAS[name] * float(rng.choice([0.25, 1.0, 3.0]))
+        yield name, m, data, delta, synth.random_subsets(n, k, 120, seed=seed + m)
+
+
+def reference_seed_case(orc, name, m, data, delta, subs, keep=None):
+    """The answer to the listed subsets, agree() of the best one (count and mask) and the algebraic least squares over it."""
+    c, p = orc.score_subsets(m, delta, data, subs)
+    out = reduce_answer(c, p, pinv_tol(name) is None, keep=keep)
+    b = int(np.argmax(c))
+    cnt, mask = orc.agree(m, delta, p[b], data)
+    inl = data[mask.astype(bool)]
+    ls = orc.least_squares(m, delta, inl, 0) if (len(inl) >= max(INFO[m][2], 4) and name != "usxw") else np.zeros(0)
+    out.update(best_params=p[b], best_agree=np.array([cnt]), mask=mask.astype(bool), ls0=ls)
+    return out
 
 
 @pytest.mark.parametrize("seed", range(4))
@@ -204,26 +307,18 @@ def test_port_matches_reference_across_seeds_and_thresholds(port, ref, seed):
     """Every model on fresh data with a threshold drawn per seed (tight thresholds put many data near the decision boundary):
     counts bit-exact, estimate() bit-exact where the reference's arithmetic is plain double, least squares over the best
     consensus set within 1e-8 (1e-6 for the cross-wire valley)."""
-    rng = np.random.default_rng(1000 + seed)
-    for name, m in ALL:
-        D, P, k = INFO[m]
-        n = 160
-        data, _ = synth.GENERATORS[name](n, seed=5000 + 37 * seed + m)
-        delta = synth.DELTAS[name] * float(rng.choice([0.25, 1.0, 3.0]))
-        subs = synth.random_subsets(n, k, 120, seed=seed + m)
+    for name, m, data, delta, subs in seed_cases(seed):
+        want = reference_answer(ref, f"seed{seed}.{name}", lambda r: reference_seed_case(r, name, m, data, delta, subs))
         c1, p1 = port.score_subsets(m, delta, data, subs)
-        c2, p2 = ref.score_subsets(m, delta, data, subs)
-        assert np.array_equal(np.isnan(p1), np.isnan(p2)), name
+        c2 = want["counts"]
+        assert np.array_equal(np.isnan(p1), want["nan"]), name
+        assert_params(p1, want, pinv_tol(name))
         if pinv_tol(name) is None:
-            assert np.array_equal(np.nan_to_num(p1), np.nan_to_num(p2)) and np.array_equal(c1, c2), name
+            assert np.array_equal(c1, c2), name
         else:
-            assert np.allclose(np.nan_to_num(p1), np.nan_to_num(p2), rtol=pinv_tol(name), atol=pinv_tol(name)), name
             # counts of the pseudo-inverse models: identical on identical parameter vectors
             b = int(np.argmax(c2))
-            assert port.agree(m, delta, p2[b], data)[0] == ref.agree(m, delta, p2[b], data)[0] == c2[b], name
-        b = int(np.argmax(c2))
-        _, mask = ref.agree(m, delta, p2[b], data)
-        inl = data[mask.astype(bool)]
-        if len(inl) >= max(k, 4) and name != "usxw":
-            a, r = port.least_squares(m, delta, inl, 0), ref.least_squares(m, delta, inl, 0)
-            assert same_up_to_sign(a, r, SIGN_IDX[name], 1e-8), name
+            assert port.agree(m, delta, want["best_params"], data)[0] == want["best_agree"][0] == c2[b], name
+        if len(want["ls0"]):
+            inl = data[want["mask"]]
+            assert same_up_to_sign(port.least_squares(m, delta, inl, 0), want["ls0"], SIGN_IDX[name], 1e-8), name
