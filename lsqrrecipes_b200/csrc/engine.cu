@@ -163,6 +163,9 @@ class Workers {
 };
 
 struct DataSet {
+  // the data of lsqr_upload: each rank of a sharded context refines its own point range and the moments are all-reduced.
+  // The data of a direct estimator call (least squares) stays whole on one device.
+  bool sharded = false;
   double* soa64 = nullptr;
   float* soa32 = nullptr;
   uint32_t* maskbits = nullptr;
@@ -207,7 +210,7 @@ struct lsqr_ctx {
   double delta = 0, aux = 0;
   int ls_type = 1;
 
-  DataSet main, scratch;
+  DataSet main{true}, scratch{false};
   unsigned char* staging = nullptr; size_t staging_cap = 0;
 
   // hypothesis buffers
@@ -235,7 +238,7 @@ struct lsqr_ctx {
   double* agree_pin = nullptr;                            // lsqr_agree on a handful of data: zero-copy parameters, data and answers
   // upload pipeline
   static constexpr int kRing = 4;
-  unsigned char* up_pin[kRing] = {nullptr, nullptr, nullptr, nullptr}; size_t up_pin_bytes = 0;
+  unsigned char* up_pin[kRing] = {nullptr, nullptr, nullptr, nullptr}; size_t up_pin_cap[kRing] = {0, 0, 0, 0};
   cudaEvent_t up_ev[kRing]{};             // chunk in ring slot i has been copied to the device
   cudaEvent_t up_land[8]{};               // chunk copies landed, round-robin
   std::unique_ptr<HostCopier> copier;
@@ -284,12 +287,21 @@ template <class T> int ensure(lsqr_ctx* ctx, T** p, size_t* cap, size_t want) {
   *cap = want;
   return 0;
 }
+// the same for page-locked host memory
+template <class T> int ensure_pinned(lsqr_ctx* ctx, T** p, size_t* cap, size_t want) {
+  if (*cap >= want && *p) return 0;
+  if (*p) cudaFreeHost(*p);
+  *p = nullptr; *cap = 0;
+  CK(cudaMallocHost((void**)p, want * sizeof(T)));
+  *cap = want;
+  return 0;
+}
 
 size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
 
 void free_dataset(DataSet& ds) {
   cudaFree(ds.soa64); cudaFree(ds.soa32); cudaFree(ds.maskbits); cudaFree(ds.center_dev);
-  ds = DataSet();
+  ds = DataSet{ds.sharded};
 }
 
 int ensure_dataset(lsqr_ctx* ctx, DataSet& ds, int D, uint32_t n) {
@@ -346,8 +358,15 @@ int comm_sum_f64(lsqr_ctx* ctx, double* dev, int count) {
   return 0;
 }
 
-// threads for staging copies between pageable and pinned memory: most of the cores, shared between the devices of a group
-int host_copy_threads(int W) { return std::min(12, std::max(1, ((int)std::thread::hardware_concurrency() * 3 / 4) / std::max(1, W))); }
+// the threads of the staging copies between pageable and pinned memory, created on first use: most of the cores, shared between
+// the devices of a group
+HostCopier& copier(lsqr_ctx* ctx) {
+  if (!ctx->copier) {
+    const int W = ctx->comm && ctx->world > 1 ? ctx->world : 1;
+    ctx->copier.reset(new HostCopier(std::min(12, std::max(1, ((int)std::thread::hardware_concurrency() * 3 / 4) / W))));
+  }
+  return *ctx->copier;
+}
 
 // ---- upload ----------------------------------------------------------------------------------------
 bool is_pinned(const void* p) {
@@ -357,6 +376,43 @@ bool is_pinned(const void* p) {
   return ok;
 }
 
+// Host -> device copies on the copy stream, overlapping the work that the compute stream does with what has landed: straight
+// from page-locked memory; from pageable memory through the ring of pinned buffers, which the staging threads fill.
+struct StagedCopy {
+  lsqr_ctx* ctx;
+  bool pinned;   // the source is page-locked
+  int ring = 0, land = 0;
+  // before the first put(): `piece` = the largest put().  The copies must not overtake work already enqueued on the compute
+  // stream (it may still read their destination).
+  int start(size_t piece) {
+    if (!pinned) {
+      CK(cudaStreamSynchronize(ctx->copy_stream));   // an earlier upload may still be reading the pinned ring
+      for (int i = 0; i < lsqr_ctx::kRing; i++) if (int rc = ensure_pinned(ctx, &ctx->up_pin[i], &ctx->up_pin_cap[i], piece)) return rc;
+      copier(ctx);
+    }
+    CK(cudaEventRecord(ctx->up_land[7], ctx->stream));
+    CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->up_land[7], 0));
+    return LSQR_OK;
+  }
+  int put(void* dst, const void* src, size_t bytes) {
+    if (pinned) { CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->copy_stream)); return LSQR_OK; }
+    const int b = ring % lsqr_ctx::kRing;
+    if (ring >= lsqr_ctx::kRing) CK(cudaEventSynchronize(ctx->up_ev[b]));   // the copy that used this buffer has finished
+    ring++;
+    ctx->copier->copy(ctx->up_pin[b], src, bytes);
+    CK(cudaMemcpyAsync(dst, ctx->up_pin[b], bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
+    CK(cudaEventRecord(ctx->up_ev[b], ctx->copy_stream));
+    return LSQR_OK;
+  }
+  // the compute stream waits for every copy enqueued so far
+  int landed() {
+    cudaEvent_t ev = ctx->up_land[land++ % 7];
+    CK(cudaEventRecord(ev, ctx->copy_stream));
+    CK(cudaStreamWaitEvent(ctx->stream, ev, 0));
+    return LSQR_OK;
+  }
+};
+
 // AoS records, host or device -> SoA fp64 + fp32 on the device, chunk by chunk.
 //   * single context: chunk c is copied on the copy stream and transposed on the compute stream as soon as it has landed;
 //   * natively sharded context (ctx->comm): rank r copies chunks r, r + W, r + 2W, ... of the host buffer and round j of
@@ -364,7 +420,7 @@ bool is_pinned(const void* p) {
 // after_round(lo, hi, first, last): called after the transposition of records [lo, hi) has been enqueued (compute() scores its
 // first round of hypotheses against every range as it lands)
 using RoundFn = std::function<int(size_t, size_t, bool, bool)>;
-int upload_to(lsqr_ctx* ctx, DataSet& ds, const void* aos, size_t n, size_t stride, bool on_device, bool allow_sharded, const RoundFn* after_round = nullptr) {
+int upload_to(lsqr_ctx* ctx, DataSet& ds, const void* aos, size_t n, size_t stride, bool on_device, const RoundFn* after_round = nullptr) {
   if (ctx->model < 0) return fail(ctx, LSQR_ERR_STATE, "lsqr_set_estimator must be called before uploading data");
   const ModelInfo mi = model_info(ctx->model);
   if (n > 0xFFFFFFF0ull) return fail(ctx, LSQR_ERR_ARG, "too many data records");
@@ -384,52 +440,24 @@ int upload_to(lsqr_ctx* ctx, DataSet& ds, const void* aos, size_t n, size_t stri
     CKL();
     return LSQR_OK;
   }
-  const bool sharded = allow_sharded && ctx->comm != nullptr && ctx->world > 1;
+  const bool sharded = ds.sharded && ctx->comm != nullptr && ctx->world > 1;
   const int W = sharded ? ctx->world : 1;
-  const bool pinned = is_pinned(aos);
+  StagedCopy up{ctx, is_pinned(aos)};
   // chunk: at least the centre sample, ~1/8 of a rank's share, between 256 KB and 16 MB (4 MB from pageable memory: the first
   // copy cannot start before the first chunk has been staged)
-  const size_t chunk_cap = pinned ? (16u << 20) : (4u << 20);
+  const size_t chunk_cap = up.pinned ? (16u << 20) : (4u << 20);
   size_t chunk_rec = std::max<size_t>(kCenterSample, std::min<size_t>(chunk_cap / stride, std::max<size_t>((256u << 10) / stride, (n / W + 7) / 8)));
   chunk_rec = round_up(chunk_rec, 1024);   // rounds start on tile boundaries of every consensus kernel
   const size_t chunk_bytes = chunk_rec * stride;
   const size_t n_chunks = (n + chunk_rec - 1) / chunk_rec, rounds = (n_chunks + W - 1) / W;
   if (int rc = ensure(ctx, &ctx->staging, &ctx->staging_cap, rounds * W * chunk_bytes)) return rc;
-  if (!pinned) {
-    if (ctx->up_pin_bytes < chunk_bytes) {
-      for (int i = 0; i < lsqr_ctx::kRing; i++) { if (ctx->up_pin[i]) cudaFreeHost(ctx->up_pin[i]); ctx->up_pin[i] = nullptr; }
-      ctx->up_pin_bytes = 0;
-      for (int i = 0; i < lsqr_ctx::kRing; i++) CK(cudaMallocHost((void**)&ctx->up_pin[i], chunk_bytes));
-      ctx->up_pin_bytes = chunk_bytes;
-    }
-    CK(cudaStreamSynchronize(ctx->copy_stream));   // an earlier upload may still be reading the pinned ring
-    if (!ctx->copier) ctx->copier.reset(new HostCopier(host_copy_threads(W)));
-  }
+  if (int rc = up.start(chunk_bytes)) return rc;
   const unsigned char* host = static_cast<const unsigned char*>(aos);
-  // the copy stream must not run ahead of work still reading the staging buffer
-  CK(cudaEventRecord(ctx->up_land[7], s));
-  CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->up_land[7], 0));
-  int ring = 0, land = 0;
   for (size_t j = 0; j < rounds; j++) {
     const size_t g = j * W + (sharded ? ctx->rank : 0);       // the chunk this rank fetches in round j
     const size_t lo = std::min(n, g * chunk_rec), hi = std::min(n, (g + 1) * chunk_rec);
-    if (hi > lo) {
-      const size_t bytes = (hi - lo) * stride;
-      const unsigned char* src = host + lo * stride;
-      if (!pinned) {
-        const int b = ring % lsqr_ctx::kRing;
-        if (ring >= lsqr_ctx::kRing) CK(cudaEventSynchronize(ctx->up_ev[b]));   // the copy that used this buffer has finished
-        ring++;
-        ctx->copier->copy(ctx->up_pin[b], src, bytes);
-        CK(cudaMemcpyAsync(ctx->staging + g * chunk_bytes, ctx->up_pin[b], bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
-        CK(cudaEventRecord(ctx->up_ev[b], ctx->copy_stream));
-      } else {
-        CK(cudaMemcpyAsync(ctx->staging + g * chunk_bytes, src, bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
-      }
-    }
-    cudaEvent_t landed = ctx->up_land[land++ % 7];
-    CK(cudaEventRecord(landed, ctx->copy_stream));
-    CK(cudaStreamWaitEvent(s, landed, 0));
+    if (hi > lo) if (int rc = up.put(ctx->staging + g * chunk_bytes, host + lo * stride, (hi - lo) * stride)) return rc;
+    if (int rc = up.landed()) return rc;
     if (sharded) CKN(nccl().AllGather(ctx->staging + g * chunk_bytes, ctx->staging + j * W * chunk_bytes, chunk_bytes, ncclUint8, ctx->comm, s));
     if (j == 0) { launch_center_sample(ctx->model, ctx->staging, stride, sample, ds.center_dev, s); ctx->launches++; }
     const size_t r_lo = std::min(n, j * W * chunk_rec), r_hi = std::min(n, (j + 1) * W * chunk_rec);
@@ -440,35 +468,6 @@ int upload_to(lsqr_ctx* ctx, DataSet& ds, const void* aos, size_t n, size_t stri
   }
   CKL();
   return LSQR_OK;
-}
-
-// ---- host copy of the device sampler (models.cuh: philox4x32_10, sample_subset) ---------------------
-// compute() draws the minimal subsets of its first round on the host so that their records can be fetched from the caller's
-// buffer ahead of the bulk upload; the indices are bit-identical to what the device draws for the same (seed, hypothesis).
-void host_philox(uint32_t c[4], uint32_t k0, uint32_t k1) {
-  for (int r = 0; r < 10; r++) {
-    const uint64_t p0 = (uint64_t)0xD2511F53u * c[0], p1 = (uint64_t)0xCD9E8D57u * c[2];
-    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c[1] ^ k0, n1 = (uint32_t)p1, n2 = (uint32_t)(p0 >> 32) ^ c[3] ^ k1, n3 = (uint32_t)p0;
-    c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
-    k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-  }
-}
-void host_sample_subset(int K, uint64_t gidx, uint64_t seed, uint32_t n, int32_t* out) {
-  uint32_t rnd[4 * ((LSQR_MAX_SUBSET + 3) / 4)];
-  for (int blk = 0; blk < (K + 3) / 4; blk++) {
-    uint32_t c[4] = {(uint32_t)gidx, (uint32_t)(gidx >> 32), (uint32_t)blk, 0u};
-    host_philox(c, (uint32_t)seed, (uint32_t)(seed >> 32));
-    for (int i = 0; i < 4; i++) rnd[4 * blk + i] = c[i];
-  }
-  uint32_t sorted[LSQR_MAX_SUBSET];
-  for (int j = 0; j < K; j++) {
-    uint32_t v = (uint32_t)(((uint64_t)rnd[j] * (uint64_t)(n - j)) >> 32);   // uniform in [0, n-j)
-    for (int i = 0; i < j; i++) if (v >= sorted[i]) v++;                       // skip taken indices, ascending
-    out[j] = (int32_t)v;
-    int pos = j;
-    for (int i = j - 1; i >= 0; i--) if (sorted[i] > v) { sorted[i + 1] = sorted[i]; pos = i; }
-    sorted[pos] = v;
-  }
 }
 
 // Number of subsets as the reference counts them (RANSAC::choose, RANSAC.hxx:254-280): the binomial
@@ -494,7 +493,27 @@ uint64_t choose_exact(uint64_t n, uint64_t k) {
   return (uint64_t)(r + 0.5L);
 }
 
+// The stop rule of RANSAC.hxx:104-110 after a new best count.
+uint64_t tries_after(uint32_t best_count, uint32_t n, int K, double numerator, unsigned int all_tries) {
+  const double denominator = log(1.0 - pow((double)best_count / (double)n, (double)K));  // :107
+  const double t = numerator / denominator + 0.5;
+  const uint64_t nt = (t >= 4294967295.0 || !(t == t)) ? 0xFFFFFFFFull : (t < 0 ? 0x80000000ull : (uint64_t)t);  // (int) cast semantics of :108
+  return std::min<uint64_t>(nt, all_tries);  // :110
+}
+
 constexpr size_t kHypBatch = (size_t)1 << 22;
+
+// The winner of a request whose first hypothesis is `first` -> its count, index, parameters and subset.
+void decode_winner(const WinnerRecord& w, uint64_t first, const ModelInfo& mi, lsqr_score_result* res) {
+  res->n_valid = (uint32_t)w.n_valid;
+  res->best_count = (uint32_t)(w.key >> 32);
+  for (int j = 0; j < LSQR_MAX_SUBSET; j++) res->best_subset[j] = -1;
+  res->best_index = 0;
+  if (res->best_count == 0) return;
+  res->best_index = first + (0xFFFFFFFFull - (w.key & 0xFFFFFFFFull));
+  for (int j = 0; j < mi.P; j++) res->best_params[j] = w.params[j];
+  for (int j = 0; j < mi.K; j++) res->best_subset[j] = w.subset[j];
+}
 
 // Minimal solve + consensus + arg-max of one request; the winner is re-derived on the device and fetched with one copy.
 int score_impl(lsqr_ctx* ctx, const lsqr_score_args* a, lsqr_score_result* res) {
@@ -582,20 +601,11 @@ int score_impl(lsqr_ctx* ctx, const lsqr_score_args* a, lsqr_score_result* res) 
   float total_ms = 0.f;
   CK(cudaEventElapsedTime(&total_ms, ctx->ev[0], ctx->ev[1]));
   if (one_batch && timed) { float ms = 0.f; CK(cudaEventElapsedTime(&ms, ctx->ev[2], ctx->ev[3])); cons_ms = ms; }
-  const WinnerRecord& w = *ctx->winner_pin;
   res->score_ms = total_ms; res->consensus_ms = cons_ms;
-  res->n_valid = (uint32_t)w.n_valid;
-  res->best_count = (uint32_t)(w.key >> 32);
-  for (int j = 0; j < LSQR_MAX_SUBSET; j++) res->best_subset[j] = -1;
-  if (res->best_count == 0) { res->best_index = 0; return LSQR_OK; }
-  const uint64_t rel = 0xFFFFFFFFull - (w.key & 0xFFFFFFFFull);
-  res->best_index = a->first + rel;
-  if (dev_winner) {
-    for (int j = 0; j < mi.P; j++) res->best_params[j] = w.params[j];
-    for (int j = 0; j < mi.K; j++) res->best_subset[j] = w.subset[j];
-    return LSQR_OK;
-  }
+  decode_winner(*ctx->winner_pin, a->first, mi, res);   // without dev_winner the record holds the key only: see below
+  if (dev_winner || res->best_count == 0) return LSQR_OK;
   // listed sampler whose winner's row is no longer on this device: upload that one row and solve it
+  const uint64_t rel = res->best_index - a->first;
   if (int rc = ensure_hyp(ctx, 1)) return rc;
   SolveArgs sa{};
   sa.model = ctx->model; sa.sampler = a->sampler; sa.seed = a->seed; sa.first = res->best_index; sa.H = 1; sa.hld = ctx->hcap;
@@ -620,17 +630,27 @@ int score_impl(lsqr_ctx* ctx, const lsqr_score_args* a, lsqr_score_result* res) 
   return LSQR_OK;
 }
 
-int reduce_moments(lsqr_ctx* ctx, int nm) {
+int reduce_moments(lsqr_ctx* ctx, const DataSet& ds, int nm) {
   launch_reduce_partials(ctx->rb, nm, ctx->stream); ctx->launches++;
-  return comm_sum_f64(ctx, ctx->rb.moments, nm);
+  return ds.sharded ? comm_sum_f64(ctx, ctx->rb.moments, nm) : LSQR_OK;
 }
 
-void shard_range(const lsqr_ctx* ctx, uint32_t n, uint32_t* begin, uint32_t* end) {
-  if (ctx->world <= 1) { *begin = 0; *end = n; return; }
+// this rank's data of the data set, [begin, end)
+void shard_range(const lsqr_ctx* ctx, const DataSet& ds, uint32_t* begin, uint32_t* end) {
+  const uint32_t n = ds.n;
+  if (!ds.sharded || ctx->world <= 1) { *begin = 0; *end = n; return; }
   const uint64_t words = ((uint64_t)n + 31) / 32;
   const uint64_t w0 = words * (uint64_t)ctx->rank / (uint64_t)ctx->world, w1 = words * (uint64_t)(ctx->rank + 1) / (uint64_t)ctx->world;
   *begin = (uint32_t)std::min<uint64_t>(w0 * 32, n);
   *end = (uint32_t)std::min<uint64_t>(w1 * 32, n);
+}
+
+// P parameters from the host -> small_dev + kSmIn, through the pinned scratch
+int put_params(lsqr_ctx* ctx, const double* params) {
+  const int P = model_info(ctx->model).P;
+  for (int j = 0; j < P; j++) ctx->pin[32 + j] = params[j];
+  CK(cudaMemcpyAsync(ctx->small_dev + kSmIn, ctx->pin + 32, sizeof(double) * P, cudaMemcpyHostToDevice, ctx->stream));
+  return LSQR_OK;
 }
 
 // Consensus set of the parameters at params_dev (device) over this rank's point shard + the least-squares moments of it,
@@ -639,7 +659,7 @@ int consensus_enqueue(lsqr_ctx* ctx, DataSet& ds, const double* params_dev, bool
   const ModelInfo mi = model_info(ctx->model);
   cudaStream_t s = ctx->stream;
   uint32_t b, e;
-  shard_range(ctx, ds.n, &b, &e);
+  shard_range(ctx, ds, &b, &e);
   const int nm = moments_count(ctx->model, false);
   if (want_bytes) if (int rc = ensure(ctx, &ctx->mask_dev, &ctx->mask_dev_cap, (size_t)std::max<uint32_t>(ds.n, 1))) return rc;
   CK(cudaEventRecord(ctx->ev[4], s));
@@ -648,7 +668,7 @@ int consensus_enqueue(lsqr_ctx* ctx, DataSet& ds, const double* params_dev, bool
   launch_mask_moments(ctx->model, ds.view(), b, e, params_dev, 1, nullptr, ctx->cfg, ctx->rb, s); ctx->launches++;
   ctx->rb.maskbytes = nullptr;
   CK(cudaEventRecord(ctx->ev[5], s));
-  if (int rc = reduce_moments(ctx, nm)) return rc;
+  if (int rc = reduce_moments(ctx, ds, nm)) return rc;
   CKL();
   ctx->refine_bytes = (double)(e - b) * mi.D * sizeof(double) + (double)(e - b) / 8.0 + (want_bytes ? (double)(e - b) : 0.0);
   ds.moments_valid = true; ds.mask_valid = true; ds.bytes_valid = want_bytes;
@@ -657,11 +677,9 @@ int consensus_enqueue(lsqr_ctx* ctx, DataSet& ds, const double* params_dev, bool
 
 int consensus_impl(lsqr_ctx* ctx, DataSet& ds, const double* params, uint32_t* out_count) {
   if (!ds.soa64) return fail(ctx, LSQR_ERR_STATE, "no data uploaded");
-  const ModelInfo mi = model_info(ctx->model);
   cudaStream_t s = ctx->stream;
   CK(cudaSetDevice(ctx->device));
-  for (int j = 0; j < mi.P; j++) ctx->pin[32 + j] = params[j];
-  CK(cudaMemcpyAsync(ctx->small_dev + kSmIn, ctx->pin + 32, sizeof(double) * mi.P, cudaMemcpyHostToDevice, s));
+  if (int rc = put_params(ctx, params)) return rc;
   if (int rc = consensus_enqueue(ctx, ds, ctx->small_dev + kSmIn, false)) return rc;
   CK(cudaMemcpyAsync(ctx->pin, ctx->rb.moments, sizeof(double), cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
@@ -680,14 +698,14 @@ int refine_enqueue(lsqr_ctx* ctx, DataSet& ds, int use_mask) {
   ctx->rb.maskbits = ds.maskbits;
   ctx->rb.maskbytes = nullptr;
   uint32_t b, e;
-  shard_range(ctx, ds.n, &b, &e);
+  shard_range(ctx, ds, &b, &e);
   const int nm = moments_count(ctx->model, false);
   ctx->lm_iterations = 0;
   if (!(use_mask && ds.moments_valid)) {
     CK(cudaEventRecord(ctx->ev[4], s));
     launch_mask_moments(ctx->model, dv, b, e, nullptr, use_mask ? 2 : 0, nullptr, ctx->cfg, ctx->rb, s); ctx->launches++;
     CK(cudaEventRecord(ctx->ev[5], s));
-    if (int rc = reduce_moments(ctx, nm)) return rc;
+    if (int rc = reduce_moments(ctx, ds, nm)) return rc;
     ds.moments_valid = false;
   }
   double* out_dev = ctx->small_dev + kSmOut;
@@ -706,7 +724,7 @@ int refine_enqueue(lsqr_ctx* ctx, DataSet& ds, int use_mask) {
     for (int it = 0; it < 5200; it += kLmAhead) {
       for (int k = 0; k < kLmAhead; k++) {
         launch_mask_moments(ctx->model, dv, b, e, nullptr, use_mask ? 2 : 0, st, ctx->cfg, ctx->rb, s); ctx->launches++;
-        if (int rc = reduce_moments(ctx, nlm)) return rc;
+        if (int rc = reduce_moments(ctx, ds, nlm)) return rc;
         launch_lm_update(ctx->model, ctx->rb.moments, st, s); ctx->launches++;
       }
       CK(cudaMemcpyAsync(ctx->pin + 48, st + lm_status_offset(), 3 * sizeof(double), cudaMemcpyDeviceToHost, s));   // status, phase, evaluations
@@ -737,17 +755,15 @@ int refine_impl(lsqr_ctx* ctx, DataSet& ds, int use_mask, double* out_params, in
 
 // pinned -> pageable copy of a result, by the staging threads when it is large
 void host_copy(lsqr_ctx* ctx, void* dst, const void* src, size_t bytes) {
-  if (bytes >= (1u << 20)) {
-    if (!ctx->copier) ctx->copier.reset(new HostCopier(host_copy_threads(ctx->world > 1 && ctx->comm ? ctx->world : 1)));
-    ctx->copier->copy(dst, src, bytes);
-  } else memcpy(dst, src, bytes);
+  if (bytes >= (1u << 20)) copier(ctx).copy(dst, src, bytes);
+  else memcpy(dst, src, bytes);
 }
 
 // Enqueues the copy of this rank's part of the consensus set (bytes [b, e) of out_bytes; everything when unsharded) and
 // reports whether a bounce through the pinned buffer has to be finished after the synchronisation.
 int mask_download_enqueue(lsqr_ctx* ctx, DataSet& ds, uint8_t* out_bytes, bool* bounce, uint32_t* pb, uint32_t* pe) {
   uint32_t b, e;
-  shard_range(ctx, ds.n, &b, &e);
+  shard_range(ctx, ds, &b, &e);
   *pb = b; *pe = e; *bounce = false;
   if (!out_bytes || e <= b) return LSQR_OK;
   if (int rc = ensure(ctx, &ctx->mask_dev, &ctx->mask_dev_cap, (size_t)std::max<uint32_t>(ds.n, 1))) return rc;
@@ -755,12 +771,7 @@ int mask_download_enqueue(lsqr_ctx* ctx, DataSet& ds, uint8_t* out_bytes, bool* 
   // a caller buffer that is itself page-locked takes the DMA directly; any other goes through the library's pinned buffer
   // (persistent: a cudaMalloc/cudaFree pair per call costs up to 0.3 s after the thousands of launches of a large request)
   const bool direct = is_pinned(out_bytes);
-  if (!direct && ctx->mask_pin_cap < ds.n) {
-    if (ctx->mask_pin) cudaFreeHost(ctx->mask_pin);
-    ctx->mask_pin = nullptr; ctx->mask_pin_cap = 0;
-    CK(cudaMallocHost((void**)&ctx->mask_pin, ds.n));
-    ctx->mask_pin_cap = ds.n;
-  }
+  if (!direct) if (int rc = ensure_pinned(ctx, &ctx->mask_pin, &ctx->mask_pin_cap, ds.n)) return rc;
   CK(cudaMemcpyAsync((direct ? out_bytes : ctx->mask_pin) + b, ctx->mask_dev + b, e - b, cudaMemcpyDeviceToHost, ctx->stream));
   *bounce = !direct;
   return LSQR_OK;
@@ -778,15 +789,15 @@ int get_mask_impl(lsqr_ctx* ctx, DataSet& ds, uint8_t* out_bytes) {
 }
 
 // winner -> consensus set -> least squares: RANSAC.hxx:129-138 / :175-185.  Everything is enqueued behind the scoring; one
-// synchronisation brings back count, parameters and the mask.
-int finish_ransac(lsqr_ctx* ctx, const lsqr_score_result& best, uint8_t* out_mask, lsqr_compute_result* res) {
+// synchronisation brings back count, parameters and the mask.  tries / score_ms: the hypotheses scored and their device time.
+int finish_ransac(lsqr_ctx* ctx, const lsqr_score_result& best, uint64_t tries, double score_ms, uint8_t* out_mask, lsqr_compute_result* res) {
+  res->tries = tries; res->device_ms = score_ms;
   res->best_count = best.best_count; res->best_index = best.best_index;
   if (best.best_count == 0) { res->n_params = 0; res->fraction = 0.0; return LSQR_OK; }
   const ModelInfo mi = model_info(ctx->model);
   cudaStream_t s = ctx->stream;
   DataSet& ds = ctx->main;
-  for (int j = 0; j < mi.P; j++) ctx->pin[32 + j] = best.best_params[j];
-  CK(cudaMemcpyAsync(ctx->small_dev + kSmIn, ctx->pin + 32, sizeof(double) * mi.P, cudaMemcpyHostToDevice, s));
+  if (int rc = put_params(ctx, best.best_params)) return rc;
   if (int rc = consensus_enqueue(ctx, ds, ctx->small_dev + kSmIn, out_mask != nullptr)) return rc;
   CK(cudaMemcpyAsync(ctx->pin, ctx->rb.moments, sizeof(double), cudaMemcpyDeviceToHost, s));
   bool bounce = false; uint32_t b = 0, e = 0;
@@ -798,6 +809,7 @@ int finish_ransac(lsqr_ctx* ctx, const lsqr_score_result& best, uint8_t* out_mas
   float ms = 0.f;
   CK(cudaEventElapsedTime(&ms, ctx->ev[4], ctx->ev[5]));
   ctx->refine_kernel_ms = ms;
+  res->device_ms += ms;
   const uint32_t cnt = (uint32_t)(ctx->pin[0] + 0.5);
   const int np = (int)ctx->pin[1];
   res->best_count = cnt;
@@ -807,7 +819,43 @@ int finish_ransac(lsqr_ctx* ctx, const lsqr_score_result& best, uint8_t* out_mas
   return LSQR_OK;
 }
 
-uint64_t tries_after(uint32_t best_count, uint32_t n, int K, double numerator, unsigned int all_tries);
+// lsqr_ransac's adaptive loop (RANSAC.hxx:100-110): hypotheses [0, done) have been scored, `best` is the first of the best.
+struct RansacRounds {
+  uint32_t n; int K;
+  double numerator;          // log(1 - prob)
+  unsigned int all_tries;    // RANSAC.hxx:41
+  uint64_t num_tries, done = 0;
+  lsqr_score_result best{};
+  bool perfect = false;      // a hypothesis agrees with every datum
+  double dev_ms = 0;
+
+  RansacRounds(uint32_t n_, int K_, double prob) : n(n_), K(K_), numerator(log(1.0 - prob)), all_tries(choose_ref(n_, (unsigned)K_)), num_tries(all_tries) {}
+  // the result of the next `count` hypotheses
+  void take(const lsqr_score_result& r, uint64_t count) {
+    dev_ms += r.score_ms;
+    done += count;
+    if (r.best_count > best.best_count) {  // strict '>' : RANSAC.hxx:100
+      best = r;
+      if (best.best_count == n) perfect = true;   // :104-105
+      else num_tries = tries_after(best.best_count, n, K, numerator, all_tries);  // :107-110
+    }
+  }
+};
+
+// Rounds of `round`, 4x, 16x ... (up to 1 Mi) Philox hypotheses until the stop rule or a perfect hypothesis ends the loop; a
+// typical problem (inlier ratio ~0.5, k = 3: 65 tries) ends after the first, small round of 256.
+int ransac_rounds(lsqr_ctx* ctx, int precision, uint64_t seed, uint64_t round, RansacRounds& st) {
+  while (!st.perfect && st.done < st.num_tries) {
+    lsqr_score_args a{};
+    a.sampler = LSQR_SAMPLE_PHILOX; a.precision = precision; a.seed = seed; a.first = st.done;
+    a.count = std::min<uint64_t>(round, st.num_tries - st.done);
+    lsqr_score_result r{};
+    if (int rc = score_impl(ctx, &a, &r)) return rc;
+    st.take(r, a.count);
+    round = std::min<uint64_t>(round * 4, (uint64_t)1 << 20);
+  }
+  return LSQR_OK;
+}
 
 int ransac_impl(lsqr_ctx* ctx, double prob, int precision, uint64_t seed, uint8_t* out_mask, lsqr_compute_result* res) {
   if (ctx->model < 0 || !ctx->main.soa64) return fail(ctx, LSQR_ERR_STATE, "set the estimator and upload data first");
@@ -816,32 +864,9 @@ int ransac_impl(lsqr_ctx* ctx, double prob, int precision, uint64_t seed, uint8_
   const uint32_t n = ctx->main.n;
   // RANSAC.hxx:16-19: fewer data than the minimal subset, or probability outside (0,1) -> return 0
   if (n < (uint32_t)mi.K || prob >= 1.0 || prob <= 0.0) return LSQR_OK;
-  const double numerator = log(1.0 - prob);
-  const unsigned int all_tries = choose_ref(n, (unsigned)mi.K);  // RANSAC.hxx:41
-  // rounds of 256, 1024, 4096 ... hypotheses: the stop rule (:107-110) is re-evaluated between rounds, and a typical problem
-  // (inlier ratio ~0.5, k = 3: 65 tries) ends after the first, small one
-  uint64_t num_tries = all_tries, done = 0, round = 256;
-  lsqr_score_result best{};
-  double dev_ms = 0;
-  while (done < num_tries) {
-    lsqr_score_args a{};
-    a.sampler = LSQR_SAMPLE_PHILOX; a.precision = precision; a.seed = seed; a.first = done;
-    a.count = std::min<uint64_t>(round, num_tries - done);
-    lsqr_score_result r{};
-    if (int rc = score_impl(ctx, &a, &r)) return rc;
-    dev_ms += r.score_ms;
-    done += a.count;
-    if (r.best_count > best.best_count) {  // strict '>' : RANSAC.hxx:100
-      best = r;
-      if (best.best_count == n) break;   // :104-105
-      num_tries = tries_after(best.best_count, n, mi.K, numerator, all_tries);  // :107-110
-    }
-    round = std::min<uint64_t>(round * 4, (uint64_t)1 << 20);
-  }
-  res->tries = done;
-  int rc = finish_ransac(ctx, best, out_mask, res);
-  res->device_ms = dev_ms + ctx->refine_kernel_ms;
-  return rc;
+  RansacRounds st(n, mi.K, prob);
+  if (int rc = ransac_rounds(ctx, precision, seed, 256, st)) return rc;
+  return finish_ransac(ctx, st.best, st.done, st.dev_ms, out_mask, res);
 }
 
 int ransac_exhaustive_impl(lsqr_ctx* ctx, int precision, uint8_t* out_mask, lsqr_compute_result* res) {
@@ -856,18 +881,7 @@ int ransac_exhaustive_impl(lsqr_ctx* ctx, int precision, uint8_t* out_mask, lsqr
   a.sampler = LSQR_SAMPLE_EXHAUSTIVE; a.precision = precision; a.first = 0; a.count = total;
   lsqr_score_result r{};
   if (int rc = score_impl(ctx, &a, &r)) return rc;
-  res->tries = total;
-  int rc = finish_ransac(ctx, r, out_mask, res);
-  res->device_ms = r.score_ms + ctx->refine_kernel_ms;
-  return rc;
-}
-
-// The stop rule of RANSAC.hxx:104-110 after a new best count.
-uint64_t tries_after(uint32_t best_count, uint32_t n, int K, double numerator, unsigned int all_tries) {
-  const double denominator = log(1.0 - pow((double)best_count / (double)n, (double)K));  // :107
-  const double t = numerator / denominator + 0.5;
-  const uint64_t nt = (t >= 4294967295.0 || !(t == t)) ? 0xFFFFFFFFull : (t < 0 ? 0x80000000ull : (uint64_t)t);  // (int) cast semantics of :108
-  return std::min<uint64_t>(nt, all_tries);  // :110
+  return finish_ransac(ctx, r, total, r.score_ms, out_mask, res);
 }
 
 // RANSAC<T,S>::compute with the data still on the host: lsqr_upload + lsqr_ransac in one pass, same results bit for bit.  The
@@ -886,24 +900,20 @@ int compute_impl(lsqr_ctx* ctx, const void* aos, size_t n, size_t stride, double
   CK(cudaSetDevice(ctx->device));
   cudaStream_t s = ctx->stream;
   const uint32_t N = (uint32_t)n;
-  const double numerator = log(1.0 - prob);
-  const unsigned int all_tries = choose_ref(N, (unsigned)mi.K);  // RANSAC.hxx:41
-  const uint64_t H0 = std::min<uint64_t>(256, all_tries);         // the first round of lsqr_ransac
+  RansacRounds st(N, mi.K, prob);
+  const uint64_t H0 = std::min<uint64_t>(256, st.all_tries);      // the first round of lsqr_ransac
   const uint64_t lo = H0 * (uint64_t)ctx->rank / (uint64_t)ctx->world, hi = H0 * (uint64_t)(ctx->rank + 1) / (uint64_t)ctx->world;
   const uint32_t B = (uint32_t)(hi - lo);
   // subsets of the whole round (every rank keeps the list: the winner is re-derived from it), records of this rank's share
   std::vector<int32_t> subs((size_t)H0 * mi.K);
-  for (uint64_t h = 0; h < H0; h++) host_sample_subset(mi.K, h, seed, N, &subs[h * mi.K]);
+#define CALL(MM) for (uint64_t h = 0; h < H0; h++) sample_subset<Model<MM>::K>(h, seed, N, &subs[h * mi.K])
+  LSQR_DISPATCH_MODEL(ctx->model, CALL)
+#undef CALL
   if (int rc = ensure_hyp(ctx, std::max<uint32_t>(B, 1))) return rc;
   if (int rc = ensure(ctx, &ctx->list_dev, &ctx->list_cap, (size_t)H0 * mi.K)) return rc;
   const size_t gbytes = (size_t)std::max<uint32_t>(B, 1) * mi.K * stride;
   if (int rc = ensure(ctx, &ctx->gather_dev, &ctx->gather_cap, gbytes)) return rc;
-  if (ctx->gather_pin_cap < gbytes + sizeof(int32_t) * H0 * mi.K) {
-    if (ctx->gather_pin) cudaFreeHost(ctx->gather_pin);
-    ctx->gather_pin = nullptr; ctx->gather_pin_cap = 0;
-    CK(cudaMallocHost((void**)&ctx->gather_pin, gbytes + sizeof(int32_t) * H0 * mi.K));
-    ctx->gather_pin_cap = gbytes + sizeof(int32_t) * H0 * mi.K;
-  }
+  if (int rc = ensure_pinned(ctx, &ctx->gather_pin, &ctx->gather_pin_cap, gbytes + sizeof(int32_t) * H0 * mi.K)) return rc;
   const unsigned char* host = static_cast<const unsigned char*>(aos);
   for (uint32_t h = 0; h < B; h++)
     for (int j = 0; j < mi.K; j++) memcpy(ctx->gather_pin + ((size_t)h * mi.K + j) * stride, host + (size_t)subs[(lo + h) * mi.K + j] * stride, sizeof(double) * mi.D);
@@ -929,7 +939,7 @@ int compute_impl(lsqr_ctx* ctx, const void* aos, size_t n, size_t stride, double
     if (r_hi > r_lo) ctx->launches += launch_consensus(ctx->model, precision, ds.range(r_lo, r_hi, last), ctx->hyp64, ctx->hyp32, ctx->hcap, B, ctx->cfg, ctx->counts, ctx->num_sms, s);
     return 0;
   };
-  if (int rc = upload_to(ctx, ds, aos, n, stride, false, true, &score_range)) return rc;
+  if (int rc = upload_to(ctx, ds, aos, n, stride, false, &score_range)) return rc;
   const DataView dv = ds.view();
   if (B) { launch_argmax(ctx->counts, B, (uint32_t)lo, ctx->key_dev, s); ctx->launches++; }
   if (int rc = comm_max_u64(ctx, ctx->key_dev)) return rc;
@@ -942,42 +952,12 @@ int compute_impl(lsqr_ctx* ctx, const void* aos, size_t n, size_t stride, double
   CK(cudaStreamSynchronize(s));
   float ms0 = 0.f;
   CK(cudaEventElapsedTime(&ms0, ctx->ev[0], ctx->ev[1]));
-  double dev_ms = ms0;   // includes the upload it overlaps
-  const WinnerRecord& w = *ctx->winner_pin;
-  lsqr_score_result best{};
-  best.best_count = (uint32_t)(w.key >> 32);
-  best.n_valid = (uint32_t)w.n_valid;
-  if (best.best_count) {
-    best.best_index = 0xFFFFFFFFull - (w.key & 0xFFFFFFFFull);
-    for (int j = 0; j < mi.P; j++) best.best_params[j] = w.params[j];
-    for (int j = 0; j < mi.K; j++) best.best_subset[j] = w.subset[j];
-  }
-  // from here on: lsqr_ransac's loop, first round done
-  uint64_t num_tries = all_tries, done = H0, round = 1024;
-  bool perfect = false;
-  if (best.best_count) {
-    if (best.best_count == N) perfect = true;   // RANSAC.hxx:104-105
-    else num_tries = tries_after(best.best_count, N, mi.K, numerator, all_tries);
-  }
-  while (!perfect && done < num_tries) {
-    lsqr_score_args a{};
-    a.sampler = LSQR_SAMPLE_PHILOX; a.precision = precision; a.seed = seed; a.first = done;
-    a.count = std::min<uint64_t>(round, num_tries - done);
-    lsqr_score_result r{};
-    if (int rc = score_impl(ctx, &a, &r)) return rc;
-    dev_ms += r.score_ms;
-    done += a.count;
-    if (r.best_count > best.best_count) {  // strict '>' : RANSAC.hxx:100
-      best = r;
-      if (best.best_count == N) break;
-      num_tries = tries_after(best.best_count, N, mi.K, numerator, all_tries);
-    }
-    round = std::min<uint64_t>(round * 4, (uint64_t)1 << 20);
-  }
-  res->tries = done;
-  int rc = finish_ransac(ctx, best, out_mask, res);
-  res->device_ms = dev_ms + ctx->refine_kernel_ms;
-  return rc;
+  lsqr_score_result r0{};
+  decode_winner(*ctx->winner_pin, 0, mi, &r0);
+  r0.score_ms = ms0;   // includes the upload it overlaps
+  st.take(r0, H0);
+  if (int rc = ransac_rounds(ctx, precision, seed, 1024, st)) return rc;
+  return finish_ransac(ctx, st.best, st.done, st.dev_ms, out_mask, res);
 }
 
 // problems [p0, p1) of a batch (offsets are absolute record offsets into `data`)
@@ -1011,23 +991,10 @@ int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint6
   // pageable memory, as lsqr_upload does) on the copy stream; each chunk's problems are solved as soon as it has landed, so the
   // kernel hides behind the copy of the chunks that follow (65 536 x 256 3-D points: 403 MB of upload against 2.3 ms of kernel).
   const size_t rec_bytes = (size_t)mi.D * sizeof(double);
-  const bool pinned = is_pinned(data + base * mi.D);
-  const uint64_t chunk_rec = std::max<uint64_t>((pinned ? (16u << 20) : (4u << 20)) / rec_bytes, 1);
-  const size_t ring_bytes = (size_t)chunk_rec * rec_bytes;
-  if (!pinned) {
-    if (ctx->up_pin_bytes < ring_bytes) {
-      for (int i = 0; i < lsqr_ctx::kRing; i++) { if (ctx->up_pin[i]) cudaFreeHost(ctx->up_pin[i]); ctx->up_pin[i] = nullptr; }
-      ctx->up_pin_bytes = 0;
-      for (int i = 0; i < lsqr_ctx::kRing; i++) CK(cudaMallocHost((void**)&ctx->up_pin[i], ring_bytes));
-      ctx->up_pin_bytes = ring_bytes;
-    }
-    CK(cudaStreamSynchronize(ctx->copy_stream));   // an earlier upload may still be reading the pinned ring
-    if (!ctx->copier) ctx->copier.reset(new HostCopier(host_copy_threads(ctx->world > 1 && ctx->comm ? ctx->world : 1)));
-  }
-  CK(cudaEventRecord(ctx->up_land[7], s));           // the copy stream must not run ahead of work still reading bt_data
-  CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->up_land[7], 0));
+  StagedCopy up{ctx, is_pinned(data + base * mi.D)};
+  const uint64_t chunk_rec = std::max<uint64_t>((up.pinned ? (16u << 20) : (4u << 20)) / rec_bytes, 1);
+  if (int rc = up.start((size_t)chunk_rec * rec_bytes)) return rc;
   std::vector<cudaEvent_t> tev;                      // kernel time = sum over the chunks' launches
-  int ring = 0, land = 0;
   // copies go in pieces of chunk_rec records; a launch covers the problems of ~32 MB of them (several thousand small problems:
   // enough thread blocks to fill the GPU -- launches of one copy piece each, ~650 blocks, tripled the kernel time)
   const uint64_t launch_rec = std::max<uint64_t>(chunk_rec, (32u << 20) / rec_bytes);
@@ -1037,24 +1004,9 @@ int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint6
     const uint64_t rec0 = offsets[q0] - base, nrec = offsets[q1] - offsets[q0];
     for (uint64_t c0 = 0; c0 < nrec; c0 += chunk_rec) {
       const uint64_t cn = std::min<uint64_t>(chunk_rec, nrec - c0);
-      const double* src = data + (offsets[q0] + c0) * mi.D;
-      double* dst = ctx->bt_data + (rec0 + c0) * mi.D;
-      if (!pinned) {
-        const int b = ring % lsqr_ctx::kRing;
-        if (ring >= lsqr_ctx::kRing) CK(cudaEventSynchronize(ctx->up_ev[b]));   // the copy that used this buffer has finished
-        ring++;
-        ctx->copier->copy(ctx->up_pin[b], src, cn * rec_bytes);
-        CK(cudaMemcpyAsync(dst, ctx->up_pin[b], cn * rec_bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
-        CK(cudaEventRecord(ctx->up_ev[b], ctx->copy_stream));
-      } else {
-        CK(cudaMemcpyAsync(dst, src, cn * rec_bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
-      }
+      if (int rc = up.put(ctx->bt_data + (rec0 + c0) * mi.D, data + (offsets[q0] + c0) * mi.D, cn * rec_bytes)) return rc;
     }
-    if (nrec) {
-      cudaEvent_t landed = ctx->up_land[land++ % 7];
-      CK(cudaEventRecord(landed, ctx->copy_stream));
-      CK(cudaStreamWaitEvent(s, landed, 0));
-    }
+    if (nrec) if (int rc = up.landed()) return rc;
     BatchArgs ba{};
     ba.model = ctx->model; ba.exhaustive = exhaustive; ba.precision = use32 ? 1 : 0; ba.tries = max_tries; ba.prob = prob; ba.seed = seed;
     ba.data = ctx->bt_data + rec0 * mi.D; ba.offsets = ctx->bt_off + (q0 - p0); ba.n_problems = (uint32_t)(q1 - q0); ba.max_n = max_n;
@@ -1278,14 +1230,14 @@ int lsqr_set_estimator(lsqr_ctx* ctx, int model, double delta, double aux, int l
 
 int lsqr_upload(lsqr_ctx* ctx, const void* aos, size_t n, size_t stride_bytes) {
   if (!ctx) return LSQR_ERR_ARG;
-  if (ctx->group) return group_run(ctx, [&](lsqr_ctx* k, int) { return upload_to(k, k->main, aos, n, stride_bytes, false, true); });
-  return upload_to(ctx, ctx->main, aos, n, stride_bytes, false, true);
+  if (ctx->group) return group_run(ctx, [&](lsqr_ctx* k, int) { return upload_to(k, k->main, aos, n, stride_bytes, false); });
+  return upload_to(ctx, ctx->main, aos, n, stride_bytes, false);
 }
 int lsqr_upload_device(lsqr_ctx* ctx, const double* dev_packed, size_t n) {
   if (!ctx) return LSQR_ERR_ARG;
   if (ctx->group) return fail(ctx, LSQR_ERR_ARG, "a device buffer belongs to one GPU; upload host memory to a multi-GPU group");
   if (ctx->model < 0) return fail(ctx, LSQR_ERR_STATE, "lsqr_set_estimator must be called first");
-  return upload_to(ctx, ctx->main, dev_packed, n, sizeof(double) * model_info(ctx->model).D, true, false);
+  return upload_to(ctx, ctx->main, dev_packed, n, sizeof(double) * model_info(ctx->model).D, true);
 }
 
 int lsqr_set_shard(lsqr_ctx* ctx, int rank, int world, lsqr_allreduce_max_u64_fn max_fn, lsqr_allreduce_sum_f64_fn sum_fn, void* user) {
@@ -1335,7 +1287,7 @@ int lsqr_get_mask_bits(lsqr_ctx* ctx, uint32_t* out_words) {
     lsqr_ctx* ctx = k;   // for CK
     if (!k->main.mask_valid) return fail(k, LSQR_ERR_STATE, "no consensus set stored");
     uint32_t b, e;
-    shard_range(k, k->main.n, &b, &e);
+    shard_range(k, k->main, &b, &e);
     if (e <= b) return LSQR_OK;
     CK(cudaSetDevice(k->device));
     const size_t w0 = b / 32, w1 = ((size_t)e + 31) / 32;
@@ -1480,13 +1432,8 @@ int lsqr_least_squares(lsqr_ctx* ctx, const double* packed, size_t n, double* ou
   *n_params = 0;
   if (n < (size_t)mi.K && ctx->model != RAY) return LSQR_OK;  // size guards, e.g. PlaneParametersEstimator.hxx:133-134
   if (n == 0) return LSQR_OK;
-  // single-GPU by construction: a direct estimator call is not part of a sharded compute()
-  const int world = ctx->world, rank = ctx->rank;
-  ctx->world = 1; ctx->rank = 0;
-  int rc = upload_to(ctx, ctx->scratch, packed, n, sizeof(double) * mi.D, false, false);
-  if (!rc) rc = refine_impl(ctx, ctx->scratch, 0, out_params, n_params);
-  ctx->world = world; ctx->rank = rank;
-  return rc;
+  if (int rc = upload_to(ctx, ctx->scratch, packed, n, sizeof(double) * mi.D, false)) return rc;
+  return refine_impl(ctx, ctx->scratch, 0, out_params, n_params);
 }
 
 int lsqr_weighted_least_squares(lsqr_ctx* ctx, const double* packed, size_t n, const double* weights, double* out_params, int* n_params) {
@@ -1495,13 +1442,9 @@ int lsqr_weighted_least_squares(lsqr_ctx* ctx, const double* packed, size_t n, c
   if (ctx->model != ABSOR) return fail(ctx, LSQR_ERR_ARG, "weighted least squares exists for the absolute-orientation estimator only");
   *n_params = 0;
   if (n < 3) return LSQR_OK;   // AbsoluteOrientationParametersEstimator.cxx:214-215
-  const int world = ctx->world, rank = ctx->rank;
-  ctx->world = 1; ctx->rank = 0;
-  int rc = upload_to(ctx, ctx->scratch, packed, n, sizeof(double) * 6, false, false);
-  ctx->world = world; ctx->rank = rank;
-  if (rc) return rc;
+  if (int rc = upload_to(ctx, ctx->scratch, packed, n, sizeof(double) * 6, false)) return rc;
   cudaStream_t s = ctx->stream;
-  if (int rc2 = ensure(ctx, &ctx->weights_dev, &ctx->weights_cap, n)) return rc2;
+  if (int rc = ensure(ctx, &ctx->weights_dev, &ctx->weights_cap, n)) return rc;
   CK(cudaMemcpyAsync(ctx->weights_dev, weights, sizeof(double) * n, cudaMemcpyHostToDevice, s));
   const DataView dv = ctx->scratch.view();
   launch_weighted_absor_moments(dv, ctx->weights_dev, ctx->rb, s);
@@ -1546,10 +1489,9 @@ int lsqr_bench_refine_pass(lsqr_ctx* ctx, const double* params, int reps, double
   const ModelInfo mi = model_info(ctx->model);
   CK(cudaSetDevice(ctx->device));
   cudaStream_t s = ctx->stream;
-  for (int j = 0; j < mi.P; j++) ctx->pin[32 + j] = params[j];
-  CK(cudaMemcpyAsync(ctx->small_dev + kSmIn, ctx->pin + 32, sizeof(double) * mi.P, cudaMemcpyHostToDevice, s));
+  if (int rc = put_params(ctx, params)) return rc;
   uint32_t b, e;
-  shard_range(ctx, ds.n, &b, &e);
+  shard_range(ctx, ds, &b, &e);
   ctx->rb.maskbits = ds.maskbits;
   ctx->rb.maskbytes = nullptr;
   launch_mask_moments(ctx->model, ds.view(), b, e, ctx->small_dev + kSmIn, 1, nullptr, ctx->cfg, ctx->rb, s);   // warm-up

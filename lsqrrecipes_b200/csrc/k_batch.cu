@@ -87,7 +87,7 @@ __global__ void __launch_bounds__(256) batch_kernel(BatchArgs a, EstCfg cfg, int
   __shared__ double sh_ctr[kMaxDim];
   if (use32) {
     __syncthreads();
-    if (threadIdx.x < (uint32_t)kMaxDim) sh_ctr[threadIdx.x] = (threadIdx.x < (uint32_t)D && n > 0 && centred_comp(M, (int)threadIdx.x)) ? pts[threadIdx.x * ldp] : 0.0;
+    if (threadIdx.x < (uint32_t)kMaxDim) sh_ctr[threadIdx.x] = (threadIdx.x < (uint32_t)D && n > 0 && centred_component(M, (int)threadIdx.x)) ? pts[threadIdx.x * ldp] : 0.0;
     __syncthreads();
     const uint32_t npad = (n + 1u) & ~1u;
     for (uint32_t i = threadIdx.x; i < npad * D; i += blockDim.x) {

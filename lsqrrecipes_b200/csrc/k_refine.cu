@@ -128,7 +128,7 @@ __global__ void __launch_bounds__(MMCfg<M, LM>::THREADS, 1) mask_moments_kernel(
   // row's critical path)
   double ctr[D];
 #pragma unroll
-  for (int d = 0; d < D; d++) ctr[d] = centred_comp(M, d) ? dv.center[d] : 0.0;
+  for (int d = 0; d < D; d++) ctr[d] = centred_component(M, d) ? dv.center[d] : 0.0;
   double lmx[LM ? Mom<M>::NPLM : 1] = {0};
   if (LM) {
     // the phase selects the evaluation point: x or the trial point

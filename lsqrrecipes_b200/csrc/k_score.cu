@@ -50,17 +50,6 @@ __device__ __forceinline__ void tma_bulk_g2s(void* dst, const void* src, uint32_
 // Ingest: AoS records -> SoA fp64 (reference arithmetic) + SoA fp32 of x - c (fast mode), one pass, chunk by chunk so
 // that it overlaps the host-to-device copy (and, with several GPUs, the all-gather) of the chunks behind it.
 // ---------------------------------------------------------------------------------------
-// Which components are positions (get centred) for each model; directions / rotations are not.
-__host__ __device__ inline bool centred_component(int model, int d) {
-  switch (model) {
-    case RAY: return d < 3;
-    case PIVOT: return d >= 9;
-    case USXW: return d >= 9 && d < 12;       // t2; rotation entries and pixel coordinates stay
-    case USCP: return false;                  // t2 and p enter as p - t2 with no free translation to absorb a shift
-    default: return model_family(model) != FAM_DENSE;   // rows of a linear system: a shift would change the solution
-  }
-}
-
 // The shift c: per-component mean of the first `count` records (count <= kCenterSample), fixed-order tree sum.  c only
 // conditions the arithmetic (fp32 copy of x - c, moments of x - c); any point near the data does, and a prefix is known
 // as soon as the first chunk has landed.

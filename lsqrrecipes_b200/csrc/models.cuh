@@ -78,6 +78,16 @@ __host__ __device__ constexpr ModelInfo model_info(int m) {
   }
   return {0, 0, 0, 0, 0};
 }
+// Which components are positions (shifted by the centre c at ingest and in the refine moments); directions / rotations are not.
+__host__ __device__ inline bool centred_component(int model, int d) {
+  switch (model) {
+    case RAY: return d < 3;
+    case PIVOT: return d >= 9;
+    case USXW: return d >= 9 && d < 12;       // t2; rotation entries and pixel coordinates stay
+    case USCP: return false;                  // t2 and p enter as p - t2 with no free translation to absorb a shift
+    default: return model_family(model) != FAM_DENSE;   // rows of a linear system: a shift would change the solution
+  }
+}
 template <int M> struct Model {
   static constexpr int D = model_info(M).D, P = model_info(M).P, K = model_info(M).K, HQ = model_info(M).HQ, Q32 = model_info(M).Q32;
   static constexpr int FAM = model_family(M), DIM = model_dim(M);
@@ -737,13 +747,23 @@ LSQR_DENSE_N_LIST(LSQR_DEF_)
 // Subset generation
 // ---------------------------------------------------------------------------------------
 
+// high 32 bits of the 64-bit product a * b
+__host__ __device__ __forceinline__ uint32_t mulhi32(uint32_t a, uint32_t b) {
+#ifdef __CUDA_ARCH__
+  return __umulhi(a, b);
+#else
+  return (uint32_t)(((uint64_t)a * (uint64_t)b) >> 32);
+#endif
+}
+
 // Philox4x32-10 (Salmon et al., SC'11): counter-based, so hypothesis h's subset depends only
-// on (seed, h) -- independent of how hypotheses are split over thread blocks or GPUs.
-__device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
+// on (seed, h) -- independent of how hypotheses are split over thread blocks or GPUs, or of
+// whether the host draws it (compute() fetches the records of its first round ahead of the upload).
+__host__ __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
 #pragma unroll
   for (int r = 0; r < 10; r++) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, ctr.x), lo0 = 0xD2511F53u * ctr.x;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, ctr.z), lo1 = 0xCD9E8D57u * ctr.z;
+    const uint32_t hi0 = mulhi32(0xD2511F53u, ctr.x), lo0 = 0xD2511F53u * ctr.x;
+    const uint32_t hi1 = mulhi32(0xCD9E8D57u, ctr.z), lo1 = 0xCD9E8D57u * ctr.z;
     ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
     key.x += 0x9E3779B9u; key.y += 0xBB67AE85u;
   }
@@ -753,7 +773,7 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
 // K distinct indices in [0, n), in draw order (the reference also hands estimate() its subset
 // in draw order, RANSAC.hxx:56-68).  Draw j picks uniformly among the n-j indices not yet taken.
 template <int K>
-__device__ __forceinline__ void sample_subset(uint64_t gidx, uint64_t seed, uint32_t n, int32_t* out) {
+__host__ __device__ __forceinline__ void sample_subset(uint64_t gidx, uint64_t seed, uint32_t n, int32_t* out) {
   constexpr int NB = (K + 3) / 4;   // one counter block per four draws
   uint32_t rnd[4 * NB];
 #pragma unroll
@@ -764,7 +784,7 @@ __device__ __forceinline__ void sample_subset(uint64_t gidx, uint64_t seed, uint
   uint32_t sorted[K];
 #pragma unroll
   for (int j = 0; j < K; j++) {
-    uint32_t v = __umulhi(rnd[j], n - j);  // uniform in [0, n-j)
+    uint32_t v = mulhi32(rnd[j], n - j);  // uniform in [0, n-j)
 #pragma unroll
     for (int i = 0; i < j; i++) if (v >= sorted[i]) v++;  // skip taken indices, ascending
     out[j] = (int32_t)v;

@@ -227,16 +227,6 @@ template <> __device__ __forceinline__ void accumulate<USCP>(const double* q, do
 // calibrated pointer: the same rows with the measured tip position p (q[14..16]) in the place of t1 and no unknown for it
 __device__ __forceinline__ void acc_uscp_lm(const double* q, const double* x, double* acc) { acc_us_lm_rows<0>(q, x, q + 14, acc); }
 
-__host__ __device__ inline bool centred_comp(int model, int d) {
-  switch (model) {
-    case RAY: return d < 3;
-    case PIVOT: return d >= 9;
-    case USXW: return d >= 9 && d < 12;
-    case USCP: return false;
-    default: return model_family(model) != FAM_DENSE;
-  }
-}
-
 // ---------------------------------------------------------------------------------------
 // moments -> parameters
 // ---------------------------------------------------------------------------------------

@@ -173,6 +173,34 @@ def test_weighted_horn_vs_oracle(port):
     assert same_up_to_sign(prm, port.weighted_absor(data, w), SIGN_IDX["absor"], REFINE_TOL)
 
 
+def test_direct_least_squares_ignore_the_shard():
+    """lsqr_least_squares / lsqr_weighted_least_squares fit all the data they are given on one device: on rank 0 of 2 (caller
+    hooks, lsqr_set_shard) they return exactly what an unsharded context returns and never call the all-reduce hooks."""
+    calls = []
+
+    def max_fn(user, dev, stream):
+        calls.append("max")
+        return 0
+
+    def sum_fn(user, dev, count, stream):
+        calls.append("sum")
+        return 0
+
+    w = np.random.default_rng(8).uniform(0.0, 2.0, 20000)
+    for name in ("plane3", "sphere3", "absor"):   # sphere3: the geometric fit's Levenberg-Marquardt passes reduce too
+        data, _ = synth.GENERATORS[name](20000, seed=17)
+        one, sharded = Engine(name, synth.DELTAS[name]), Engine(name, synth.DELTAS[name])
+        sharded.set_shard(0, 2, max_fn, sum_fn)
+        want = one.least_squares(data)
+        assert len(want) and np.array_equal(sharded.least_squares(data), want), name
+        if name == "absor":
+            want = one.weighted_least_squares(data, w)
+            assert len(want) and np.array_equal(sharded.weighted_least_squares(data, w), want)
+        one.close()
+        sharded.close()
+    assert calls == []
+
+
 def test_crosswire_operator_interface(port):
     """SingleUnknownPointTargetUSCalibrationParametersEstimator through the Python mirror of the reference API:
     estimate() wants exactly four data (.cxx:21-22), ANALYTIC / ITERATIVE least squares, RANSAC::compute."""
