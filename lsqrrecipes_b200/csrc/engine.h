@@ -2,6 +2,9 @@
 #pragma once
 #include <cstddef>
 #include <cstdint>
+#include <map>
+#include <mutex>
+#include <utility>
 #include <cuda_runtime.h>
 
 #include "../../include/lsqr_b200.h"
@@ -34,6 +37,41 @@ struct WinnerRecord {
   int32_t subset[LSQR_MAX_SUBSET];
   double params[LSQR_MAX_PARAMS];
 };
+
+// ---- launch set-up shared by the kernel translation units -------------------------------
+// Point chunks (grid.y) of the tiled consensus kernels: enough (hypothesis block x chunk) work items for ~16 CTAs per SM,
+// chunks of at least 4 tiles, at most 65535 chunks, none of them empty.
+struct TileChunks { uint32_t chunks, tiles_per_chunk; };
+inline TileChunks plan_tile_chunks(uint32_t tiles_total, uint32_t hyp_blocks, int num_sms) {
+  uint32_t want = (uint32_t)num_sms * 16;
+  uint32_t chunks = (want + hyp_blocks - 1) / hyp_blocks;
+  uint32_t max_chunks = (tiles_total + 3) / 4;
+  if (max_chunks == 0) max_chunks = 1;
+  if (chunks > max_chunks) chunks = max_chunks;
+  if (chunks > 65535) chunks = 65535;
+  if (chunks == 0) chunks = 1;
+  const uint32_t tiles_per_chunk = (tiles_total + chunks - 1) / chunks;
+  chunks = (tiles_total + tiles_per_chunk - 1) / tiles_per_chunk;
+  return {chunks, tiles_per_chunk};
+}
+
+// Per-device tables of the launchers (constant-bank lock, occupancy) hold this many devices; device ids alias beyond it.
+constexpr int kMaxDevices = 64;
+
+// Lets `kernel` launch with up to `bytes` of dynamic shared memory on the current device (more than 48 KB needs the limit
+// raised).  The limit belongs to one kernel on one device, so the table is keyed by both: instantiations with the same
+// signature are different kernels, and a multi-device context launches from one thread per device.
+inline void allow_dynamic_smem(const void* kernel, size_t bytes) {
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> raised;
+  int dev = 0;
+  cudaGetDevice(&dev);
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& limit = raised[{kernel, dev}];
+  if (bytes <= limit) return;
+  if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) == cudaSuccess) limit = bytes;
+}
+template <class Kernel> void allow_dynamic_smem(Kernel* kernel, size_t bytes) { allow_dynamic_smem(reinterpret_cast<const void*>(kernel), bytes); }
 
 // ---- k_score.cu -------------------------------------------------------------------------
 // c = mean of the first `count` AoS records (device buffer), per centred component -> center_dev[kMaxDim].

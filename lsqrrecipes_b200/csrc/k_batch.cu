@@ -273,7 +273,7 @@ int launch_batch(const BatchArgs& a, const EstCfg& cfg, int ls_type, cudaStream_
 #define CALL(MM)                                                                                  \
   {                                                                                               \
     auto kern = batch_kernel<MM>;                                                                 \
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);          \
+    allow_dynamic_smem(kern, smem);                                                               \
     kern<<<a.n_problems, threads, smem, s>>>(a, cfg, ls_type, group);                            \
   }
 #define LSQR_DEF_(ID, DIM) case ID: CALL(ID) break;

@@ -11,7 +11,7 @@
 //     the 64 KB constant bank, a point pair is a UNIFORM-register operand (LDCU -> `FFMA2 R, R.F32, UR.F32x2, R.F32x2`) and an
 //     FFMA2 reads 2-3 registers instead of the 5-6 it reads when the pair comes out of shared memory.
 //   * Small requests (adaptive RANSAC rounds, tests) take consensus32_kernel: point tiles staged by TMA bulk copies into a
-//     2-deep shared-memory ring (as in k_score.cu), pairs through LDS.128.
+//     2-deep shared-memory ring (TileRing, bulk_copy.cuh), pairs through LDS.128.
 //   * Counting, three ALU instructions per two residuals in the hot kernel:
 //       - hyperplanes, dense systems, hypersphere family: CARRY CHAIN (count_carry) -- the residual arrives shifted (the hoisted
 //         constant carries +delta; hypersphere: t' = d^2 - (r - delta)^2), inlier <=> bits(s') < bits(window) unsigned (window 2 delta,
@@ -27,32 +27,12 @@
 // Tensor cores are deliberately unused: contraction depth <= 8 (BASELINE.json north_star: <= 4 for its estimators), and
 // TF32 / bf16 operands would destroy a residual of 0.5 on coordinates of 1000.
 #include "engine.h"
+#include "bulk_copy.cuh"
 #include "fast_forms.cuh"
 
 #include <mutex>
 
 namespace lsqr {
-
-// ---- mbarrier / TMA-bulk helpers ---------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbarrier_init(uint64_t* bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(bar)), "r"(count)); }
-__device__ __forceinline__ void mbarrier_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbarrier_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_addr(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_load_1d(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_addr(dst)), "l"(src), "r"(bytes),
-               "r"(smem_addr(bar))
-               : "memory");
-}
 
 template <int M>
 __global__ void hoist32_kernel(const double* __restrict__ hyp64, size_t hld, uint32_t H, DataView dv, EstCfg cfg, float* __restrict__ hyp32) {
@@ -106,10 +86,7 @@ __global__ void __launch_bounds__(THREADS) consensus32_kernel(const float* __res
                                                                const float* __restrict__ hyp, size_t hld, uint32_t H, float delta, float delta2,
                                                                uint32_t* __restrict__ counts) {
   constexpr int D = Model<M>::D, Q = Model<M>::Q32;
-  constexpr uint32_t kTileBytes = (uint32_t)(TILE * sizeof(float));
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  float* tile0 = reinterpret_cast<float*>(smem_raw);
-  float* tile1 = tile0 + D * TILE;
   __shared__ __align__(8) uint64_t bars[2];
 
   const int tid = threadIdx.x;
@@ -133,21 +110,10 @@ __global__ void __launch_bounds__(THREADS) consensus32_kernel(const float* __res
 
   const uint32_t t0 = blockIdx.y * tiles_per_chunk;
   const uint32_t t1 = min(t0 + tiles_per_chunk, tiles_total);
-  if (tid == 0) { mbarrier_init(&bars[0], 1); mbarrier_init(&bars[1], 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-  __syncthreads();
-  auto issue = [&](uint32_t t, int buf) {
-    float* dst = buf ? tile1 : tile0;
-    mbarrier_expect_tx(&bars[buf], kTileBytes * D);
-#pragma unroll
-    for (int d = 0; d < D; d++) tma_load_1d(dst + d * TILE, soa + (size_t)d * ld + (size_t)t * TILE, kTileBytes, &bars[buf]);
-  };
-  if (tid == 0 && t0 < t1) issue(t0, 0);
-  uint32_t phase0 = 0, phase1 = 0;
+  TileRing<D, TILE, float> ring{soa, ld, t0, t1, reinterpret_cast<float*>(smem_raw), bars, tid};
+  ring.start();
   for (uint32_t t = t0; t < t1; t++) {
-    const int buf = (t - t0) & 1;
-    if (tid == 0 && t + 1 < t1) issue(t + 1, buf ^ 1);
-    if (buf) { mbarrier_wait(&bars[1], phase1); phase1 ^= 1; } else { mbarrier_wait(&bars[0], phase0); phase0 ^= 1; }
-    const float* tl = buf ? tile1 : tile0;
+    const float* tl = ring.wait(t);
 #pragma unroll 1
     for (int i = 0; i < TILE; i += 2 * PPI) {
       f2 x[PPI][D];
@@ -176,7 +142,7 @@ __global__ void __launch_bounds__(THREADS) consensus32_kernel(const float* __res
         }
       }
     }
-    __syncthreads();  // everyone is done with this buffer before it is refilled
+    ring.release();
   }
 #pragma unroll
   for (int r = 0; r < R; r++) {
@@ -191,23 +157,12 @@ template <int M, int R, int THREADS, int TILE, int PPI>
 static int run_consensus32(const DataView& dv, const float* hyp, size_t hld, uint32_t H, const EstCfg& cfg, uint32_t* counts, int num_sms, cudaStream_t s) {
   const uint32_t tiles_total = (uint32_t)(dv.span / TILE);
   const uint32_t hyp_blocks = (H + THREADS * R - 1) / (THREADS * R);
-  uint32_t want = (uint32_t)num_sms * 16;  // ~16 work items per SM for load balance
-  uint32_t chunks = (want + hyp_blocks - 1) / hyp_blocks;
-  uint32_t max_chunks = (tiles_total + 3) / 4;
-  if (max_chunks == 0) max_chunks = 1;
-  if (chunks > max_chunks) chunks = max_chunks;
-  if (chunks > 65535) chunks = 65535;
-  if (chunks == 0) chunks = 1;
-  const uint32_t tiles_per_chunk = (tiles_total + chunks - 1) / chunks;
-  chunks = (tiles_total + tiles_per_chunk - 1) / tiles_per_chunk;
+  const TileChunks plan = plan_tile_chunks(tiles_total, hyp_blocks, num_sms);
   const size_t smem = 2 * (size_t)Model<M>::D * TILE * sizeof(float);
   auto kern = consensus32_kernel<M, R, THREADS, TILE, PPI>;
-  // the attribute is per device (a multi-device context launches the same kernel on every GPU of the process)
-  static bool attr_set[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!attr_set[dev & 63]) { cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); attr_set[dev & 63] = true; }
-  kern<<<dim3(hyp_blocks, chunks), THREADS, smem, s>>>(dv.soa32, dv.ld, tiles_total, tiles_per_chunk, hyp, hld, H, (float)cfg.delta, (float)cfg.delta2, counts);
+  allow_dynamic_smem(kern, smem);
+  kern<<<dim3(hyp_blocks, plan.chunks), THREADS, smem, s>>>(dv.soa32, dv.ld, tiles_total, plan.tiles_per_chunk, hyp, hld, H, (float)cfg.delta, (float)cfg.delta2,
+                                                             counts);
   return 1;
 }
 
@@ -220,7 +175,7 @@ static int run_consensus32(const DataView& dv, const float* hyp, size_t hld, uin
 constexpr int kCbFloats = 16320;              // 65280 B of the 64 KB bank
 constexpr uint32_t kCbMinHyps = 98304;        // below this the per-launch overhead outweighs the gain
 __constant__ float4 c_tile[kCbFloats / 4];
-static std::mutex g_cb_mutex[16];             // the bank is per device, not per context
+static std::mutex g_cb_mutex[kMaxDevices];    // the bank is per device, not per context
 
 #ifndef LSQR_CB_MINBLOCKS
 #define LSQR_CB_MINBLOCKS 5
@@ -369,16 +324,16 @@ static int run_consensus_cb(const DataView& dv, const float* hyp, size_t hld, ui
   auto kern = consensus_cb_kernel<M, R, THREADS, PPI>;
   int dev = 0;
   cudaGetDevice(&dev);
-  static int occ[16] = {0};
-  if (!occ[dev & 15]) {
+  static int occ[kMaxDevices] = {0};
+  if (!occ[dev % kMaxDevices]) {
     int o = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, kern, THREADS, 0) != cudaSuccess || o < 1) o = 4;
-    occ[dev & 15] = o;
+    occ[dev % kMaxDevices] = o;
   }
   void* bank = nullptr;
   if (cudaGetSymbolAddress(&bank, c_tile) != cudaSuccess) return -1;
   const uint32_t hyp_blocks = (H + THREADS * R - 1) / (THREADS * R);
-  const uint32_t slots = (uint32_t)num_sms * (uint32_t)occ[dev & 15];
+  const uint32_t slots = (uint32_t)num_sms * (uint32_t)occ[dev % kMaxDevices];
   // sub-chunks per launch: fill the last wave (the launches of one request serialise on the bank)
   constexpr bool kRaw = Eval<M>::kHasAbsForm && !Eval<M>::kShifted;
   auto pick_sub = [&](uint32_t npts) {
@@ -394,7 +349,7 @@ static int run_consensus_cb(const DataView& dv, const float* hyp, size_t hld, ui
     }
     return best_sub;
   };
-  std::lock_guard<std::mutex> lock(g_cb_mutex[dev & 15]);
+  std::lock_guard<std::mutex> lock(g_cb_mutex[dev % kMaxDevices]);
   int launches = 0;
   for (size_t base = 0; base < dv.span; base += cp) {
     const uint32_t npts = (uint32_t)((dv.span - base < cp) ? (dv.span - base) : cp);   // span is a multiple of 1024, cp of 16

@@ -12,33 +12,12 @@
 //
 // All position components are accumulated relative to dv.center (shift-invariant scatter / normal
 // equations), which keeps the fp64 sums well conditioned for coordinates far from the origin.
+#include "bulk_copy.cuh"
 #include "refine_common.cuh"
 
 namespace lsqr {
 
 int moments_count(int model, bool lm) { return n_moments(model, lm); }
-
-// ---- mbarrier / TMA-bulk helpers (SASS: SYNCS / UBLKCP) ------------------------------------
-__device__ __forceinline__ uint32_t mm_smem(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mm_bar_init(uint64_t* bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(mm_smem(bar)), "r"(count)); }
-__device__ __forceinline__ void mm_bar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mm_smem(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mm_bar_arrive(uint64_t* bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(mm_smem(bar)) : "memory"); }
-__device__ __forceinline__ void mm_bar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(mm_smem(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void mm_tma_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(mm_smem(dst)), "l"(src), "r"(bytes),
-               "r"(mm_smem(bar))
-               : "memory");
-}
 
 // Blocking of the streaming pass: one persistent CTA per SM walks tiles of TILE data; a tile is D rows of TILE doubles in
 // shared memory, filled by D bulk copies (cp.async.bulk, one mbarrier per stage), STAGES tiles deep.  The bytes in flight per
@@ -102,15 +81,15 @@ __global__ void __launch_bounds__(MMCfg<M, LM>::THREADS, 1) mask_moments_kernel(
   auto issue = [&](uint32_t k, uint32_t s) {   // tile number k of this CTA into stage s
     const size_t base = (size_t)(first + k * gridDim.x) * TILE;
     double* dst = ring + (size_t)s * D * TILE;
-    mm_bar_expect_tx(&full_bar[s], (uint32_t)C::TILE_BYTES);
+    mbar_expect_tx(&full_bar[s], (uint32_t)C::TILE_BYTES);
 #pragma unroll
-    for (int d = 0; d < D; d++) mm_tma_g2s(dst + d * TILE, dv.soa64 + (size_t)d * dv.ld + base, TILE * 8, &full_bar[s]);
+    for (int d = 0; d < D; d++) bulk_g2s(dst + d * TILE, dv.soa64 + (size_t)d * dv.ld + base, TILE * 8, &full_bar[s]);
   };
   // the first tiles are on their way before anything else is set up
   if (tid == 0) {
 #pragma unroll
-    for (int s = 0; s < STAGES; s++) { mm_bar_init(&full_bar[s], 1); mm_bar_init(&empty_bar[s], THREADS / 32); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < STAGES; s++) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], THREADS / 32); }
+    mbar_fence_init();
     for (uint32_t k = 0; k < (uint32_t)STAGES && k < n_mine; k++) issue(k, k);
   }
 
@@ -186,7 +165,7 @@ __global__ void __launch_bounds__(MMCfg<M, LM>::THREADS, 1) mask_moments_kernel(
   for (uint32_t k = 0; k < n_mine; k++) {
     const uint32_t base = (first + k * gridDim.x) * (uint32_t)TILE;
     const double* tile = ring + (size_t)s * D * TILE;
-    mm_bar_wait(&full_bar[s], parity);
+    mbar_wait(&full_bar[s], parity);
     double x[PPT][D];
 #pragma unroll
     for (int u = 0; u < PPT; u++) {
@@ -198,8 +177,8 @@ __global__ void __launch_bounds__(MMCfg<M, LM>::THREADS, 1) mask_moments_kernel(
     }
     // the stage is free as soon as every warp holds its data in registers; thread 0 refills it STAGES tiles ahead
     __syncwarp();
-    if (lane == 0) mm_bar_arrive(&empty_bar[s]);
-    if (tid == 0 && k + STAGES < n_mine) { mm_bar_wait(&empty_bar[s], parity); issue(k + STAGES, s); }
+    if (lane == 0) mbar_arrive(&empty_bar[s]);
+    if (tid == 0 && k + STAGES < n_mine) { mbar_wait(&empty_bar[s], parity); issue(k + STAGES, s); }
     const uint32_t s_next = (s + 1 == (uint32_t)STAGES) ? 0u : s + 1;
     parity ^= (s_next == 0u) ? 1u : 0u;
     s = s_next;
@@ -229,10 +208,7 @@ static void run_mask_moments(const DataView& dv, uint32_t begin, uint32_t end, c
                              const RefineBuffers& rb, cudaStream_t s) {
   using C = MMCfg<M, LM>;
   auto kern = mask_moments_kernel<M, MODE, LM>;
-  static bool attr_set[64] = {false};   // per device
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!attr_set[dev & 63]) { cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM); attr_set[dev & 63] = true; }
+  allow_dynamic_smem(kern, C::SMEM);
   kern<<<rb.blocks, C::THREADS, C::SMEM, s>>>(dv, begin, end, params_dev, lm_state, cfg, rb.maskbits, rb.maskbytes, rb.partials);
 }
 

@@ -6,7 +6,7 @@
 //     keeps R prepared hypotheses in registers for the whole kernel.
 //   * The point chunk is streamed through shared memory in SoA tiles of TILE points, staged by
 //     TMA bulk copies (cp.async.bulk ... mbarrier::complete_tx) in a 2-deep ring, one copy per
-//     component per tile, issued by one elected thread.
+//     component per tile, issued by one elected thread (TileRing, bulk_copy.cuh).
 //   * Inside a tile every thread reads the same point (shared-memory broadcast, vector loads of
 //     UNR consecutive points) and evaluates agree() for its R hypotheses.
 //   * Per-hypothesis counts go to global memory with one atomicAdd per (hypothesis, chunk).
@@ -14,37 +14,12 @@
 // mode lives in k_fast.cu.
 // Tensor cores are deliberately unused: the contraction depth is <= 4 (BASELINE.json north_star).
 #include "engine.h"
+#include "bulk_copy.cuh"
 #include "../../include/lsqr_b200.h"
 
 #include <cstdio>
 
 namespace lsqr {
-
-// ---------------------------------------------------------------------------------------
-// mbarrier / TMA-bulk helpers (sm_90+ PTX; SASS: SYNCS / UBLKCP)
-// ---------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)), "l"(src),
-               "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
 
 // ---------------------------------------------------------------------------------------
 // Ingest: AoS records -> SoA fp64 (reference arithmetic) + SoA fp32 of x - c (fast mode), one pass, chunk by chunk so
@@ -216,77 +191,50 @@ void launch_winner(const SolveArgs& a, const unsigned long long* key_dev, const 
 #undef CALL
 }
 
-// Traits binding the generic consensus kernel to one (model, precision).
-template <int M> struct Exact {
-  using real = double;
-  using thr_t = EstCfg;
-  static constexpr int D = Model<M>::D, NIN = Model<M>::P, HQ = Model<M>::HQ, UNR = 2;
-  __device__ static __forceinline__ void load(const double* raw, const EstCfg& t, double* hq) { prepare<M>(raw, t, hq); }
-  __device__ static __forceinline__ bool test(const double* hq, const double* x, const EstCfg& t) { return agree<M>(hq, x, t); }
-};
-template <class T, int R, int THREADS, int TILE>
-__global__ void __launch_bounds__(THREADS) consensus_kernel(const typename T::real* __restrict__ soa, size_t ld, uint32_t tiles_total, uint32_t tiles_per_chunk,
-                                                             const typename T::real* __restrict__ hyp, size_t hld, uint32_t H, typename T::thr_t thr,
+// UNR = 2 data per inner iteration: one LDS.128 per component
+template <int M, int R, int THREADS, int TILE>
+__global__ void __launch_bounds__(THREADS) consensus_kernel(const double* __restrict__ soa, size_t ld, uint32_t tiles_total, uint32_t tiles_per_chunk,
+                                                             const double* __restrict__ hyp, size_t hld, uint32_t H, EstCfg thr,
                                                              uint32_t* __restrict__ counts) {
-  using real = typename T::real;
-  constexpr int D = T::D, UNR = T::UNR;
-  constexpr uint32_t kTileBytes = (uint32_t)(TILE * sizeof(real));
+  constexpr int D = Model<M>::D, P = Model<M>::P, HQ = Model<M>::HQ, UNR = 2;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  real* tile0 = reinterpret_cast<real*>(smem_raw);
-  real* tile1 = tile0 + D * TILE;
   __shared__ __align__(8) uint64_t bars[2];
 
   const int tid = threadIdx.x;
   const uint32_t hbase = blockIdx.x * (THREADS * R);
-  real hq[R][T::HQ];
+  double hq[R][HQ];
   uint32_t cnt[R];
 #pragma unroll
   for (int r = 0; r < R; r++) {
     const uint32_t h = hbase + r * THREADS + tid;
-    real raw[T::NIN];
+    double raw[P];
 #pragma unroll
-    for (int j = 0; j < T::NIN; j++) raw[j] = (h < H) ? hyp[(size_t)j * hld + h] : (real)NAN;
-    T::load(raw, thr, hq[r]);
+    for (int j = 0; j < P; j++) raw[j] = (h < H) ? hyp[(size_t)j * hld + h] : (double)NAN;
+    prepare<M>(raw, thr, hq[r]);
     cnt[r] = 0;
   }
 
   const uint32_t t0 = blockIdx.y * tiles_per_chunk;
   const uint32_t t1 = min(t0 + tiles_per_chunk, tiles_total);
-  if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); fence_barrier_init(); }
-  __syncthreads();
-  auto issue = [&](uint32_t t, int buf) {
-    real* dst = buf ? tile1 : tile0;
-    mbar_expect_tx(&bars[buf], kTileBytes * D);
-#pragma unroll
-    for (int d = 0; d < D; d++) tma_bulk_g2s(dst + d * TILE, soa + (size_t)d * ld + (size_t)t * TILE, kTileBytes, &bars[buf]);
-  };
-  if (tid == 0 && t0 < t1) issue(t0, 0);
-  uint32_t phase0 = 0, phase1 = 0;
+  TileRing<D, TILE, double> ring{soa, ld, t0, t1, reinterpret_cast<double*>(smem_raw), bars, tid};
+  ring.start();
   for (uint32_t t = t0; t < t1; t++) {
-    const int buf = (t - t0) & 1;
-    if (tid == 0 && t + 1 < t1) issue(t + 1, buf ^ 1);
-    if (buf) { mbar_wait(&bars[1], phase1); phase1 ^= 1; } else { mbar_wait(&bars[0], phase0); phase0 ^= 1; }
-    const real* tl = buf ? tile1 : tile0;
+    const double* tl = ring.wait(t);
 #pragma unroll 1
     for (int i = 0; i < TILE; i += UNR) {
-      real x[UNR][D];
+      double x[UNR][D];
 #pragma unroll
       for (int d = 0; d < D; d++) {
-        if constexpr (sizeof(real) == 4) {
-          const float4 v = *reinterpret_cast<const float4*>(tl + d * TILE + i);
-          x[0][d] = v.x; x[1][d] = v.y; x[2][d] = v.z; x[3][d] = v.w;
-        } else {
-          const double2 v = *reinterpret_cast<const double2*>(tl + d * TILE + i);
-          x[0][d] = v.x; x[1][d] = v.y;
-        }
+        const double2 v = *reinterpret_cast<const double2*>(tl + d * TILE + i);
+        x[0][d] = v.x; x[1][d] = v.y;
       }
 #pragma unroll
       for (int r = 0; r < R; r++) {
 #pragma unroll
-        for (int u = 0; u < UNR; u++) cnt[r] += T::test(hq[r], x[u], thr) ? 1u : 0u;
+        for (int u = 0; u < UNR; u++) cnt[r] += agree<M>(hq[r], x[u], thr) ? 1u : 0u;
       }
     }
-    __syncthreads();  // everyone is done with this buffer before it is refilled
+    ring.release();
   }
 #pragma unroll
   for (int r = 0; r < R; r++) {
@@ -295,31 +243,15 @@ __global__ void __launch_bounds__(THREADS) consensus_kernel(const typename T::re
   }
 }
 
-template <class T, int R, int THREADS, int TILE>
-static int run_consensus(const typename T::real* soa, size_t ld, size_t span, const typename T::real* hyp, size_t hld, uint32_t H, const typename T::thr_t& thr,
-                         uint32_t* counts, int num_sms, cudaStream_t s) {
-  using real = typename T::real;
-  const uint32_t tiles_total = (uint32_t)(span / TILE);
+template <int M, int R, int THREADS, int TILE>
+static int run_consensus(const DataView& dv, const double* hyp, size_t hld, uint32_t H, const EstCfg& cfg, uint32_t* counts, int num_sms, cudaStream_t s) {
+  const uint32_t tiles_total = (uint32_t)(dv.span / TILE);
   const uint32_t hyp_blocks = (H + THREADS * R - 1) / (THREADS * R);
-  // enough (hypothesis block x point chunk) work items for ~16 CTAs per SM, chunks not below 4 tiles
-  uint32_t want = (uint32_t)num_sms * 16;
-  uint32_t chunks = (want + hyp_blocks - 1) / hyp_blocks;
-  uint32_t max_chunks = (tiles_total + 3) / 4;
-  if (max_chunks == 0) max_chunks = 1;
-  if (chunks > max_chunks) chunks = max_chunks;
-  if (chunks > 65535) chunks = 65535;
-  if (chunks == 0) chunks = 1;
-  const uint32_t tiles_per_chunk = (tiles_total + chunks - 1) / chunks;
-  chunks = (tiles_total + tiles_per_chunk - 1) / tiles_per_chunk;
-  const size_t smem = 2 * (size_t)T::D * TILE * sizeof(real);
-  auto kern = consensus_kernel<T, R, THREADS, TILE>;
-  // the attribute is per device (a multi-device context launches the same kernel on every GPU of the process)
-  static bool attr_set[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!attr_set[dev & 63]) { cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); attr_set[dev & 63] = true; }
-  dim3 grid(hyp_blocks, chunks);
-  kern<<<grid, THREADS, smem, s>>>(soa, ld, tiles_total, tiles_per_chunk, hyp, hld, H, thr, counts);
+  const TileChunks plan = plan_tile_chunks(tiles_total, hyp_blocks, num_sms);
+  const size_t smem = 2 * (size_t)Model<M>::D * TILE * sizeof(double);
+  auto kern = consensus_kernel<M, R, THREADS, TILE>;
+  allow_dynamic_smem(kern, smem);
+  kern<<<dim3(hyp_blocks, plan.chunks), THREADS, smem, s>>>(dv.soa64, dv.ld, tiles_total, plan.tiles_per_chunk, hyp, hld, H, cfg, counts);
   return 1;
 }
 
@@ -332,8 +264,8 @@ int launch_consensus(int model, int precision, const DataView& dv, const double*
   if (H == 0 || dv.n == 0) return 0;
   if (precision == 0) {
 #define CALL(MM)                                                                                                             \
-  if (H <= 4096) return run_consensus<Exact<MM>, 1, 128, 256>(dv.soa64, dv.ld, dv.span, hyp64, hld, H, cfg, counts, num_sms, s);       \
-  return run_consensus<Exact<MM>, (Model<MM>::HQ >= 12 ? 2 : LSQR_FP64_R), 128, 256>(dv.soa64, dv.ld, dv.span, hyp64, hld, H, cfg, counts, num_sms, s)
+  if (H <= 4096) return run_consensus<MM, 1, 128, 256>(dv, hyp64, hld, H, cfg, counts, num_sms, s);                                \
+  return run_consensus<MM, (Model<MM>::HQ >= 12 ? 2 : LSQR_FP64_R), 128, 256>(dv, hyp64, hld, H, cfg, counts, num_sms, s)
     LSQR_DISPATCH_MODEL(model, CALL)
 #undef CALL
   } else {

@@ -91,9 +91,9 @@ def test_constant_bank_kernels_read_their_points_through_uniform_registers(sass,
 
 
 def test_fp64_validation_kernel_compares_on_the_integer_alu(sass):
-    """consensus_kernel<Exact<PLANE3>, 4, 128, 256>: nine FP64-pipe instructions per evaluation (5 DADD + 4 DMUL as the reference
+    """consensus_kernel<PLANE3, 4, 128, 256>: nine FP64-pipe instructions per evaluation (5 DADD + 4 DMUL as the reference
     writes them, minus the leading `0 +`), the threshold test as a 64-bit integer compare (ISETP + ISETP.EX) -- no DSETP."""
-    ins = _one(sass, r"consensus_kernelINS_5ExactILi0EEELi4ELi128ELi256E")
+    ins = _one(sass, r"consensus_kernelILi0ELi4ELi128ELi256E")
     assert not [i for i in ins if i.startswith("DSETP")], "the squared-distance compare must not occupy the FP64 pipe"
     assert sum(i.startswith("DADD") for i in ins) == 40 and sum(i.startswith("DMUL") for i in ins) == 32   # 8 evaluations per iteration
     assert not [i for i in ins if i.startswith("DFMA")], "validation mode must not contract (the reference is built without FMA)"
