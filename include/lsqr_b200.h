@@ -167,7 +167,10 @@ typedef struct lsqr_score_args {
   uint64_t count;        /* H: number of hypotheses in this request (global, before sharding) */
   const int32_t* subsets;/* LSQR_SAMPLE_LIST: host int32 [H][k] */
   const double* params;  /* LSQR_SAMPLE_PARAMS: host double [H][P]; NaN row = degenerate */
-  uint32_t* out_counts;  /* optional host [H]: full inlier count per hypothesis (no early exit, RANSAC.hxx:239-244) */
+  uint32_t* out_counts;  /* optional host [H]: full inlier count per hypothesis (no early exit, RANSAC.hxx:239-244).  Without it,
+                            fp32 requests of at least 98304 hypotheses exit early (RANSAC.hxx:94): a hypothesis stops being
+                            scored once its inliers so far plus the data left cannot reach the full count of one already
+                            scored; the result is exactly that of the full pass, with less work on data with many inliers */
   double* out_params;    /* optional host [H][P]: estimate() output per hypothesis, NaN row if degenerate */
 } lsqr_score_args;
 
@@ -179,8 +182,11 @@ typedef struct lsqr_score_result {
   double best_params[LSQR_MAX_PARAMS];
   double score_ms;       /* device time of solve + consensus + arg-max (CUDA events) */
   double consensus_ms;   /* device time of the consensus kernel(s) alone */
+  uint64_t evals;        /* hypothesis x datum evaluations launched (this rank; H x N without the early exit) */
 } lsqr_score_result;
 
+/* Scores `count` hypotheses against the uploaded data and returns the winner (most inliers, lowest index on ties).  The
+ * winner is the same with and without out_counts; only the per-hypothesis counts need the full pass. */
 int lsqr_score(lsqr_ctx* ctx, const lsqr_score_args* args, lsqr_score_result* res);
 
 /* ---- consensus set + least-squares refine ------------------------------------------ */

@@ -46,7 +46,7 @@ class ScoreArgs(ctypes.Structure):
 class ScoreResult(ctypes.Structure):
     _fields_ = [("best_index", ctypes.c_uint64), ("best_count", ctypes.c_uint32), ("n_valid", ctypes.c_uint32),
                 ("best_subset", ctypes.c_int32 * 10), ("best_params", ctypes.c_double * 20),
-                ("score_ms", ctypes.c_double), ("consensus_ms", ctypes.c_double)]
+                ("score_ms", ctypes.c_double), ("consensus_ms", ctypes.c_double), ("evals", ctypes.c_uint64)]
 
 
 class ComputeResult(ctypes.Structure):
@@ -248,7 +248,7 @@ class Engine:
         return {
             "best_index": int(r.best_index), "best_count": int(r.best_count), "n_valid": int(r.n_valid),
             "best_subset": np.array(r.best_subset[: self.k]), "best_params": np.array(r.best_params[: self.n_params]),
-            "score_ms": r.score_ms, "consensus_ms": r.consensus_ms, "counts": counts, "params": oparams,
+            "score_ms": r.score_ms, "consensus_ms": r.consensus_ms, "evals": int(r.evals), "counts": counts, "params": oparams,
         }
 
     def consensus(self, params):

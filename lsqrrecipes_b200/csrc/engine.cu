@@ -216,6 +216,7 @@ struct lsqr_ctx {
   // hypothesis buffers
   size_t hcap = 0;
   int32_t* subsets = nullptr; double* hyp64 = nullptr; float* hyp32 = nullptr; uint32_t* counts = nullptr;
+  float* hyp32b = nullptr; uint32_t* live_counts = nullptr; uint32_t* live_ids = nullptr; uint32_t* prune_dev = nullptr;   // early exit (Prune)
   int32_t* list_dev = nullptr; size_t list_cap = 0;
   double* params_in_dev = nullptr; size_t params_in_cap = 0;
   unsigned long long* key_dev = nullptr;  // [0] key, [1] n_valid (as u32 in low half)
@@ -333,11 +334,17 @@ int ensure_hyp(lsqr_ctx* ctx, size_t H) {
   if (ctx->hyp64) cudaFree(ctx->hyp64);
   if (ctx->hyp32) cudaFree(ctx->hyp32);
   if (ctx->counts) cudaFree(ctx->counts);
+  cudaFree(ctx->hyp32b); cudaFree(ctx->live_counts); cudaFree(ctx->live_ids); cudaFree(ctx->prune_dev);
   ctx->subsets = nullptr; ctx->hyp64 = nullptr; ctx->hyp32 = nullptr; ctx->counts = nullptr; ctx->hcap = 0;
+  ctx->hyp32b = nullptr; ctx->live_counts = nullptr; ctx->live_ids = nullptr; ctx->prune_dev = nullptr;
   CK(cudaMalloc((void**)&ctx->subsets, sizeof(int32_t) * LSQR_MAX_SUBSET * want));
   CK(cudaMalloc((void**)&ctx->hyp64, sizeof(double) * LSQR_MAX_PARAMS * want));
   CK(cudaMalloc((void**)&ctx->hyp32, sizeof(float) * 16 * want));   // up to four float4 groups per hypothesis (8-D line: 16 constants)
   CK(cudaMalloc((void**)&ctx->counts, sizeof(uint32_t) * want));
+  CK(cudaMalloc((void**)&ctx->hyp32b, sizeof(float) * 16 * want));
+  CK(cudaMalloc((void**)&ctx->live_counts, sizeof(uint32_t) * 2 * want));
+  CK(cudaMalloc((void**)&ctx->live_ids, sizeof(uint32_t) * 2 * want));
+  CK(cudaMalloc((void**)&ctx->prune_dev, sizeof(uint32_t) * prune_dev_words(want)));
   ctx->hcap = want;
   return 0;
 }
@@ -526,7 +533,7 @@ int score_impl(lsqr_ctx* ctx, const lsqr_score_args* a, lsqr_score_result* res) 
   if (a->sampler == LSQR_SAMPLE_LIST && !a->subsets) return fail(ctx, LSQR_ERR_ARG, "subset list missing");
   if (a->sampler == LSQR_SAMPLE_PARAMS && !a->params) return fail(ctx, LSQR_ERR_ARG, "parameter list missing");
   CK(cudaSetDevice(ctx->device));
-  memset(res, 0, sizeof(*res));
+  memset(res, 0, sizeof(*res));   // (res->evals accumulates over the batches below)
   const uint64_t H = a->count;
   const uint64_t lo = H * (uint64_t)ctx->rank / (uint64_t)ctx->world, hi = H * (uint64_t)(ctx->rank + 1) / (uint64_t)ctx->world;
   const bool can_sample = ds.n >= (uint32_t)mi.K || a->sampler == LSQR_SAMPLE_PARAMS;
@@ -557,9 +564,15 @@ int score_impl(lsqr_ctx* ctx, const lsqr_score_args* a, lsqr_score_result* res) 
       launch_solve(sa, dv, ctx->cfg, s); ctx->launches++;
       if (a->precision == LSQR_FP32) { launch_hoist32(ctx->model, ctx->hyp64, ctx->hcap, B, dv, ctx->cfg, ctx->hyp32, s); ctx->launches++; }
       CK(cudaMemsetAsync(ctx->counts, 0, sizeof(uint32_t) * B, s));
+      // without per-hypothesis counts only the winner matters: hypotheses that can no longer tie it stop being scored; the
+      // request's hoisted constants are not read again once the live list has been compacted out of them
+      Prune pr{{ctx->hyp32b, ctx->hyp32}, {ctx->live_counts, ctx->live_counts + ctx->hcap}, {ctx->live_ids, ctx->live_ids + ctx->hcap},
+               ctx->prune_dev, reinterpret_cast<uint32_t*>(ctx->pin) /* host scratch */, ctx->key_dev, (uint64_t)B * dv.n};
       CK(cudaEventRecord(ctx->ev[2], s));
-      ctx->launches += launch_consensus(ctx->model, a->precision, dv, ctx->hyp64, ctx->hyp32, ctx->hcap, B, ctx->cfg, ctx->counts, ctx->num_sms, s);
+      ctx->launches += launch_consensus(ctx->model, a->precision, dv, ctx->hyp64, ctx->hyp32, ctx->hcap, B, ctx->cfg, ctx->counts, ctx->num_sms, s,
+                                        a->out_counts ? nullptr : &pr);
       CK(cudaEventRecord(ctx->ev[3], s));
+      res->evals += pr.evals;
       timed = true;
       launch_argmax(ctx->counts, B, (uint32_t)b0, ctx->key_dev, s); ctx->launches++;
       CKL();
@@ -1175,6 +1188,7 @@ void lsqr_ctx_destroy(lsqr_ctx* ctx) {
   cudaFree(ctx->gather_dev); if (ctx->gather_pin) cudaFreeHost(ctx->gather_pin);
   for (int i = 0; i < lsqr_ctx::kRing; i++) if (ctx->up_pin[i]) cudaFreeHost(ctx->up_pin[i]);
   cudaFree(ctx->staging); cudaFree(ctx->subsets); cudaFree(ctx->hyp64); cudaFree(ctx->hyp32); cudaFree(ctx->counts);
+  cudaFree(ctx->hyp32b); cudaFree(ctx->live_counts); cudaFree(ctx->live_ids); cudaFree(ctx->prune_dev);
   cudaFree(ctx->list_dev); cudaFree(ctx->params_in_dev); cudaFree(ctx->key_dev); cudaFree(ctx->winner_dev); cudaFree(ctx->small_dev);
   cudaFree(ctx->rb.partials); cudaFree(ctx->rb.moments);
   if (ctx->pin) cudaFreeHost(ctx->pin);
@@ -1259,8 +1273,9 @@ int lsqr_score(lsqr_ctx* ctx, const lsqr_score_args* args, lsqr_score_result* re
     if (rc) return rc;
     *res = rs[0];
     uint32_t nv = 0;
-    for (const auto& r : rs) { nv += r.n_valid; res->score_ms = std::max(res->score_ms, r.score_ms); res->consensus_ms = std::max(res->consensus_ms, r.consensus_ms); }
-    res->n_valid = nv;
+    uint64_t ev = 0;
+    for (const auto& r : rs) { nv += r.n_valid; ev += r.evals; res->score_ms = std::max(res->score_ms, r.score_ms); res->consensus_ms = std::max(res->consensus_ms, r.consensus_ms); }
+    res->n_valid = nv; res->evals = ev;
     return LSQR_OK;
   }
   return score_impl(ctx, args, res);

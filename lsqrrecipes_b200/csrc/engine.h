@@ -99,12 +99,31 @@ void launch_solve(const SolveArgs& a, const DataView& dv, const EstCfg& cfg, cud
 // a.list / a.params_in = the request's device-resident list (samplers 2, 3)
 void launch_winner(const SolveArgs& a, const unsigned long long* key_dev, const DataView& dv, const EstCfg& cfg, WinnerRecord* out, cudaStream_t s);
 void launch_hoist32(int model, const double* hyp64, size_t hld, uint32_t H, const DataView& dv, const EstCfg& cfg, float* hyp32, cudaStream_t s);
-// counts[h] (+)= |{m : agree(h, datum m)}|.  counts must be zeroed by the caller.  Returns #launches.
+
+// Early exit of the fp32 constant-bank scoring (k_fast.cu), for requests that want the winner only.  A hypothesis with c
+// inliers among the first p data ends with at most c + (n - p); once that is below the full count L of some hypothesis it
+// can neither beat nor tie the winner, so it stops being scored and keeps its partial count (< L) in counts[].  The winner,
+// its count and the arg-max key are exactly those of the full pass.  Buffers come from ensure_hyp (engine.cu), [hld] each.
+struct Prune {
+  float* hyp32[2];                // [16][hld] each: the compacted live list's hoisted constants (may alias the request's)
+  uint32_t* live_counts[2];       // running counts of the live list
+  uint32_t* live_ids[2];          // the live hypotheses' indices in the launch
+  uint32_t* dev;                  // scratch: [0, 16) seed hypothesis constants, [16, 18) seed key, [18] L, [19] live count,
+                                  // [20, 20 + hld / 1024 + 1) per-block survivor tallies
+  uint32_t* host;                 // pinned, 4 words
+  const unsigned long long* floor_key;   // arg-max key of the request's earlier batches: its count is a valid L as well
+  uint64_t evals;                 // out: hypothesis x datum evaluations launched (real data only), the seed included; left as
+                                  // the caller set it (H n) when the request takes the full pass
+};
+constexpr size_t prune_dev_words(size_t hld) { return 20 + hld / 1024 + 1; }
+
+// counts[h] (+)= |{m : agree(h, datum m)}|.  counts must be zeroed by the caller.  Returns #launches.  With `prune`, fp32
+// requests that take the constant-bank kernel exit early (see Prune); the others ignore it.
 int launch_consensus(int model, int precision, const DataView& dv, const double* hyp64, const float* hyp32, size_t hld, uint32_t H,
-                     const EstCfg& cfg, uint32_t* counts, int num_sms, cudaStream_t s);
+                     const EstCfg& cfg, uint32_t* counts, int num_sms, cudaStream_t s, Prune* prune = nullptr);
 // fp32 fast mode (k_fast.cu)
 int launch_consensus32(int model, const DataView& dv, const float* hyp32, size_t hld, uint32_t H, const EstCfg& cfg, uint32_t* counts, int num_sms,
-                       cudaStream_t s);
+                       cudaStream_t s, Prune* prune = nullptr);
 // key = max over h of (counts[h] << 32) | (0xFFFFFFFF - (index_base + h)); key must be zeroed first.
 void launch_argmax(const uint32_t* counts, uint32_t H, uint32_t index_base, unsigned long long* key, cudaStream_t s);
 

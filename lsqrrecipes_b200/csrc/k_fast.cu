@@ -30,6 +30,8 @@
 #include "bulk_copy.cuh"
 #include "fast_forms.cuh"
 
+#include <algorithm>
+#include <cmath>
 #include <mutex>
 
 namespace lsqr {
@@ -268,6 +270,82 @@ __global__ void __launch_bounds__(THREADS, LSQR_CB_MINBLOCKS) consensus_cb_kerne
   }
 }
 
+// ---- early exit of the constant-bank path (Prune, engine.h) ------------------------------------
+constexpr uint32_t kPruneThreads = 1024;
+
+// The hoisted constants of the hypothesis that holds the arg-max key (index relative to the launch) -> one column (hld 1).
+__global__ void prune_seed_kernel(const unsigned long long* __restrict__ key, const float4* __restrict__ hyp, size_t hld, int groups, float4* __restrict__ col) {
+  const uint32_t h = 0xFFFFFFFFu - (uint32_t)(*key & 0xFFFFFFFFull);
+  if ((int)threadIdx.x < groups) col[threadIdx.x] = hyp[threadIdx.x * hld + h];
+}
+
+// Survivors among the live hypotheses [1024 b, 1024 b + 1024): i stays iff cnt[i] + rem >= L (rem: data not scored yet).
+__global__ void __launch_bounds__(kPruneThreads) prune_tally_kernel(const uint32_t* __restrict__ cnt, uint32_t H, uint32_t rem, uint32_t L, uint32_t* __restrict__ tally) {
+  const uint32_t i = blockIdx.x * kPruneThreads + threadIdx.x;
+  const int k = __syncthreads_count(i < H && cnt[i] + rem >= L);
+  if (threadIdx.x == 0) tally[blockIdx.x] = (uint32_t)k;
+}
+
+// Order-preserving compaction of the live list (constants [groups][hld] float4, running count, index in the launch) with
+// the tallies of prune_tally_kernel; a hypothesis that drops out leaves its partial count in counts[id].  id_in == nullptr:
+// the list is still the launch's own (counts themselves, identity ids).  The last thread writes the new live count.
+__global__ void __launch_bounds__(kPruneThreads) prune_move_kernel(const float4* __restrict__ hyp_in, const uint32_t* __restrict__ cnt_in,
+                                                                   const uint32_t* __restrict__ id_in, size_t hld, int groups, uint32_t H, uint32_t rem,
+                                                                   uint32_t L, const uint32_t* __restrict__ tally, float4* __restrict__ hyp_out,
+                                                                   uint32_t* __restrict__ cnt_out, uint32_t* __restrict__ id_out,
+                                                                   uint32_t* __restrict__ counts, uint32_t* __restrict__ live) {
+  __shared__ uint32_t warp_base[kPruneThreads / 32];
+  __shared__ uint32_t block_base;
+  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  uint32_t before = 0;   // survivors of the blocks ahead of this one
+  for (uint32_t j = threadIdx.x; j < blockIdx.x; j += kPruneThreads) before += tally[j];
+  before = __reduce_add_sync(0xffffffffu, before);
+  if (lane == 0) warp_base[warp] = before;
+  __syncthreads();
+  if (warp == 0) {
+    const uint32_t v = __reduce_add_sync(0xffffffffu, warp_base[lane]);
+    if (lane == 0) block_base = v;
+  }
+  __syncthreads();
+  const uint32_t i = blockIdx.x * kPruneThreads + threadIdx.x;
+  const uint32_t c = i < H ? cnt_in[i] : 0u;
+  const bool keep = i < H && c + rem >= L;
+  const uint32_t ball = __ballot_sync(0xffffffffu, keep);
+  if (lane == 0) warp_base[warp] = __popc(ball);
+  __syncthreads();
+  if (warp == 0) {   // exclusive scan of the 32 warp tallies
+    const uint32_t v = warp_base[lane];
+    uint32_t x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= (uint32_t)o) x += y;
+    }
+    warp_base[lane] = block_base + x - v;
+  }
+  __syncthreads();
+  const uint32_t pos = warp_base[warp] + __popc(ball & ((1u << lane) - 1u));
+  if (keep) {
+    for (int g = 0; g < groups; g++) hyp_out[(size_t)g * hld + pos] = hyp_in[(size_t)g * hld + i];
+    cnt_out[pos] = c;
+    id_out[pos] = id_in ? id_in[i] : i;
+  } else if (i < H && id_in) {
+    counts[id_in[i]] = c;
+  }
+  if (blockIdx.x == gridDim.x - 1 && threadIdx.x == kPruneThreads - 1) *live = pos + (keep ? 1u : 0u);
+}
+
+// The survivors' full counts back to their hypotheses.
+__global__ void prune_scatter_kernel(const uint32_t* __restrict__ cnt, const uint32_t* __restrict__ id, uint32_t H, uint32_t* __restrict__ counts) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < H) counts[id[i]] = cnt[i];
+}
+
+// What a compaction costs, in hypotheses of one plane launch (0.52 ms per 2^20 on a B200, so ~32 us): its two small kernels
+// (6.5 us of device time at the bench configuration, profiles/r03_prune_probe.jsonl) and the host round trip for the new
+// live count, which leaves the device idle until the next launch arrives.
+constexpr double kCompactCostHyps = 65536.0;
+
 // Hypotheses per thread (R) / point pairs per iteration (PPI) of the constant-bank kernel (128 threads), from the sweeps in
 // profiles/r01_tune_cb_sweep_models.txt and profiles/r02_tune_cb_blocking.txt (the plane's 12 x 8 -- sixteen points per iteration --
 // is 4.6 % faster than the 10 x 4 it replaced: half the loop overhead per point).  Two things decide them:
@@ -318,8 +396,9 @@ constexpr int cb_blocking(int m, bool want_r) {
 template <int M> struct BlockCB { static constexpr int R = cb_blocking(M, true), PPI = cb_blocking(M, false); };
 
 template <int M>
-static int run_consensus_cb(const DataView& dv, const float* hyp, size_t hld, uint32_t H, const EstCfg& cfg, uint32_t* counts, int num_sms, cudaStream_t s) {
-  constexpr int D = Model<M>::D, R = BlockCB<M>::R, PPI = BlockCB<M>::PPI, THREADS = LSQR_CB_THREADS;
+static int run_consensus_cb(const DataView& dv, const float* hyp, size_t hld, uint32_t H, const EstCfg& cfg, uint32_t* counts, int num_sms, cudaStream_t s,
+                            Prune* pr) {
+  constexpr int D = Model<M>::D, R = BlockCB<M>::R, PPI = BlockCB<M>::PPI, THREADS = LSQR_CB_THREADS, G = (Model<M>::Q32 + 3) / 4;
   constexpr uint32_t cp = cb_points<M>();
   auto kern = consensus_cb_kernel<M, R, THREADS, PPI>;
   int dev = 0;
@@ -332,7 +411,7 @@ static int run_consensus_cb(const DataView& dv, const float* hyp, size_t hld, ui
   }
   void* bank = nullptr;
   if (cudaGetSymbolAddress(&bank, c_tile) != cudaSuccess) return -1;
-  const uint32_t hyp_blocks = (H + THREADS * R - 1) / (THREADS * R);
+  uint32_t hyp_blocks = 0;   // of the live hypotheses, per launch
   const uint32_t slots = (uint32_t)num_sms * (uint32_t)occ[dev % kMaxDevices];
   // sub-chunks per launch: fill the last wave (the launches of one request serialise on the bank)
   constexpr bool kRaw = Eval<M>::kHasAbsForm && !Eval<M>::kShifted;
@@ -351,14 +430,65 @@ static int run_consensus_cb(const DataView& dv, const float* hyp, size_t hld, ui
   };
   std::lock_guard<std::mutex> lock(g_cb_mutex[dev % kMaxDevices]);
   int launches = 0;
-  for (size_t base = 0; base < dv.span; base += cp) {
+  // The live list: all H hypotheses in place until the first compaction, then alternately in pr->hyp32[0] and [1].
+  const float* live_hyp = hyp;
+  uint32_t* live_cnt = counts;
+  const uint32_t* live_id = nullptr;
+  uint32_t live = H, L = 0;   // L = 0: no early exit
+  uint64_t evals = 0;
+  int flip = 0;
+  // the floor L is seeded after the launches that cover ~1 % of the data (at least one)
+  const size_t seed_end = pr ? std::max<size_t>(1, (dv.n / 100 + cp - 1) / cp) * cp : 0;
+  size_t next_compact = 0, last_compact = SIZE_MAX;
+  for (size_t base = 0; base < dv.span && live; base += cp) {
     const uint32_t npts = (uint32_t)((dv.span - base < cp) ? (dv.span - base) : cp);   // span is a multiple of 1024, cp of 16
     if (base >= dv.n) break;                                                        // only NaN padding left
+    const uint32_t rem = dv.n - (uint32_t)base;                                     // data not scored yet
+    if (pr && base == seed_end) {
+      // L: the full count of the hypothesis with the best partial count, through consensus32_kernel (the same fp32 predicate)
+      unsigned long long* key = reinterpret_cast<unsigned long long*>(pr->dev + 16);
+      if (cudaMemsetAsync(pr->dev + 16, 0, 4 * sizeof(uint32_t), s) != cudaSuccess) return -1;
+      launch_argmax(counts, H, 0, key, s);
+      prune_seed_kernel<<<1, 32, 0, s>>>(key, reinterpret_cast<const float4*>(hyp), hld, G, reinterpret_cast<float4*>(pr->dev));
+      launches += 2 + launch_consensus32(M, dv, reinterpret_cast<const float*>(pr->dev), 1, 1, cfg, pr->dev + 18, num_sms, s);
+      if (cudaMemcpyAsync(pr->host, pr->dev + 18, sizeof(uint32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+          cudaMemcpyAsync(pr->host + 2, pr->floor_key, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+          cudaStreamSynchronize(s) != cudaSuccess) return -1;
+      L = std::max(pr->host[0], (uint32_t)(*reinterpret_cast<const unsigned long long*>(pr->host + 2) >> 32));
+      evals += dv.n;
+    }
+    if (L > rem && base >= next_compact) {   // some c + rem may now be < L
+      const uint32_t blocks = (live + kPruneThreads - 1) / kPruneThreads;
+      float* out_hyp = pr->hyp32[flip];
+      uint32_t* out_cnt = pr->live_counts[flip];
+      uint32_t* out_id = pr->live_ids[flip];
+      prune_tally_kernel<<<blocks, kPruneThreads, 0, s>>>(live_cnt, live, rem, L, pr->dev + 20);
+      prune_move_kernel<<<blocks, kPruneThreads, 0, s>>>(reinterpret_cast<const float4*>(live_hyp), live_cnt, live_id, hld, G, live, rem, L, pr->dev + 20,
+                                                         reinterpret_cast<float4*>(out_hyp), out_cnt, out_id, counts, pr->dev + 19);
+      if (cudaMemcpyAsync(pr->host + 1, pr->dev + 19, sizeof(uint32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) return -1;
+      launches += 2;
+      // next compaction when the hypotheses expected to drop out by then (at the rate seen since the last one) cost more
+      // evaluations than a compaction: interval k launches minimises d k / 2 + cost / k at k = sqrt(2 cost / d)
+      const double window = last_compact == SIZE_MAX ? 1.0 : (double)((base - last_compact) / cp);
+      const double d = std::max(1.0, (double)(live - pr->host[1]) / window);
+      next_compact = base + cp * (size_t)std::min(64.0, std::max(1.0, std::sqrt(2.0 * kCompactCostHyps / d)));
+      last_compact = base;
+      live_hyp = out_hyp; live_cnt = out_cnt; live_id = out_id; live = pr->host[1];
+      flip ^= 1;
+      if (!live) break;
+    }
+    hyp_blocks = (live + THREADS * R - 1) / (THREADS * R);
     if (cudaMemcpy2DAsync(bank, sizeof(float) * cp, dv.soa32 + base, sizeof(float) * dv.ld, sizeof(float) * npts, D, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return -1;
     const uint32_t sub = pick_sub(npts);
-    kern<<<dim3(hyp_blocks, (npts + sub - 1) / sub), THREADS, 0, s>>>(npts, sub, hyp, hld, H, (float)cfg.delta, (float)cfg.delta2, counts);
+    kern<<<dim3(hyp_blocks, (npts + sub - 1) / sub), THREADS, 0, s>>>(npts, sub, live_hyp, hld, live, (float)cfg.delta, (float)cfg.delta2, live_cnt);
     launches += 2;
+    evals += (uint64_t)live * std::min(npts, rem);
   }
+  if (live_id && live) {
+    prune_scatter_kernel<<<(live + 255) / 256, 256, 0, s>>>(live_cnt, live_id, live, counts);
+    launches++;
+  }
+  if (pr) pr->evals = evals;
   // the bank is shared by every context on this device: finish before another request may refill it
   if (cudaStreamSynchronize(s) != cudaSuccess) return -1;
   return launches;
@@ -378,10 +508,10 @@ constexpr int block32_r(int m) {
 template <int M> struct Block32 { static constexpr int R = block32_r(M), PPI = (M == ABSOR || M == RAY || M == PIVOT || M == USXW || M == USCP) ? 1 : ((M == LINE2D || M == LINE2) ? 4 : 2); };
 
 int launch_consensus32(int model, const DataView& dv, const float* hyp32, size_t hld, uint32_t H, const EstCfg& cfg, uint32_t* counts, int num_sms,
-                       cudaStream_t s) {
+                       cudaStream_t s, Prune* prune) {
   if (H == 0 || dv.n == 0) return 0;
   if (H >= kCbMinHyps) {
-#define CALL(MM) return run_consensus_cb<MM>(dv, hyp32, hld, H, cfg, counts, num_sms, s)
+#define CALL(MM) return run_consensus_cb<MM>(dv, hyp32, hld, H, cfg, counts, num_sms, s, prune)
     LSQR_DISPATCH_MODEL(model, CALL)
 #undef CALL
   }

@@ -260,7 +260,7 @@ static int run_consensus(const DataView& dv, const double* hyp, size_t hld, uint
 #define LSQR_FP64_R 4
 #endif
 int launch_consensus(int model, int precision, const DataView& dv, const double* hyp64, const float* hyp32, size_t hld, uint32_t H,
-                     const EstCfg& cfg, uint32_t* counts, int num_sms, cudaStream_t s) {
+                     const EstCfg& cfg, uint32_t* counts, int num_sms, cudaStream_t s, Prune* prune) {
   if (H == 0 || dv.n == 0) return 0;
   if (precision == 0) {
 #define CALL(MM)                                                                                                             \
@@ -269,7 +269,7 @@ int launch_consensus(int model, int precision, const DataView& dv, const double*
     LSQR_DISPATCH_MODEL(model, CALL)
 #undef CALL
   } else {
-    return launch_consensus32(model, dv, hyp32, hld, H, cfg, counts, num_sms, s);
+    return launch_consensus32(model, dv, hyp32, hld, H, cfg, counts, num_sms, s, prune);
   }
   return 0;
 }
