@@ -234,18 +234,26 @@ int lsqr_compute(lsqr_ctx* ctx, const void* aos, size_t n, size_t stride_bytes, 
  * lexicographic order, first maximum wins. */
 int lsqr_ransac_exhaustive(lsqr_ctx* ctx, int precision, uint8_t* out_mask_bytes, lsqr_compute_result* res);
 
-/* Many independent small problems, one thread block per problem (a host loop of
- * RANSAC::compute calls in the reference).  data: host packed doubles, problems back to
- * back; `offsets` [n_problems+1] in records.  exhaustive != 0 enumerates all C(n,k) subsets
+/* Many independent problems (a host loop of RANSAC::compute calls in the reference).  data: host packed doubles, problems
+ * back to back; `offsets` [n_problems+1] in records.  exhaustive != 0 enumerates all C(n,k) subsets
  * of each problem (RANSAC.hxx:150-249); otherwise rounds of Philox hypotheses with the stop
  * rule of RANSAC.hxx:107-110 for `prob` (prob <= 0: exactly max_tries hypotheses), capped at
  * max_tries, scored in `precision` (LSQR_FP32: the fast forms on an fp32 copy of the points relative to the problem's
  * first point; exhaustive mode always scores in fp64).  Minimal solves, the winner's consensus set, its count and the
  * refine are fp64 in every mode.  Outputs per problem: params [n_problems][P] (NaN row = empty), counts
- * [n_problems], optional masks (bytes, same indexing as data). */
+ * [n_problems], optional masks (bytes, same indexing as data).
+ * A problem of up to `one_block` records (lsqr_batch_capacity) is solved by one thread block with its points in shared
+ * memory.  A larger one, in randomized mode, by a thread-block cluster of 2 to 16 blocks that split its points between their
+ * shared memories (the smallest cluster that holds it), up to `max_records`; its result depends only on the problem, its
+ * index, the seed, prob and max_tries.  Exhaustive mode keeps the one-block limit.  A problem above the limit fails the
+ * call with LSQR_ERR_ARG. */
 int lsqr_ransac_batch(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint64_t n_problems,
                       int exhaustive, double prob, uint32_t max_tries, uint64_t seed, int precision,
                       double* out_params, uint32_t* out_counts, uint8_t* out_masks, double* device_ms);
+/* The problem sizes lsqr_ransac_batch takes for the context's model on its device (a group context: its first device), in
+ * records: *one_block, the largest one thread block holds, and *max_records, the largest the call takes at all (equal to
+ * one_block in exhaustive mode).  LSQR_ERR_ARG for a model without batched mode (the ultrasound calibrations). */
+int lsqr_batch_capacity(lsqr_ctx* ctx, int precision, int exhaustive, uint64_t* one_block, uint64_t* max_records);
 
 /* ---- the estimator's own methods, for callers that use them directly ---------------- */
 /* estimate() on k (or more) data in host memory; *n_params = 0 when degenerate. */

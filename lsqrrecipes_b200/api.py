@@ -103,6 +103,7 @@ def load_library():
         "lsqr_ransac_exhaustive": (c.c_int, [c.c_void_p, c.c_int, _u8p, c.POINTER(ComputeResult)]),
         "lsqr_compute": (c.c_int, [c.c_void_p, c.c_void_p, c.c_size_t, c.c_size_t, c.c_double, c.c_int, c.c_uint64, _u8p, c.POINTER(ComputeResult)]),
         "lsqr_ransac_batch": (c.c_int, [c.c_void_p, _dp, _u64p, c.c_uint64, c.c_int, c.c_double, c.c_uint32, c.c_uint64, c.c_int, _dp, _u32p, _u8p, _dp]),
+        "lsqr_batch_capacity": (c.c_int, [c.c_void_p, c.c_int, c.c_int, _u64p, _u64p]),
         "lsqr_estimate": (c.c_int, [c.c_void_p, _dp, c.c_size_t, _dp, c.POINTER(c.c_int)]),
         "lsqr_agree": (c.c_int, [c.c_void_p, _dp, _dp, c.c_size_t, _u8p]),
         "lsqr_least_squares": (c.c_int, [c.c_void_p, _dp, c.c_size_t, _dp, c.POINTER(c.c_int)]),
@@ -126,6 +127,7 @@ EXPORTED_SYMBOLS = [
     "lsqr_microbench_fma", "lsqr_last_refine_stats", "lsqr_weighted_least_squares",
     "lsqr_device_count", "lsqr_ctx_create_multi", "lsqr_ctx_world", "lsqr_nccl_unique_id", "lsqr_ctx_init_nccl", "lsqr_get_mask_bits",
     "lsqr_compute", "lsqr_bench_refine_pass", "lsqr_model_plane", "lsqr_model_sphere", "lsqr_model_line", "lsqr_model_dense",
+    "lsqr_batch_capacity",
 ]
 
 
@@ -317,6 +319,13 @@ class Engine:
         self._ck(self.lib.lsqr_ransac_batch(self.h, _ptr(d, _dp), _ptr(off, _u64p), nprob, 1 if exhaustive else 0, float(prob),
                                             int(max_tries), seed, int(precision), _ptr(prm, _dp), _ptr(cnt, _u32p), _ptr(masks, _u8p), ctypes.byref(ms)))
         return {"params": prm, "counts": cnt, "masks": masks, "device_ms": ms.value}
+
+    def batch_capacity(self, precision=FP64, exhaustive=False):
+        """(one_block, max_records): the largest problem, in records, that ransac_batch solves in one thread block, and the
+        largest it takes at all (a thread-block cluster per problem; exhaustive mode keeps the one-block limit)."""
+        one, most = ctypes.c_uint64(0), ctypes.c_uint64(0)
+        self._ck(self.lib.lsqr_batch_capacity(self.h, int(precision), 1 if exhaustive else 0, ctypes.byref(one), ctypes.byref(most)))
+        return int(one.value), int(most.value)
 
     # -- the estimator's own methods ---------------------------------------------------
     def estimate(self, data):

@@ -232,6 +232,7 @@ struct lsqr_ctx {
   uint64_t* bt_off = nullptr; size_t bt_off_cap = 0;
   double* bt_prm = nullptr; size_t bt_prm_cap = 0;
   uint32_t* bt_cnt = nullptr; size_t bt_cnt_cap = 0;
+  uint32_t* bt_cl = nullptr; size_t bt_cl_cap = 0;         //   the problems that take the cluster path, grouped by cluster size
   unsigned char* gather_dev = nullptr; size_t gather_cap = 0;        // compute(): records of the first round's minimal subsets
   unsigned char* gather_pin = nullptr; size_t gather_pin_cap = 0;
   uint8_t* mask_dev = nullptr; size_t mask_dev_cap = 0;   // consensus set, one byte per datum (device)
@@ -984,13 +985,27 @@ int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint6
   const ModelInfo mi = model_info(ctx->model);
   CK(cudaSetDevice(ctx->device));
   const uint64_t base = offsets[p0], total = offsets[p1] - base;
+  const bool use32 = precision == LSQR_FP32 && !exhaustive;   // fp32 scoring keeps an fp32 copy of the points next to the fp64 one
+  // A problem that fits one block takes batch_kernel (max_n is taken over those problems only); a larger one a cluster of
+  // C CTAs, the smallest that holds it.  cl[k] lists the problems (relative to p0) of cluster size 2 << k, cl_slice[k] the
+  // largest slice among them.
+  const BatchLimits L = batch_limits(ctx->model, use32 ? 1 : 0, exhaustive);
   uint32_t max_n = 1;
+  std::vector<uint32_t> cl[4];
+  uint32_t cl_slice[4] = {0, 0, 0, 0};
   for (uint64_t b = p0; b < p1; b++) {
     if (offsets[b + 1] < offsets[b]) return fail(ctx, LSQR_ERR_ARG, "offsets must be non-decreasing");
-    max_n = std::max<uint64_t>(max_n, offsets[b + 1] - offsets[b]);
+    const uint64_t nb = offsets[b + 1] - offsets[b];
+    if (nb <= L.one_block) { max_n = std::max<uint64_t>(max_n, nb); continue; }
+    if (L.max_cluster == 0) return fail(ctx, LSQR_ERR_ARG, "a problem does not fit in shared memory; use lsqr_ransac for large problems");
+    if (nb > L.max_records)
+      return fail(ctx, LSQR_ERR_ARG, "a problem of " + std::to_string(nb) + " records exceeds the batch limit of " + std::to_string(L.max_records) +
+                                         " records for this model and precision; use lsqr_compute for larger problems");
+    const uint32_t c = batch_cluster_size(L, nb);
+    const int k = c == 2 ? 0 : c == 4 ? 1 : c == 8 ? 2 : 3;
+    cl[k].push_back((uint32_t)(b - p0));
+    cl_slice[k] = std::max<uint32_t>(cl_slice[k], (uint32_t)(((nb + c - 1) / c + 1) & ~1ull));
   }
-  const bool use32 = precision == LSQR_FP32 && !exhaustive;   // fp32 scoring keeps an fp32 copy of the points next to the fp64 one
-  if ((size_t)max_n * mi.D * (sizeof(double) + (use32 ? sizeof(float) : 0)) + 16 > 200 * 1024) return fail(ctx, LSQR_ERR_ARG, "a problem does not fit in shared memory; use lsqr_ransac for large problems");
   cudaStream_t s = ctx->stream;
   // persistent buffers (a cudaMalloc/cudaFree set per call cost more than the kernel)
   if (int rc = ensure(ctx, &ctx->bt_data, &ctx->bt_data_cap, (size_t)std::max<uint64_t>(total, 1) * mi.D)) return rc;
@@ -1020,6 +1035,9 @@ int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint6
       if (int rc = up.put(ctx->bt_data + (rec0 + c0) * mi.D, data + (offsets[q0] + c0) * mi.D, cn * rec_bytes)) return rc;
     }
     if (nrec) if (int rc = up.landed()) return rc;
+    bool any_small = false;
+    for (uint64_t b = q0; b < q1 && !any_small; b++) any_small = offsets[b + 1] - offsets[b] <= L.one_block;
+    if (!any_small) { q0 = q1; continue; }   // every problem of this piece takes the cluster path
     BatchArgs ba{};
     ba.model = ctx->model; ba.exhaustive = exhaustive; ba.precision = use32 ? 1 : 0; ba.tries = max_tries; ba.prob = prob; ba.seed = seed;
     ba.data = ctx->bt_data + rec0 * mi.D; ba.offsets = ctx->bt_off + (q0 - p0); ba.n_problems = (uint32_t)(q1 - q0); ba.max_n = max_n;
@@ -1033,6 +1051,33 @@ int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint6
     ctx->launches++;
     CK(cudaEventRecord(e1, s));
     q0 = q1;
+  }
+  // the large problems, once every piece has landed: one launch per cluster size
+  std::vector<uint32_t> cl_all;
+  for (const auto& v : cl) cl_all.insert(cl_all.end(), v.begin(), v.end());
+  if (!cl_all.empty()) {
+    if (int rc = ensure(ctx, &ctx->bt_cl, &ctx->bt_cl_cap, cl_all.size())) return rc;
+    CK(cudaMemcpyAsync(ctx->bt_cl, cl_all.data(), sizeof(uint32_t) * cl_all.size(), cudaMemcpyHostToDevice, s));
+    BatchArgs ba{};
+    ba.model = ctx->model; ba.precision = use32 ? 1 : 0; ba.tries = max_tries; ba.prob = prob; ba.seed = seed;
+    ba.data = ctx->bt_data; ba.offsets = ctx->bt_off; ba.base = base; ba.first_problem = p0;
+    ba.out_params = ctx->bt_prm; ba.out_counts = ctx->bt_cnt; ba.out_masks = out_masks ? ctx->mask_dev : nullptr;
+    size_t first = 0;
+    for (int k = 0; k < 4; k++) {
+      if (cl[k].empty()) continue;
+      ba.n_problems = (uint32_t)cl[k].size();
+      cudaEvent_t e0, e1;
+      CK(cudaEventCreate(&e0)); tev.push_back(e0);
+      CK(cudaEventCreate(&e1)); tev.push_back(e1);
+      CK(cudaEventRecord(e0, s));
+      if (launch_batch_cluster(ba, ctx->bt_cl + first, ba.n_problems, 2u << k, cl_slice[k], ctx->cfg, ctx->ls_type, s) < 0) {
+        for (cudaEvent_t e : tev) cudaEventDestroy(e);
+        return fail(ctx, LSQR_ERR_CUDA, std::string("batch cluster launch: ") + cudaGetErrorString(cudaGetLastError()));
+      }
+      ctx->launches++;
+      CK(cudaEventRecord(e1, s));
+      first += cl[k].size();
+    }
   }
   CKL();
   CK(cudaMemcpyAsync(out_params + p0 * mi.P, ctx->bt_prm, sizeof(double) * np * mi.P, cudaMemcpyDeviceToHost, s));
@@ -1183,7 +1228,7 @@ void lsqr_ctx_destroy(lsqr_ctx* ctx) {
   if (ctx->comm && nccl().ok) nccl().CommDestroy(ctx->comm);
   ctx->copier.reset();
   free_dataset(ctx->main); free_dataset(ctx->scratch);
-  cudaFree(ctx->bt_data); cudaFree(ctx->bt_off); cudaFree(ctx->bt_prm); cudaFree(ctx->bt_cnt);
+  cudaFree(ctx->bt_data); cudaFree(ctx->bt_off); cudaFree(ctx->bt_prm); cudaFree(ctx->bt_cnt); cudaFree(ctx->bt_cl);
   cudaFree(ctx->weights_dev); cudaFree(ctx->mask_dev); if (ctx->mask_pin) cudaFreeHost(ctx->mask_pin); if (ctx->agree_pin) cudaFreeHost(ctx->agree_pin);
   cudaFree(ctx->gather_dev); if (ctx->gather_pin) cudaFreeHost(ctx->gather_pin);
   for (int i = 0; i < lsqr_ctx::kRing; i++) if (ctx->up_pin[i]) cudaFreeHost(ctx->up_pin[i]);
@@ -1381,6 +1426,19 @@ int lsqr_ransac_batch(lsqr_ctx* ctx, const double* data, const uint64_t* offsets
     return rc;
   }
   return batch_impl(ctx, data, offsets, 0, n_problems, exhaustive, prob, max_tries, seed, precision, out_params, out_counts, out_masks, device_ms);
+}
+
+int lsqr_batch_capacity(lsqr_ctx* ctx, int precision, int exhaustive, uint64_t* one_block, uint64_t* max_records) {
+  if (!ctx || !one_block || !max_records) return LSQR_ERR_ARG;
+  if (ctx->group) { lsqr_ctx* k = ctx->group->kids[0]; const int rc = lsqr_batch_capacity(k, precision, exhaustive, one_block, max_records); if (rc) ctx->err = k->err; return rc; }
+  if (ctx->model < 0) return fail(ctx, LSQR_ERR_STATE, "lsqr_set_estimator must be called first");
+  if (precision != LSQR_FP64 && precision != LSQR_FP32) return fail(ctx, LSQR_ERR_ARG, "bad precision");
+  if (ctx->model == USXW || ctx->model == USCP) return fail(ctx, LSQR_ERR_ARG, "the ultrasound calibrations have no batched mode");
+  CK(cudaSetDevice(ctx->device));
+  const BatchLimits L = batch_limits(ctx->model, precision == LSQR_FP32 ? 1 : 0, exhaustive);
+  *one_block = L.one_block;
+  *max_records = L.max_records;
+  return LSQR_OK;
 }
 
 int lsqr_estimate(lsqr_ctx* ctx, const double* packed, size_t n, double* out_params, int* n_params) {

@@ -176,6 +176,21 @@ struct BatchArgs {
   uint8_t* out_masks;        // [total] or null
 };
 int launch_batch(const BatchArgs& a, const EstCfg& cfg, int ls_type, cudaStream_t s);
+// Problem sizes, in records, of one lsqr_ransac_batch call on the current device.  A problem of up to one_block records takes
+// batch_kernel; a larger one takes batch_cluster_kernel on a cluster of C CTAs of `slice` records each (C = 2, 4, .., max_cluster),
+// up to max_records.  Exhaustive mode, and a model without the cluster kernel, stop at one_block (max_cluster = 0).
+struct BatchLimits { uint64_t one_block, max_records; uint32_t slice; int max_cluster; };
+BatchLimits batch_limits(int model, int precision, int exhaustive);
+// the smallest cluster whose slices hold n records (0: none)
+inline uint32_t batch_cluster_size(const BatchLimits& L, uint64_t n) {
+  for (uint32_t c = 2; c <= (uint32_t)L.max_cluster; c *= 2)
+    if ((((n + c - 1) / c + 1) & ~1ull) <= L.slice) return c;
+  return 0;
+}
+// The problems a.offsets[problems[i]] (count of them, all of one cluster size) on clusters of `cluster` CTAs whose dynamic
+// shared memory holds `slice` records (the largest slice among them).
+int launch_batch_cluster(const BatchArgs& a, const uint32_t* problems, uint32_t count, uint32_t cluster, uint32_t slice, const EstCfg& cfg,
+                         int ls_type, cudaStream_t s);
 
 // ---- k_score.cu (single-call helpers) ---------------------------------------------------
 void launch_estimate_one(int model, const double* packed_dev, const EstCfg& cfg, double* out_dev /* [0]=n_params, [1..P] */, cudaStream_t s);
