@@ -10,7 +10,8 @@
  *
  * Plain pointers and sizes only; no C++ or torch types.  All entry points return 0 on
  * success or a negative lsqr_status; lsqr_last_error() gives the text.  Nothing throws
- * across this boundary.  One context per host thread; calls are synchronous at return.
+ * across this boundary.  One context per host thread; calls are synchronous at return (lsqr_ransac_batch_device excepted: it
+ * is stream-ordered).
  * There is NO CPU fallback: without a CUDA device every call fails with LSQR_ERR_CUDA.
  *
  * Data layouts are the reference's host layouts (SURVEY.md 8a-11): a datum is `dim` doubles
@@ -115,8 +116,8 @@ int lsqr_device_count(void);
  * and the refine are sharded by point range; the exchange steps are native NCCL calls inside the library (one
  * ncclAllReduce(max) on the packed 64-bit key per request, one ncclAllReduce(sum) of <= 91 doubles per refine pass, and the
  * all-gather that replicates the uploaded points over NVLink).  Every entry point below accepts such a context and returns
- * what a single-GPU context returns (lsqr_upload_device, lsqr_set_shard, lsqr_ctx_set_stream and lsqr_ctx_init_nccl excepted:
- * LSQR_ERR_ARG).  The estimator's own methods (estimate / agree / least squares) run on the first device. */
+ * what a single-GPU context returns (lsqr_upload_device, lsqr_ransac_batch_device, lsqr_set_shard, lsqr_ctx_set_stream and
+ * lsqr_ctx_init_nccl excepted: LSQR_ERR_ARG).  The estimator's own methods (estimate / agree / least squares) run on the first device. */
 int lsqr_ctx_create_multi(lsqr_ctx** out, int ngpus);
 /* Number of GPUs / ranks behind the context (1 for lsqr_ctx_create). */
 int lsqr_ctx_world(const lsqr_ctx* ctx);
@@ -250,6 +251,23 @@ int lsqr_ransac_exhaustive(lsqr_ctx* ctx, int precision, uint8_t* out_mask_bytes
 int lsqr_ransac_batch(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint64_t n_problems,
                       int exhaustive, double prob, uint32_t max_tries, uint64_t seed, int precision,
                       double* out_params, uint32_t* out_counts, uint8_t* out_masks, double* device_ms);
+/* lsqr_ransac_batch on data that already live in device memory of the context's device, stream-ordered.
+ * dev_data: packed doubles [offsets[n_problems]][dim] in device memory (record i at dev_data + i*dim, as in lsqr_ransac_batch;
+ * may be NULL when every problem is empty).
+ * offsets: HOST array [n_problems+1] of absolute record offsets (they pick the kernel, its shared memory and the cluster size).
+ * dev_params [n_problems][P], dev_counts [n_problems], dev_masks [offsets[n_problems]] bytes (optional, same indexing as the
+ * data): device memory of the context's device.  Every byte of [offsets[0], offsets[n_problems]) of dev_masks is written.
+ * cuda_stream: the stream the work is ordered on (NULL: the context's stream; the legacy default stream is cudaStreamLegacy).
+ * The call enqueues and returns.  It does not wait for the device except while it grows its internal buffers, or when two
+ * earlier calls' small host-to-device copies (offsets, cluster lists) are still queued.  The inputs must stay valid and
+ * unchanged, and the outputs untouched, until the stream has passed the call.  Results are bit for bit those of
+ * lsqr_ransac_batch with the same arguments.  Work on another stream than the context's is ordered after the context's earlier
+ * work, and the context's later work after it.  The uploaded data set and its stored consensus set are left as they are.
+ * LSQR_ERR_ARG: a pointer that is not device memory of this context's device, a multi-GPU group context, or any condition
+ * under which lsqr_ransac_batch fails (problem above lsqr_batch_capacity, decreasing offsets, bad precision). */
+int lsqr_ransac_batch_device(lsqr_ctx* ctx, const double* dev_data, const uint64_t* offsets, uint64_t n_problems,
+                             int exhaustive, double prob, uint32_t max_tries, uint64_t seed, int precision,
+                             double* dev_params, uint32_t* dev_counts, uint8_t* dev_masks, void* cuda_stream);
 /* The problem sizes lsqr_ransac_batch takes for the context's model on its device (a group context: its first device), in
  * records: *one_block, the largest one thread block holds, and *max_records, the largest the call takes at all (equal to
  * one_block in exhaustive mode).  LSQR_ERR_ARG for a model without batched mode (the ultrasound calibrations). */

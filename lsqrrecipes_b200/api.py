@@ -104,6 +104,8 @@ def load_library():
         "lsqr_compute": (c.c_int, [c.c_void_p, c.c_void_p, c.c_size_t, c.c_size_t, c.c_double, c.c_int, c.c_uint64, _u8p, c.POINTER(ComputeResult)]),
         "lsqr_ransac_batch": (c.c_int, [c.c_void_p, _dp, _u64p, c.c_uint64, c.c_int, c.c_double, c.c_uint32, c.c_uint64, c.c_int, _dp, _u32p, _u8p, _dp]),
         "lsqr_batch_capacity": (c.c_int, [c.c_void_p, c.c_int, c.c_int, _u64p, _u64p]),
+        "lsqr_ransac_batch_device": (c.c_int, [c.c_void_p, c.c_void_p, _u64p, c.c_uint64, c.c_int, c.c_double, c.c_uint32, c.c_uint64, c.c_int,
+                                               c.c_void_p, c.c_void_p, c.c_void_p, c.c_void_p]),
         "lsqr_estimate": (c.c_int, [c.c_void_p, _dp, c.c_size_t, _dp, c.POINTER(c.c_int)]),
         "lsqr_agree": (c.c_int, [c.c_void_p, _dp, _dp, c.c_size_t, _u8p]),
         "lsqr_least_squares": (c.c_int, [c.c_void_p, _dp, c.c_size_t, _dp, c.POINTER(c.c_int)]),
@@ -127,12 +129,58 @@ EXPORTED_SYMBOLS = [
     "lsqr_microbench_fma", "lsqr_last_refine_stats", "lsqr_weighted_least_squares",
     "lsqr_device_count", "lsqr_ctx_create_multi", "lsqr_ctx_world", "lsqr_nccl_unique_id", "lsqr_ctx_init_nccl", "lsqr_get_mask_bits",
     "lsqr_compute", "lsqr_bench_refine_pass", "lsqr_model_plane", "lsqr_model_sphere", "lsqr_model_line", "lsqr_model_dense",
-    "lsqr_batch_capacity",
+    "lsqr_batch_capacity", "lsqr_ransac_batch_device",
 ]
 
 
 def _ptr(a, t):
     return a.ctypes.data_as(t) if a is not None else None
+
+
+_CUDA_STREAM_LEGACY = 1   # cudaStreamLegacy: the handle that names the legacy default stream, which torch reports as 0
+
+
+def check_batch_device_args(data, offsets, dim, device_index=None):
+    """The arguments of Engine.ransac_batch_device, checked on the host before any library call: `data` a contiguous
+    torch.float64 CUDA tensor, [total, dim] with `offsets` or [B, n, dim] without; `offsets` in host memory (a sequence, numpy
+    array or CPU tensor: reading a CUDA tensor would wait for its stream), B + 1 non-negative, non-decreasing record offsets
+    inside `data`.  Returns the data as [total, dim] and the offsets as a uint64 numpy array.  Raises ValueError."""
+    import torch
+    if not isinstance(data, torch.Tensor):
+        raise ValueError("data must be a torch tensor in CUDA memory")
+    if data.dtype != torch.float64:
+        raise ValueError(f"data must be torch.float64, not {data.dtype}")
+    if not data.is_contiguous():
+        raise ValueError("data must be contiguous")
+    if data.dim() == 3 and offsets is None:
+        if data.shape[2] != dim:
+            raise ValueError(f"data [B, n, dim] must have dim = {dim}, not {data.shape[2]}")
+        off = np.arange(data.shape[0] + 1, dtype=np.uint64) * np.uint64(data.shape[1])
+        data = data.reshape(-1, dim)
+    else:
+        if data.dim() != 2 or data.shape[1] != dim:
+            raise ValueError(f"data must be [total, {dim}] with offsets, or [B, n, {dim}] without, not {list(data.shape)}")
+        if offsets is None:
+            raise ValueError("data [total, dim] needs offsets")
+        if isinstance(offsets, torch.Tensor):
+            if offsets.device.type != "cpu":
+                raise ValueError("offsets must be in host memory (a sequence, numpy array or CPU tensor)")
+            offsets = offsets.numpy()
+        off = np.asarray(offsets)
+        if off.ndim != 1 or off.size < 1:
+            raise ValueError(f"offsets must be one-dimensional with n_problems + 1 >= 1 entries, not of shape {off.shape}")
+        if off.dtype.kind not in "iu" or (off.dtype.kind == "i" and (off < 0).any()):
+            raise ValueError("offsets must be non-negative integers")
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        if (off[1:] < off[:-1]).any():
+            raise ValueError("offsets must be non-decreasing")
+        if int(off[-1]) > data.shape[0]:
+            raise ValueError(f"offsets end at record {int(off[-1])}, past the {data.shape[0]} records of data")
+    if data.device.type != "cuda":
+        raise ValueError(f"data must be in CUDA memory, not on {data.device}")
+    if device_index is not None and data.device.index != device_index:
+        raise ValueError(f"data is on {data.device}; the engine runs on cuda:{device_index}")
+    return data, off
 
 
 class Engine:
@@ -154,6 +202,7 @@ class Engine:
         if rc != 0:
             raise LsqrError(f"{what} failed with status {rc}: no usable sm_100 CUDA device / NCCL (there is no CPU fallback)")
         self.h = h
+        self.device = device if gpus is None else None   # the device of a single-device context
         self._hooks = None
         self.n = 0
         self._ck(self.lib.lsqr_set_estimator(self.h, self.model, float(delta), float(aux), int(ls_type)))
@@ -319,6 +368,27 @@ class Engine:
         self._ck(self.lib.lsqr_ransac_batch(self.h, _ptr(d, _dp), _ptr(off, _u64p), nprob, 1 if exhaustive else 0, float(prob),
                                             int(max_tries), seed, int(precision), _ptr(prm, _dp), _ptr(cnt, _u32p), _ptr(masks, _u8p), ctypes.byref(ms)))
         return {"params": prm, "counts": cnt, "masks": masks, "device_ms": ms.value}
+
+    def ransac_batch_device(self, data, offsets=None, exhaustive=False, prob=0.999, max_tries=1024, seed=0, want_masks=False, precision=FP64):
+        """ransac_batch on a torch.float64 CUDA tensor on the engine's device: [total, dim] with host `offsets`, or [B, n, dim]
+        (B problems of n records each) without.  Returns CUDA tensors -- params [B, P] float64 (NaN row = empty), counts [B] int32,
+        masks [total] uint8 or None -- enqueued on torch.cuda.current_stream() and not waited for; bit for bit what ransac_batch
+        returns for the same data."""
+        import torch
+        d, off = check_batch_device_args(data, offsets, self.dim, self.device)
+        nprob = len(off) - 1
+        dev = d.device
+        prm = torch.empty((nprob, self.n_params), dtype=torch.float64, device=dev)
+        cnt = torch.empty(nprob, dtype=torch.int32, device=dev)   # every count is below max_records < 2**31
+        masks = torch.empty(d.shape[0], dtype=torch.uint8, device=dev) if want_masks else None
+        stream = torch.cuda.current_stream(dev).cuda_stream or _CUDA_STREAM_LEGACY
+        self._ck(self.lib.lsqr_ransac_batch_device(self.h, d.data_ptr(), _ptr(off, _u64p), nprob, 1 if exhaustive else 0, float(prob),
+                                                   int(max_tries), seed, int(precision), prm.data_ptr(), cnt.data_ptr(),
+                                                   masks.data_ptr() if masks is not None else None, stream))
+        if masks is not None:   # records outside the problems, as ransac_batch leaves them
+            masks[: int(off[0])].zero_()
+            masks[int(off[-1]):].zero_()
+        return {"params": prm, "counts": cnt, "masks": masks}
 
     def batch_capacity(self, precision=FP64, exhaustive=False):
         """(one_block, max_records): the largest problem, in records, that ransac_batch solves in one thread block, and the

@@ -233,6 +233,12 @@ struct lsqr_ctx {
   double* bt_prm = nullptr; size_t bt_prm_cap = 0;
   uint32_t* bt_cnt = nullptr; size_t bt_cnt_cap = 0;
   uint32_t* bt_cl = nullptr; size_t bt_cl_cap = 0;         //   the problems that take the cluster path, grouped by cluster size
+  // lsqr_ransac_batch_device: offsets and cluster lists go up from two page-locked slots used in turn (a copy from pageable
+  // memory may wait for the stream); bd_ev[i] is recorded after slot i's copies
+  unsigned char* bd_pin[2] = {nullptr, nullptr}; size_t bd_pin_cap[2] = {0, 0};
+  cudaEvent_t bd_ev[2]{};
+  uint64_t bd_calls = 0;
+  cudaEvent_t bd_order[2]{};              // [0]: the caller's stream waits for the context's stream, [1]: the reverse
   unsigned char* gather_dev = nullptr; size_t gather_cap = 0;        // compute(): records of the first round's minimal subsets
   unsigned char* gather_pin = nullptr; size_t gather_pin_cap = 0;
   uint8_t* mask_dev = nullptr; size_t mask_dev_cap = 0;   // consensus set, one byte per datum (device)
@@ -974,6 +980,65 @@ int compute_impl(lsqr_ctx* ctx, const void* aos, size_t n, size_t stride, double
   return finish_ransac(ctx, st.best, st.done, st.dev_ms, out_mask, res);
 }
 
+// Routing of problems [p0, p1) of a batch call, from the host offsets alone.  A problem that fits one block takes batch_kernel
+// (max_n is taken over those problems only); a larger one a cluster of C CTAs, the smallest that holds it.  cl[k] lists the
+// problems (relative to p0) of cluster size 2 << k, cl_slice[k] the largest slice among them; cl_all is cl[0..3] back to back,
+// the list the cluster launches read on the device.
+struct BatchPlan {
+  BatchLimits L;
+  bool use32;                // fp32 scoring keeps an fp32 copy of the points next to the fp64 one
+  uint32_t max_n = 1;
+  std::vector<uint32_t> cl[4];
+  uint32_t cl_slice[4] = {0, 0, 0, 0};
+  std::vector<uint32_t> cl_all;
+};
+int plan_batch(lsqr_ctx* ctx, const uint64_t* offsets, uint64_t p0, uint64_t p1, int exhaustive, int precision, BatchPlan* plan) {
+  CK(cudaSetDevice(ctx->device));
+  BatchPlan& P = *plan;
+  P.use32 = precision == LSQR_FP32 && !exhaustive;
+  const BatchLimits L = P.L = batch_limits(ctx->model, P.use32 ? 1 : 0, exhaustive);
+  for (uint64_t b = p0; b < p1; b++) {
+    if (offsets[b + 1] < offsets[b]) return fail(ctx, LSQR_ERR_ARG, "offsets must be non-decreasing");
+    const uint64_t nb = offsets[b + 1] - offsets[b];
+    if (nb <= L.one_block) { P.max_n = std::max<uint64_t>(P.max_n, nb); continue; }
+    if (L.max_cluster == 0) return fail(ctx, LSQR_ERR_ARG, "a problem does not fit in shared memory; use lsqr_ransac for large problems");
+    if (nb > L.max_records)
+      return fail(ctx, LSQR_ERR_ARG, "a problem of " + std::to_string(nb) + " records exceeds the batch limit of " + std::to_string(L.max_records) +
+                                         " records for this model and precision; use lsqr_compute for larger problems");
+    const uint32_t c = batch_cluster_size(L, nb);
+    const int k = c == 2 ? 0 : c == 4 ? 1 : c == 8 ? 2 : 3;
+    P.cl[k].push_back((uint32_t)(b - p0));
+    P.cl_slice[k] = std::max<uint32_t>(P.cl_slice[k], (uint32_t)(((nb + c - 1) / c + 1) & ~1ull));
+  }
+  for (const auto& v : P.cl) P.cl_all.insert(P.cl_all.end(), v.begin(), v.end());
+  return LSQR_OK;
+}
+
+// The plan's large problems: one cluster launch per cluster size.  `ba` locates the data, offsets and outputs of the whole
+// call; cl_dev holds plan.cl_all on the device.  With `tev`, each launch is bracketed by a pair of timing events appended to it
+// (all of them destroyed if a launch fails).
+int launch_clusters(lsqr_ctx* ctx, const BatchPlan& plan, BatchArgs ba, const uint32_t* cl_dev, cudaStream_t s, std::vector<cudaEvent_t>* tev) {
+  size_t first = 0;
+  for (int k = 0; k < 4; k++) {
+    if (plan.cl[k].empty()) continue;
+    ba.n_problems = (uint32_t)plan.cl[k].size();
+    cudaEvent_t e0, e1;
+    if (tev) {
+      CK(cudaEventCreate(&e0)); tev->push_back(e0);
+      CK(cudaEventCreate(&e1)); tev->push_back(e1);
+      CK(cudaEventRecord(e0, s));
+    }
+    if (launch_batch_cluster(ba, cl_dev + first, ba.n_problems, 2u << k, plan.cl_slice[k], ctx->cfg, ctx->ls_type, s) < 0) {
+      if (tev) for (cudaEvent_t e : *tev) cudaEventDestroy(e);
+      return fail(ctx, LSQR_ERR_CUDA, std::string("batch cluster launch: ") + cudaGetErrorString(cudaGetLastError()));
+    }
+    ctx->launches++;
+    if (tev) CK(cudaEventRecord(e1, s));
+    first += plan.cl[k].size();
+  }
+  return LSQR_OK;
+}
+
 // problems [p0, p1) of a batch (offsets are absolute record offsets into `data`)
 int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint64_t p0, uint64_t p1, int exhaustive, double prob, uint32_t max_tries,
                uint64_t seed, int precision, double* out_params, uint32_t* out_counts, uint8_t* out_masks, double* device_ms) {
@@ -983,29 +1048,9 @@ int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint6
   const uint64_t np = p1 - p0;
   if (np > 0x7FFFFFFFull) return fail(ctx, LSQR_ERR_ARG, "too many problems");
   const ModelInfo mi = model_info(ctx->model);
-  CK(cudaSetDevice(ctx->device));
+  BatchPlan plan;
+  if (int rc = plan_batch(ctx, offsets, p0, p1, exhaustive, precision, &plan)) return rc;
   const uint64_t base = offsets[p0], total = offsets[p1] - base;
-  const bool use32 = precision == LSQR_FP32 && !exhaustive;   // fp32 scoring keeps an fp32 copy of the points next to the fp64 one
-  // A problem that fits one block takes batch_kernel (max_n is taken over those problems only); a larger one a cluster of
-  // C CTAs, the smallest that holds it.  cl[k] lists the problems (relative to p0) of cluster size 2 << k, cl_slice[k] the
-  // largest slice among them.
-  const BatchLimits L = batch_limits(ctx->model, use32 ? 1 : 0, exhaustive);
-  uint32_t max_n = 1;
-  std::vector<uint32_t> cl[4];
-  uint32_t cl_slice[4] = {0, 0, 0, 0};
-  for (uint64_t b = p0; b < p1; b++) {
-    if (offsets[b + 1] < offsets[b]) return fail(ctx, LSQR_ERR_ARG, "offsets must be non-decreasing");
-    const uint64_t nb = offsets[b + 1] - offsets[b];
-    if (nb <= L.one_block) { max_n = std::max<uint64_t>(max_n, nb); continue; }
-    if (L.max_cluster == 0) return fail(ctx, LSQR_ERR_ARG, "a problem does not fit in shared memory; use lsqr_ransac for large problems");
-    if (nb > L.max_records)
-      return fail(ctx, LSQR_ERR_ARG, "a problem of " + std::to_string(nb) + " records exceeds the batch limit of " + std::to_string(L.max_records) +
-                                         " records for this model and precision; use lsqr_compute for larger problems");
-    const uint32_t c = batch_cluster_size(L, nb);
-    const int k = c == 2 ? 0 : c == 4 ? 1 : c == 8 ? 2 : 3;
-    cl[k].push_back((uint32_t)(b - p0));
-    cl_slice[k] = std::max<uint32_t>(cl_slice[k], (uint32_t)(((nb + c - 1) / c + 1) & ~1ull));
-  }
   cudaStream_t s = ctx->stream;
   // persistent buffers (a cudaMalloc/cudaFree set per call cost more than the kernel)
   if (int rc = ensure(ctx, &ctx->bt_data, &ctx->bt_data_cap, (size_t)std::max<uint64_t>(total, 1) * mi.D)) return rc;
@@ -1036,11 +1081,11 @@ int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint6
     }
     if (nrec) if (int rc = up.landed()) return rc;
     bool any_small = false;
-    for (uint64_t b = q0; b < q1 && !any_small; b++) any_small = offsets[b + 1] - offsets[b] <= L.one_block;
+    for (uint64_t b = q0; b < q1 && !any_small; b++) any_small = offsets[b + 1] - offsets[b] <= plan.L.one_block;
     if (!any_small) { q0 = q1; continue; }   // every problem of this piece takes the cluster path
     BatchArgs ba{};
-    ba.model = ctx->model; ba.exhaustive = exhaustive; ba.precision = use32 ? 1 : 0; ba.tries = max_tries; ba.prob = prob; ba.seed = seed;
-    ba.data = ctx->bt_data + rec0 * mi.D; ba.offsets = ctx->bt_off + (q0 - p0); ba.n_problems = (uint32_t)(q1 - q0); ba.max_n = max_n;
+    ba.model = ctx->model; ba.exhaustive = exhaustive; ba.precision = plan.use32 ? 1 : 0; ba.tries = max_tries; ba.prob = prob; ba.seed = seed;
+    ba.data = ctx->bt_data + rec0 * mi.D; ba.offsets = ctx->bt_off + (q0 - p0); ba.n_problems = (uint32_t)(q1 - q0); ba.max_n = plan.max_n;
     ba.base = offsets[q0]; ba.first_problem = q0;
     ba.out_params = ctx->bt_prm + (q0 - p0) * mi.P; ba.out_counts = ctx->bt_cnt + (q0 - p0); ba.out_masks = out_masks ? ctx->mask_dev + rec0 : nullptr;
     cudaEvent_t e0, e1;
@@ -1052,32 +1097,15 @@ int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint6
     CK(cudaEventRecord(e1, s));
     q0 = q1;
   }
-  // the large problems, once every piece has landed: one launch per cluster size
-  std::vector<uint32_t> cl_all;
-  for (const auto& v : cl) cl_all.insert(cl_all.end(), v.begin(), v.end());
-  if (!cl_all.empty()) {
-    if (int rc = ensure(ctx, &ctx->bt_cl, &ctx->bt_cl_cap, cl_all.size())) return rc;
-    CK(cudaMemcpyAsync(ctx->bt_cl, cl_all.data(), sizeof(uint32_t) * cl_all.size(), cudaMemcpyHostToDevice, s));
+  // the large problems, once every piece has landed
+  if (!plan.cl_all.empty()) {
+    if (int rc = ensure(ctx, &ctx->bt_cl, &ctx->bt_cl_cap, plan.cl_all.size())) return rc;
+    CK(cudaMemcpyAsync(ctx->bt_cl, plan.cl_all.data(), sizeof(uint32_t) * plan.cl_all.size(), cudaMemcpyHostToDevice, s));
     BatchArgs ba{};
-    ba.model = ctx->model; ba.precision = use32 ? 1 : 0; ba.tries = max_tries; ba.prob = prob; ba.seed = seed;
+    ba.model = ctx->model; ba.precision = plan.use32 ? 1 : 0; ba.tries = max_tries; ba.prob = prob; ba.seed = seed;
     ba.data = ctx->bt_data; ba.offsets = ctx->bt_off; ba.base = base; ba.first_problem = p0;
     ba.out_params = ctx->bt_prm; ba.out_counts = ctx->bt_cnt; ba.out_masks = out_masks ? ctx->mask_dev : nullptr;
-    size_t first = 0;
-    for (int k = 0; k < 4; k++) {
-      if (cl[k].empty()) continue;
-      ba.n_problems = (uint32_t)cl[k].size();
-      cudaEvent_t e0, e1;
-      CK(cudaEventCreate(&e0)); tev.push_back(e0);
-      CK(cudaEventCreate(&e1)); tev.push_back(e1);
-      CK(cudaEventRecord(e0, s));
-      if (launch_batch_cluster(ba, ctx->bt_cl + first, ba.n_problems, 2u << k, cl_slice[k], ctx->cfg, ctx->ls_type, s) < 0) {
-        for (cudaEvent_t e : tev) cudaEventDestroy(e);
-        return fail(ctx, LSQR_ERR_CUDA, std::string("batch cluster launch: ") + cudaGetErrorString(cudaGetLastError()));
-      }
-      ctx->launches++;
-      CK(cudaEventRecord(e1, s));
-      first += cl[k].size();
-    }
+    if (int rc = launch_clusters(ctx, plan, ba, ctx->bt_cl, s, &tev)) return rc;
   }
   CKL();
   CK(cudaMemcpyAsync(out_params + p0 * mi.P, ctx->bt_prm, sizeof(double) * np * mi.P, cudaMemcpyDeviceToHost, s));
@@ -1088,6 +1116,51 @@ int batch_impl(lsqr_ctx* ctx, const double* data, const uint64_t* offsets, uint6
   for (size_t i = 0; i + 1 < tev.size(); i += 2) { float ms = 0.f; if (cudaEventElapsedTime(&ms, tev[i], tev[i + 1]) == cudaSuccess) total_ms += ms; }
   for (cudaEvent_t e : tev) cudaEventDestroy(e);
   if (device_ms) *device_ms = total_ms;
+  return LSQR_OK;
+}
+
+// `p` is memory of this context's device (not page-locked or pageable host memory, not managed memory, not another GPU's),
+// aligned to `align` bytes
+int check_device_ptr(lsqr_ctx* ctx, const void* p, size_t align, const char* name) {
+  cudaPointerAttributes attr{};
+  const bool ok = p && cudaPointerGetAttributes(&attr, p) == cudaSuccess && attr.type == cudaMemoryTypeDevice && attr.device == ctx->device;
+  if (!ok) cudaGetLastError();   // a refused query is an answer here, not an error of the next call
+  if (!ok) return fail(ctx, LSQR_ERR_ARG, std::string(name) + " is not device memory of device " + std::to_string(ctx->device));
+  if (reinterpret_cast<uintptr_t>(p) % align) return fail(ctx, LSQR_ERR_ARG, std::string(name) + " is not aligned to " + std::to_string(align) + " bytes");
+  return LSQR_OK;
+}
+
+// lsqr_ransac_batch_device on stream s, which the caller has ordered after the context's stream.  All one-block problems go in
+// one batch_kernel launch: there is no copy for smaller launches to hide behind.
+int batch_device_enqueue(lsqr_ctx* ctx, const BatchPlan& plan, const double* dev_data, const uint64_t* offsets, uint64_t np, int exhaustive,
+                         double prob, uint32_t max_tries, uint64_t seed, double* dev_params, uint32_t* dev_counts, uint8_t* dev_masks,
+                         cudaStream_t s) {
+  const ModelInfo mi = model_info(ctx->model);
+  // growing these may synchronise the device (cudaFree); the sizes of one call repeated do not grow them
+  if (int rc = ensure(ctx, &ctx->bt_off, &ctx->bt_off_cap, (size_t)np + 1)) return rc;
+  if (!plan.cl_all.empty()) if (int rc = ensure(ctx, &ctx->bt_cl, &ctx->bt_cl_cap, plan.cl_all.size())) return rc;
+  // the slot's previous copies belong to the call before last: this waits only while that call's copies are still queued
+  const int slot = (int)(ctx->bd_calls++ & 1);
+  CK(cudaEventSynchronize(ctx->bd_ev[slot]));
+  const size_t off_bytes = sizeof(uint64_t) * (np + 1), cl_bytes = sizeof(uint32_t) * plan.cl_all.size();
+  if (int rc = ensure_pinned(ctx, &ctx->bd_pin[slot], &ctx->bd_pin_cap[slot], off_bytes + cl_bytes)) return rc;
+  memcpy(ctx->bd_pin[slot], offsets, off_bytes);
+  if (cl_bytes) memcpy(ctx->bd_pin[slot] + off_bytes, plan.cl_all.data(), cl_bytes);
+  CK(cudaMemcpyAsync(ctx->bt_off, ctx->bd_pin[slot], off_bytes, cudaMemcpyHostToDevice, s));
+  if (cl_bytes) CK(cudaMemcpyAsync(ctx->bt_cl, ctx->bd_pin[slot] + off_bytes, cl_bytes, cudaMemcpyHostToDevice, s));
+  CK(cudaEventRecord(ctx->bd_ev[slot], s));
+  const uint64_t base = offsets[0];
+  BatchArgs ba{};
+  ba.model = ctx->model; ba.exhaustive = exhaustive; ba.precision = plan.use32 ? 1 : 0; ba.tries = max_tries; ba.prob = prob; ba.seed = seed;
+  ba.data = dev_data + base * mi.D; ba.offsets = ctx->bt_off; ba.base = base; ba.first_problem = 0; ba.max_n = plan.max_n;
+  ba.out_params = dev_params; ba.out_counts = dev_counts; ba.out_masks = dev_masks ? dev_masks + base : nullptr;
+  if (plan.cl_all.size() < np) {   // some problem fits one block (batch_kernel returns at once for the others)
+    ba.n_problems = (uint32_t)np;
+    if (launch_batch(ba, ctx->cfg, ctx->ls_type, s) < 0) return fail(ctx, LSQR_ERR_ARG, "batch launch rejected");
+    ctx->launches++;
+  }
+  if (int rc = launch_clusters(ctx, plan, ba, ctx->bt_cl, s, nullptr)) return rc;
+  CKL();
   return LSQR_OK;
 }
 
@@ -1117,6 +1190,8 @@ int create_single(lsqr_ctx** out, int device) {
   for (int i = 0; ok && i < 6; i++) ok = cudaEventCreate(&ctx->ev[i]) == cudaSuccess;
   for (int i = 0; ok && i < lsqr_ctx::kRing; i++) ok = cudaEventCreateWithFlags(&ctx->up_ev[i], cudaEventDisableTiming) == cudaSuccess;
   for (int i = 0; ok && i < 8; i++) ok = cudaEventCreateWithFlags(&ctx->up_land[i], cudaEventDisableTiming) == cudaSuccess;
+  for (int i = 0; ok && i < 2; i++) ok = cudaEventCreateWithFlags(&ctx->bd_ev[i], cudaEventDisableTiming) == cudaSuccess &&
+                                         cudaEventCreateWithFlags(&ctx->bd_order[i], cudaEventDisableTiming) == cudaSuccess;
   if (!ok) return bail(LSQR_ERR_CUDA);
   *out = ctx;
   return LSQR_OK;
@@ -1240,6 +1315,11 @@ void lsqr_ctx_destroy(lsqr_ctx* ctx) {
   for (int i = 0; i < 6; i++) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
   for (int i = 0; i < lsqr_ctx::kRing; i++) if (ctx->up_ev[i]) cudaEventDestroy(ctx->up_ev[i]);
   for (int i = 0; i < 8; i++) if (ctx->up_land[i]) cudaEventDestroy(ctx->up_land[i]);
+  for (int i = 0; i < 2; i++) {
+    if (ctx->bd_pin[i]) cudaFreeHost(ctx->bd_pin[i]);
+    if (ctx->bd_ev[i]) cudaEventDestroy(ctx->bd_ev[i]);
+    if (ctx->bd_order[i]) cudaEventDestroy(ctx->bd_order[i]);
+  }
   if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
   if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
@@ -1426,6 +1506,39 @@ int lsqr_ransac_batch(lsqr_ctx* ctx, const double* data, const uint64_t* offsets
     return rc;
   }
   return batch_impl(ctx, data, offsets, 0, n_problems, exhaustive, prob, max_tries, seed, precision, out_params, out_counts, out_masks, device_ms);
+}
+
+int lsqr_ransac_batch_device(lsqr_ctx* ctx, const double* dev_data, const uint64_t* offsets, uint64_t n_problems, int exhaustive, double prob,
+                             uint32_t max_tries, uint64_t seed, int precision, double* dev_params, uint32_t* dev_counts, uint8_t* dev_masks,
+                             void* cuda_stream) {
+  if (!ctx || !offsets) return LSQR_ERR_ARG;
+  if (ctx->group) return fail(ctx, LSQR_ERR_ARG, "a device buffer belongs to one GPU; a multi-GPU group takes host batches (lsqr_ransac_batch)");
+  if (precision != LSQR_FP64 && precision != LSQR_FP32) return fail(ctx, LSQR_ERR_ARG, "bad precision");
+  if (n_problems == 0) return LSQR_OK;
+  if (ctx->model < 0) return fail(ctx, LSQR_ERR_STATE, "lsqr_set_estimator must be called first");
+  if (n_problems > 0x7FFFFFFFull) return fail(ctx, LSQR_ERR_ARG, "too many problems");
+  BatchPlan plan;
+  if (int rc = plan_batch(ctx, offsets, 0, n_problems, exhaustive, precision, &plan)) return rc;
+  const bool records = offsets[n_problems] > offsets[0];   // data and masks are neither read nor written when every problem is empty
+  if (records) if (int rc = check_device_ptr(ctx, dev_data, alignof(double), "dev_data")) return rc;
+  if (int rc = check_device_ptr(ctx, dev_params, alignof(double), "dev_params")) return rc;
+  if (int rc = check_device_ptr(ctx, dev_counts, alignof(uint32_t), "dev_counts")) return rc;
+  if (dev_masks && records) if (int rc = check_device_ptr(ctx, dev_masks, 1, "dev_masks")) return rc;
+  // bt_off and bt_cl are shared with every other call on the context: work on another stream is ordered after the context's
+  // stream at entry, and the context's stream after it at exit (also when enqueueing failed half-way)
+  cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
+  const bool side = s != ctx->stream;
+  if (side) {
+    CK(cudaEventRecord(ctx->bd_order[0], ctx->stream));
+    CK(cudaStreamWaitEvent(s, ctx->bd_order[0], 0));
+  }
+  const int rc = batch_device_enqueue(ctx, plan, dev_data, offsets, n_problems, exhaustive, prob, max_tries, seed, dev_params, dev_counts,
+                                      dev_masks, s);
+  if (side) {
+    CK(cudaEventRecord(ctx->bd_order[1], s));
+    CK(cudaStreamWaitEvent(ctx->stream, ctx->bd_order[1], 0));
+  }
+  return rc;
 }
 
 int lsqr_batch_capacity(lsqr_ctx* ctx, int precision, int exhaustive, uint64_t* one_block, uint64_t* max_records) {
