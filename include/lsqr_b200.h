@@ -283,6 +283,25 @@ int lsqr_least_squares(lsqr_ctx* ctx, const double* packed, size_t n, double* ou
 /* AbsoluteOrientationParametersEstimator::weightedLeastSquaresEstimate (AbsoluteOrientationParametersEstimator.cxx:208-297):
  * Horn's method with one weight per pair; LSQR_ABSOR contexts only; *n_params = 0 for fewer than 3 pairs. */
 int lsqr_weighted_least_squares(lsqr_ctx* ctx, const double* packed, size_t n, const double* weights, double* out_params, int* n_params);
+/* leastSquaresEstimate() of every problem of a batch in device memory, stream-ordered: what lsqr_least_squares (or, with
+ * weights, lsqr_weighted_least_squares) returns for each problem's selected records.
+ * dev_data and offsets as for lsqr_ransac_batch_device: packed doubles [offsets[n_problems]][dim] in device memory (may be
+ * NULL when every problem is empty) and a HOST array [n_problems+1] of absolute record offsets.
+ * dev_masks: optional, one byte per record with the same indexing as the data; a record is used when its byte is non-zero
+ * (leastSquaresEstimate over a consensus set, RANSAC.hxx:138).  The masks lsqr_ransac_batch_device writes can be passed back.
+ * dev_weights: optional, one double per record with the same indexing, LSQR_ABSOR only: weightedLeastSquaresEstimate over the
+ * selected pairs (a masked-out pair is neither weighted nor counted).
+ * dev_params [n_problems][P]: a NaN row is the reference's empty parameter vector.  Size guards are counted on the selected
+ * records: fewer than k gives NaN (except LSQR_RAY), weighted Horn with fewer than 3 pairs gives NaN.  The hyperspheres with
+ * LSQR_LS_GEOMETRIC run the algebraic fit and then the Levenberg-Marquardt controller of lsqr_least_squares.
+ * Moments are taken relative to each problem's first record; the records are streamed from device memory, so there is no
+ * size limit below 2^32 - 1 records per problem.  A problem's result depends only on its records (and the device's largest
+ * thread-block cluster), not on the other problems of the call or its position.
+ * Stream semantics, pointer checks and ordering against the context's work are those of lsqr_ransac_batch_device.
+ * LSQR_ERR_ARG: a pointer that is not device memory of this context's device, weights on a model other than LSQR_ABSOR, the
+ * ultrasound calibrations (no batched mode), decreasing offsets, a problem above 2^32 - 1 records, a multi-GPU group context. */
+int lsqr_least_squares_batch_device(lsqr_ctx* ctx, const double* dev_data, const uint64_t* offsets, uint64_t n_problems,
+                                    const uint8_t* dev_masks, const double* dev_weights, double* dev_params, void* cuda_stream);
 
 /* ---- measurement helpers ------------------------------------------------------------ */
 /* Register-resident FMA-chain microbenchmarks: returns lane-FMA/s of the fp32 (kind 0),

@@ -106,6 +106,8 @@ def load_library():
         "lsqr_batch_capacity": (c.c_int, [c.c_void_p, c.c_int, c.c_int, _u64p, _u64p]),
         "lsqr_ransac_batch_device": (c.c_int, [c.c_void_p, c.c_void_p, _u64p, c.c_uint64, c.c_int, c.c_double, c.c_uint32, c.c_uint64, c.c_int,
                                                c.c_void_p, c.c_void_p, c.c_void_p, c.c_void_p]),
+        "lsqr_least_squares_batch_device": (c.c_int, [c.c_void_p, c.c_void_p, _u64p, c.c_uint64, c.c_void_p, c.c_void_p, c.c_void_p,
+                                                      c.c_void_p]),
         "lsqr_estimate": (c.c_int, [c.c_void_p, _dp, c.c_size_t, _dp, c.POINTER(c.c_int)]),
         "lsqr_agree": (c.c_int, [c.c_void_p, _dp, _dp, c.c_size_t, _u8p]),
         "lsqr_least_squares": (c.c_int, [c.c_void_p, _dp, c.c_size_t, _dp, c.POINTER(c.c_int)]),
@@ -129,7 +131,7 @@ EXPORTED_SYMBOLS = [
     "lsqr_microbench_fma", "lsqr_last_refine_stats", "lsqr_weighted_least_squares",
     "lsqr_device_count", "lsqr_ctx_create_multi", "lsqr_ctx_world", "lsqr_nccl_unique_id", "lsqr_ctx_init_nccl", "lsqr_get_mask_bits",
     "lsqr_compute", "lsqr_bench_refine_pass", "lsqr_model_plane", "lsqr_model_sphere", "lsqr_model_line", "lsqr_model_dense",
-    "lsqr_batch_capacity", "lsqr_ransac_batch_device",
+    "lsqr_batch_capacity", "lsqr_ransac_batch_device", "lsqr_least_squares_batch_device",
 ]
 
 
@@ -181,6 +183,37 @@ def check_batch_device_args(data, offsets, dim, device_index=None):
     if device_index is not None and data.device.index != device_index:
         raise ValueError(f"data is on {data.device}; the engine runs on cuda:{device_index}")
     return data, off
+
+
+def check_ls_batch_device_args(data, offsets, dim, model, masks=None, weights=None, device_index=None):
+    """The arguments of Engine.least_squares_batch_device: `data` and `offsets` as check_batch_device_args takes them; `masks`
+    (optional) a contiguous torch.uint8 or torch.bool CUDA tensor and `weights` (optional, absolute orientation only) a contiguous
+    torch.float64 CUDA tensor, each [total] for the [total, dim] layout or [B, n] for [B, n, dim], on the device of `data`.
+    Everything but the devices is checked before the data's device, so no device is needed to find a malformed argument.
+    Returns the data as [total, dim], the offsets as a uint64 numpy array and masks and weights flattened.  Raises ValueError."""
+    import torch
+    if weights is not None and model != MODELS["absor"]:
+        raise ValueError("weights exist for the absolute-orientation estimator (absor) only")
+    if isinstance(data, torch.Tensor):
+        shape = tuple(data.shape[:2]) if data.dim() == 3 and offsets is None else tuple(data.shape[:1])
+        for what, t, dtypes in (("masks", masks, (torch.uint8, torch.bool)), ("weights", weights, (torch.float64,))):
+            if t is None:
+                continue
+            if not isinstance(t, torch.Tensor):
+                raise ValueError(f"{what} must be a torch tensor in CUDA memory")
+            if t.dtype not in dtypes:
+                raise ValueError(f"{what} must be {' or '.join(str(d) for d in dtypes)}, not {t.dtype}")
+            if not t.is_contiguous():
+                raise ValueError(f"{what} must be contiguous")
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{what} must have shape {list(shape)} (one entry per record of data), not {list(t.shape)}")
+    data, off = check_batch_device_args(data, offsets, dim, device_index)
+    out = []
+    for what, t in (("masks", masks), ("weights", weights)):
+        if t is not None and t.device != data.device:
+            raise ValueError(f"{what} must be in CUDA memory on {data.device}, not on {t.device}")
+        out.append(t.reshape(-1) if t is not None else None)
+    return data, off, out[0], out[1]
 
 
 class Engine:
@@ -429,6 +462,21 @@ class Engine:
         n = ctypes.c_int(0)
         self._ck(self.lib.lsqr_weighted_least_squares(self.h, _ptr(d, _dp), d.shape[0], _ptr(w, _dp), _ptr(out, _dp), ctypes.byref(n)))
         return out[: n.value].copy()
+
+    def least_squares_batch_device(self, data, offsets=None, masks=None, weights=None):
+        """least_squares (weighted_least_squares with `weights`, absor only) of every problem of a batch in a torch.float64 CUDA
+        tensor on the engine's device: [total, dim] with host `offsets`, or [B, n, dim] without.  `masks` (uint8 or bool, [total]
+        or [B, n]) selects the records each fit uses -- e.g. the masks of ransac_batch_device; `weights` (float64, same shape)
+        weigh them.  Returns params [B, P] float64 (NaN row = empty), enqueued on torch.cuda.current_stream() and not waited
+        for."""
+        import torch
+        d, off, m, w = check_ls_batch_device_args(data, offsets, self.dim, self.model, masks, weights, self.device)
+        prm = torch.empty((len(off) - 1, self.n_params), dtype=torch.float64, device=d.device)
+        stream = torch.cuda.current_stream(d.device).cuda_stream or _CUDA_STREAM_LEGACY
+        self._ck(self.lib.lsqr_least_squares_batch_device(self.h, d.data_ptr(), _ptr(off, _u64p), len(off) - 1,
+                                                          m.data_ptr() if m is not None else None,
+                                                          w.data_ptr() if w is not None else None, prm.data_ptr(), stream))
+        return prm
 
     # -- measurement ------------------------------------------------------------------
     def microbench_fma(self, kind, iters=4096):

@@ -36,7 +36,8 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
 // initialises the barriers and issues one bulk copy per row.  Every thread of the block runs
 //   ring.start();
 //   for (uint32_t t = t0; t < t1; t++) { const T* tile = ring.wait(t); /* row d at tile[d * TILE] */ ring.release(); }
-// and release() synchronises the block, so a buffer is refilled only when everyone is done with it.  (The loop stays with the
+// and release() synchronises the block, so a buffer is refilled only when everyone is done with it.  restart() instead of start()
+// walks the tiles once more.  (The loop stays with the
 // caller: with the tile body in a lambda, ptxas allocates the fp64 kernel's registers differently.)
 template <int D, int TILE, class T>
 struct TileRing {
@@ -58,6 +59,10 @@ struct TileRing {
   __device__ __forceinline__ void start() {
     if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); mbar_fence_init(); }
     __syncthreads();
+    if (tid == 0 && t0 < t1) issue(t0, 0);
+  }
+  // walks [t0, t1) again with the initialised barriers (their phases carry on); every thread has released the last tile
+  __device__ __forceinline__ void restart() {
     if (tid == 0 && t0 < t1) issue(t0, 0);
   }
   // issues tile t + 1 into the other buffer, then waits for tile t

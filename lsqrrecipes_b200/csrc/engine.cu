@@ -1130,25 +1130,50 @@ int check_device_ptr(lsqr_ctx* ctx, const void* p, size_t align, const char* nam
   return LSQR_OK;
 }
 
+// The device entry points: `enqueue(s)` on the caller's stream (the context's when cuda_stream is null).  bt_off, bt_cl and the
+// page-locked slots are shared with every other call on the context: work on another stream is ordered after the context's
+// stream at entry, and the context's stream after it at exit (also when enqueueing failed half-way).
+template <class Enqueue> int on_caller_stream(lsqr_ctx* ctx, void* cuda_stream, const Enqueue& enqueue) {
+  cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
+  const bool side = s != ctx->stream;
+  if (side) {
+    CK(cudaEventRecord(ctx->bd_order[0], ctx->stream));
+    CK(cudaStreamWaitEvent(s, ctx->bd_order[0], 0));
+  }
+  const int rc = enqueue(s);
+  if (side) {
+    CK(cudaEventRecord(ctx->bd_order[1], s));
+    CK(cudaStreamWaitEvent(ctx->stream, ctx->bd_order[1], 0));
+  }
+  return rc;
+}
+
+// The host offsets (np + 1) -> bt_off and the problem list -> bt_cl on stream s, through one of the two page-locked slots (a copy
+// from pageable memory may wait for the stream).  The slot's previous copies belong to the call before last: this waits only
+// while that call's copies are still queued.  Growing the device buffers may synchronise the device (cudaFree); the sizes of one
+// call repeated do not grow them.
+int stage_offsets(lsqr_ctx* ctx, const uint64_t* offsets, uint64_t np, const std::vector<uint32_t>& list, cudaStream_t s) {
+  if (int rc = ensure(ctx, &ctx->bt_off, &ctx->bt_off_cap, (size_t)np + 1)) return rc;
+  if (!list.empty()) if (int rc = ensure(ctx, &ctx->bt_cl, &ctx->bt_cl_cap, list.size())) return rc;
+  const int slot = (int)(ctx->bd_calls++ & 1);
+  CK(cudaEventSynchronize(ctx->bd_ev[slot]));
+  const size_t off_bytes = sizeof(uint64_t) * (np + 1), cl_bytes = sizeof(uint32_t) * list.size();
+  if (int rc = ensure_pinned(ctx, &ctx->bd_pin[slot], &ctx->bd_pin_cap[slot], off_bytes + cl_bytes)) return rc;
+  memcpy(ctx->bd_pin[slot], offsets, off_bytes);
+  if (cl_bytes) memcpy(ctx->bd_pin[slot] + off_bytes, list.data(), cl_bytes);
+  CK(cudaMemcpyAsync(ctx->bt_off, ctx->bd_pin[slot], off_bytes, cudaMemcpyHostToDevice, s));
+  if (cl_bytes) CK(cudaMemcpyAsync(ctx->bt_cl, ctx->bd_pin[slot] + off_bytes, cl_bytes, cudaMemcpyHostToDevice, s));
+  CK(cudaEventRecord(ctx->bd_ev[slot], s));
+  return LSQR_OK;
+}
+
 // lsqr_ransac_batch_device on stream s, which the caller has ordered after the context's stream.  All one-block problems go in
 // one batch_kernel launch: there is no copy for smaller launches to hide behind.
 int batch_device_enqueue(lsqr_ctx* ctx, const BatchPlan& plan, const double* dev_data, const uint64_t* offsets, uint64_t np, int exhaustive,
                          double prob, uint32_t max_tries, uint64_t seed, double* dev_params, uint32_t* dev_counts, uint8_t* dev_masks,
                          cudaStream_t s) {
   const ModelInfo mi = model_info(ctx->model);
-  // growing these may synchronise the device (cudaFree); the sizes of one call repeated do not grow them
-  if (int rc = ensure(ctx, &ctx->bt_off, &ctx->bt_off_cap, (size_t)np + 1)) return rc;
-  if (!plan.cl_all.empty()) if (int rc = ensure(ctx, &ctx->bt_cl, &ctx->bt_cl_cap, plan.cl_all.size())) return rc;
-  // the slot's previous copies belong to the call before last: this waits only while that call's copies are still queued
-  const int slot = (int)(ctx->bd_calls++ & 1);
-  CK(cudaEventSynchronize(ctx->bd_ev[slot]));
-  const size_t off_bytes = sizeof(uint64_t) * (np + 1), cl_bytes = sizeof(uint32_t) * plan.cl_all.size();
-  if (int rc = ensure_pinned(ctx, &ctx->bd_pin[slot], &ctx->bd_pin_cap[slot], off_bytes + cl_bytes)) return rc;
-  memcpy(ctx->bd_pin[slot], offsets, off_bytes);
-  if (cl_bytes) memcpy(ctx->bd_pin[slot] + off_bytes, plan.cl_all.data(), cl_bytes);
-  CK(cudaMemcpyAsync(ctx->bt_off, ctx->bd_pin[slot], off_bytes, cudaMemcpyHostToDevice, s));
-  if (cl_bytes) CK(cudaMemcpyAsync(ctx->bt_cl, ctx->bd_pin[slot] + off_bytes, cl_bytes, cudaMemcpyHostToDevice, s));
-  CK(cudaEventRecord(ctx->bd_ev[slot], s));
+  if (int rc = stage_offsets(ctx, offsets, np, plan.cl_all, s)) return rc;
   const uint64_t base = offsets[0];
   BatchArgs ba{};
   ba.model = ctx->model; ba.exhaustive = exhaustive; ba.precision = plan.use32 ? 1 : 0; ba.tries = max_tries; ba.prob = prob; ba.seed = seed;
@@ -1524,21 +1549,52 @@ int lsqr_ransac_batch_device(lsqr_ctx* ctx, const double* dev_data, const uint64
   if (int rc = check_device_ptr(ctx, dev_params, alignof(double), "dev_params")) return rc;
   if (int rc = check_device_ptr(ctx, dev_counts, alignof(uint32_t), "dev_counts")) return rc;
   if (dev_masks && records) if (int rc = check_device_ptr(ctx, dev_masks, 1, "dev_masks")) return rc;
-  // bt_off and bt_cl are shared with every other call on the context: work on another stream is ordered after the context's
-  // stream at entry, and the context's stream after it at exit (also when enqueueing failed half-way)
-  cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
-  const bool side = s != ctx->stream;
-  if (side) {
-    CK(cudaEventRecord(ctx->bd_order[0], ctx->stream));
-    CK(cudaStreamWaitEvent(s, ctx->bd_order[0], 0));
+  return on_caller_stream(ctx, cuda_stream, [&](cudaStream_t s) {
+    return batch_device_enqueue(ctx, plan, dev_data, offsets, n_problems, exhaustive, prob, max_tries, seed, dev_params, dev_counts, dev_masks, s);
+  });
+}
+
+int lsqr_least_squares_batch_device(lsqr_ctx* ctx, const double* dev_data, const uint64_t* offsets, uint64_t n_problems, const uint8_t* dev_masks,
+                                    const double* dev_weights, double* dev_params, void* cuda_stream) {
+  if (!ctx || !offsets) return LSQR_ERR_ARG;
+  if (ctx->group) return fail(ctx, LSQR_ERR_ARG, "a device buffer belongs to one GPU; a multi-GPU group has no batched least squares");
+  if (n_problems == 0) return LSQR_OK;
+  if (ctx->model < 0) return fail(ctx, LSQR_ERR_STATE, "lsqr_set_estimator must be called first");
+  if (ctx->model == USXW || ctx->model == USCP) return fail(ctx, LSQR_ERR_ARG, "the ultrasound calibrations have no batched mode");
+  if (dev_weights && ctx->model != ABSOR) return fail(ctx, LSQR_ERR_ARG, "dev_weights: weighted least squares exists for the absolute-orientation estimator only");
+  if (n_problems > 0x7FFFFFFFull) return fail(ctx, LSQR_ERR_ARG, "too many problems");
+  CK(cudaSetDevice(ctx->device));
+  // route by size alone: the problems of cluster size 1 << k in by[k], then all of them back to back in `list`
+  const int cmax = ls_batch_max_cluster(ctx->model, dev_weights != nullptr);
+  std::vector<uint32_t> by[5], list;
+  for (uint64_t b = 0; b < n_problems; b++) {
+    if (offsets[b + 1] < offsets[b]) return fail(ctx, LSQR_ERR_ARG, "offsets must be non-decreasing");
+    const uint64_t nb = offsets[b + 1] - offsets[b];
+    if (nb > 0xFFFFFFFFull) return fail(ctx, LSQR_ERR_ARG, "a problem of " + std::to_string(nb) + " records exceeds the limit of 2^32 - 1 records");
+    const uint32_t c = ls_batch_cluster(nb, cmax);
+    by[c == 1 ? 0 : c == 2 ? 1 : c == 4 ? 2 : c == 8 ? 3 : 4].push_back((uint32_t)b);
   }
-  const int rc = batch_device_enqueue(ctx, plan, dev_data, offsets, n_problems, exhaustive, prob, max_tries, seed, dev_params, dev_counts,
-                                      dev_masks, s);
-  if (side) {
-    CK(cudaEventRecord(ctx->bd_order[1], s));
-    CK(cudaStreamWaitEvent(ctx->stream, ctx->bd_order[1], 0));
-  }
-  return rc;
+  for (const auto& v : by) list.insert(list.end(), v.begin(), v.end());
+  const bool records = offsets[n_problems] > offsets[0];   // data, masks and weights are not read when every problem is empty
+  if (records) if (int rc = check_device_ptr(ctx, dev_data, alignof(double), "dev_data")) return rc;
+  if (int rc = check_device_ptr(ctx, dev_params, alignof(double), "dev_params")) return rc;
+  if (dev_masks && records) if (int rc = check_device_ptr(ctx, dev_masks, 1, "dev_masks")) return rc;
+  if (dev_weights && records) if (int rc = check_device_ptr(ctx, dev_weights, alignof(double), "dev_weights")) return rc;
+  return on_caller_stream(ctx, cuda_stream, [&](cudaStream_t s) {
+    if (int rc = stage_offsets(ctx, offsets, n_problems, list, s)) return rc;
+    LsBatchArgs a{};
+    a.model = ctx->model; a.data = dev_data; a.offsets = ctx->bt_off; a.masks = dev_masks; a.weights = dev_weights; a.out_params = dev_params;
+    size_t first = 0;
+    for (int k = 0; k < 5; k++) {
+      if (by[k].empty()) continue;
+      if (launch_ls_batch(a, ctx->bt_cl + first, (uint32_t)by[k].size(), 1u << k, ctx->ls_type, s) < 0)
+        return fail(ctx, LSQR_ERR_CUDA, std::string("batched least-squares launch: ") + cudaGetErrorString(cudaGetLastError()));
+      ctx->launches++;
+      first += by[k].size();
+    }
+    CKL();
+    return (int)LSQR_OK;
+  });
 }
 
 int lsqr_batch_capacity(lsqr_ctx* ctx, int precision, int exhaustive, uint64_t* one_block, uint64_t* max_records) {

@@ -192,6 +192,30 @@ inline uint32_t batch_cluster_size(const BatchLimits& L, uint64_t n) {
 int launch_batch_cluster(const BatchArgs& a, const uint32_t* problems, uint32_t count, uint32_t cluster, uint32_t slice, const EstCfg& cfg,
                          int ls_type, cudaStream_t s);
 
+// Batched least squares (lsqr_least_squares_batch_device): problem b's records are data[offsets[b] .. offsets[b + 1]) (records of
+// D doubles), selected by masks (one byte per record, non-zero = used) when given; weights (one double per record) select the
+// weighted Horn fit of the absolute orientation.
+struct LsBatchArgs {
+  int model;
+  const double* data;        // packed records on device, indexed by absolute record offset
+  const uint64_t* offsets;   // [n_problems + 1] on device
+  const uint8_t* masks;      // optional, indexed like the records
+  const double* weights;     // optional (ABSOR only), indexed like the records
+  double* out_params;        // [n_problems][P]
+};
+// A problem of n records takes a cluster of C CTAs (1, 2, 4, .., cmax): the smallest whose CTAs get at most kLsSliceRecords each.
+// It depends on n and the device alone, so a problem's result does not depend on the rest of the call.
+constexpr uint64_t kLsSliceRecords = 16384;
+inline uint32_t ls_batch_cluster(uint64_t n, int cmax) {
+  uint32_t c = 1;
+  while (c < (uint32_t)cmax && (n + c - 1) / c > kLsSliceRecords) c *= 2;
+  return c;
+}
+// the largest cluster of the model's kernel (weighted: the weighted Horn kernel) the current device schedules: 8 or 16; 0 = no kernel
+int ls_batch_max_cluster(int model, bool weighted);
+// the problems a.offsets[problems[i]], i < count, each on a cluster of `cluster` CTAs
+int launch_ls_batch(const LsBatchArgs& a, const uint32_t* problems, uint32_t count, uint32_t cluster, int ls_type, cudaStream_t s);
+
 // ---- k_score.cu (single-call helpers) ---------------------------------------------------
 void launch_estimate_one(int model, const double* packed_dev, const EstCfg& cfg, double* out_dev /* [0]=n_params, [1..P] */, cudaStream_t s);
 void launch_agree_many(int model, const double* params_dev, const double* packed_dev, uint32_t n, const EstCfg& cfg, uint8_t* out, cudaStream_t s);

@@ -1,4 +1,5 @@
 // Batched small problems (BASELINE.json configs[4]): one thread block per problem, see the comment above batch_kernel.
+#include "bulk_copy.cuh"
 #include "refine_common.cuh"
 #include "fast_forms.cuh"
 #include <cooperative_groups.h>
@@ -621,6 +622,234 @@ int launch_batch_cluster(const BatchArgs& a, const uint32_t* problems, uint32_t 
   BatchArgs args = a;
   EstCfg c = cfg;
   void* params[] = {&args, &problems, &c, &ls_type};
+  return cudaLaunchKernelExC(&lc, kern, params) == cudaSuccess ? 1 : -1;
+}
+
+// ---------------------------------------------------------------------------------------
+// Batched least squares (lsqr_least_squares_batch_device): leastSquaresEstimate of every problem of a batch over its selected
+// records, one cluster of C CTAs per problem (C from ls_batch_cluster).  CTA r takes records [r S, min((r + 1) S, n)),
+// S = ceil(n / C), and streams them from global memory -- nothing stays resident, so a problem has no size limit.  Record j of
+// the slice goes to thread j % kLsThreads, in increasing j, whatever the path that brings it in; moments are taken relative to
+// the problem's first record and reduced within the block, then over the cluster in rank order, so a problem's result depends
+// on its records and the device only.  Thread 0 of every CTA solves the same sums; for the geometric sphere fit every CTA runs
+// the same Levenberg-Marquardt controller, one streaming pass per evaluation.
+//
+// The slice is packed AoS doubles whose start need not be 16-byte aligned.  Tiles of TR records pass through the TileRing as
+// one bulk copy each, taken from the first 16-byte boundary of the slice (h = 1 double in when the slice starts off it): a tile
+// then lacks the first double of its first record, which that record's thread reads from global memory.  The records after the
+// last whole tile are read with plain loads.
+// ---------------------------------------------------------------------------------------
+constexpr int kLsThreads = 256;
+// records per tile: about 12 KB of 2- and 3-D records (two or three per thread), one record per thread above
+__host__ __device__ constexpr int ls_tile_records(int D) { return kLsThreads * (D <= 3 ? 6 / D : 1); }
+__host__ __device__ constexpr size_t ls_smem(int D) { return 2 * (size_t)ls_tile_records(D) * D * sizeof(double); }
+
+struct LsSlice {
+  const double* x;        // the CTA's records
+  uint32_t h, tiles, ns;  // 1 when x is not 16-byte aligned; whole tiles; records
+  const uint8_t* masks;   // the CTA's mask bytes, or null
+  const double* weights;  // the CTA's weights (weighted Horn)
+};
+
+// One streaming pass over the CTA's records -> the block's NM moments in `out` (thread tid < NM), read after a block or cluster
+// barrier.  LM: the sphere's Levenberg-Marquardt moments at lmx; W: weighted Horn with the number of pairs in [16].
+template <int M, bool W, bool LM, int NM, int TD>
+__device__ __forceinline__ void ls_pass(TileRing<1, TD, double>& ring, const LsSlice& sl, const double* sh_ctr, const double* lmx, double* sh_part,
+                                        double* out) {
+  constexpr int D = Model<M>::D, TR = TD / D;
+  const uint32_t tid = threadIdx.x;
+  double ctr[D];
+#pragma unroll
+  for (int d = 0; d < D; d++) ctr[d] = sh_ctr[d];
+  double acc[NM];
+#pragma unroll
+  for (int j = 0; j < NM; j++) acc[j] = 0.0;
+  auto take = [&](uint32_t j, const double* x) {
+    if (sl.masks && !sl.masks[j]) return;
+    double q[D];
+#pragma unroll
+    for (int d = 0; d < D; d++) q[d] = x[d] - ctr[d];
+    if constexpr (LM) acc_sphere_lm<Model<M>::DIM>(q, lmx, acc);
+    else if constexpr (W) { acc_absor_weighted(q, sl.weights[j], acc); acc[16] += 1.0; }
+    else { acc[0] += 1.0; accumulate<M>(q, acc); }
+  };
+  for (uint32_t t = 0; t < sl.tiles; t++) {
+    const double* tile = ring.wait(t);
+#pragma unroll
+    for (int u = 0; u < TR / kLsThreads; u++) {
+      const uint32_t r = u * kLsThreads + tid;
+      double x[D];
+#pragma unroll
+      for (int d = 0; d < D; d++) {
+        const int e = (int)(r * D + d) - (int)sl.h;
+        x[d] = e >= 0 ? tile[e] : sl.x[(size_t)t * TD];
+      }
+      take(t * TR + r, x);
+    }
+    ring.release();
+  }
+  for (uint32_t j = sl.tiles * TR + tid; j < sl.ns; j += kLsThreads) {
+    double x[D];
+#pragma unroll
+    for (int d = 0; d < D; d++) x[d] = sl.x[(size_t)j * D + d];
+    take(j, x);
+  }
+  const uint32_t lane = tid & 31, warp = tid >> 5;
+#pragma unroll
+  for (int j = 0; j < NM; j++) {
+    double v = acc[j];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (lane == 0) sh_part[warp * NM + j] = v;
+  }
+  __syncthreads();
+  if (tid < (uint32_t)NM) {
+    double v = 0.0;
+#pragma unroll
+    for (int w = 0; w < kLsThreads / 32; w++) v += sh_part[w * NM + tid];
+    out[tid] = v;
+  }
+}
+
+template <int M, bool W>
+__global__ void __launch_bounds__(kLsThreads) ls_batch_kernel(LsBatchArgs a, const uint32_t* __restrict__ problems, int ls_type) {
+  constexpr int D = Model<M>::D, P = Model<M>::P, K = Model<M>::K;
+  constexpr int TD = ls_tile_records(D) * D;
+  constexpr bool kSphere = Model<M>::FAM == FAM_SPHERE;
+  constexpr int NA = W ? 17 : Mom<M>::N;          // the analytic pass; weighted Horn counts the pairs in [16]
+  constexpr int NL = kSphere ? Mom<M>::NLM : 1;   // a Levenberg-Marquardt pass
+  constexpr int NMAX = NA > NL ? NA : NL;
+  const cg::cluster_group cluster = cg::this_cluster();
+  const uint32_t C = cluster.num_blocks(), rank = cluster.block_rank(), tid = threadIdx.x;
+  extern __shared__ __align__(16) unsigned char ls_smem_raw[];   // the tile ring: 2 x TD doubles
+  __shared__ __align__(8) uint64_t sh_bars[2];
+  __shared__ double sh_part[(kLsThreads / 32) * NMAX];
+  __shared__ double sh_mom[2][NMAX];   // this CTA's moments, by pass parity
+  __shared__ double sh_tot[NMAX];      // the cluster's
+  __shared__ double sh_out[LSQR_MAX_PARAMS + 4];
+  __shared__ double sh_state[LM_SIZE];
+  __shared__ double sh_ctr[kMaxDim];
+
+  const uint32_t b = problems[blockIdx.x / C];
+  const uint64_t off = a.offsets[b];
+  const uint32_t n = (uint32_t)(a.offsets[b + 1] - off);
+  const double* rec = a.data + off * D;
+  const uint32_t S = (uint32_t)(((uint64_t)n + C - 1) / C);
+  const uint32_t lo = min(rank * S, n), ns = min(S, n - lo);
+  LsSlice sl;
+  sl.x = rec + (size_t)lo * D;
+  sl.h = (uint32_t)((reinterpret_cast<uintptr_t>(sl.x) >> 3) & 1u);
+  sl.tiles = (uint64_t)ns * D >= sl.h ? (uint32_t)(((uint64_t)ns * D - sl.h) / TD) : 0u;
+  sl.ns = ns;
+  sl.masks = a.masks ? a.masks + off + lo : nullptr;
+  sl.weights = W ? a.weights + off + lo : nullptr;
+  if (tid < (uint32_t)kMaxDim) sh_ctr[tid] = (n > 0 && tid < (uint32_t)D && centred_component(M, (int)tid)) ? rec[tid] : 0.0;
+  TileRing<1, TD, double> ring{sl.x + sl.h, 0, 0, sl.tiles, reinterpret_cast<double*>(ls_smem_raw), sh_bars, (int)tid};
+  ring.start();   // (its barrier also publishes sh_ctr)
+
+  uint32_t pass = 0;
+  ls_pass<M, W, false, NA>(ring, sl, sh_ctr, nullptr, sh_part, sh_mom[pass & 1]);
+  cluster_sum(cluster, sh_mom[pass++ & 1], NA, sh_tot);
+  const bool lm = kSphere && ls_type == 1;   // geometric sphere fit: Levenberg-Marquardt from the algebraic fit
+  if (tid == 0) {
+    // the size guards of lsqr_least_squares / lsqr_weighted_least_squares on the selected records
+    double p[LSQR_MAX_PARAMS];
+    int np = 0;
+    if constexpr (W) {
+      if (sh_tot[16] >= 3.0) np = solve_absor(sh_tot, sh_ctr, p, true);
+    } else if (sh_tot[0] >= (double)K || (M == RAY && sh_tot[0] > 0.0)) {
+      np = solve_model(M, sh_tot, sh_ctr, lm ? 1 : 0, p);   // LM starts in centred coordinates
+    }
+    sh_out[0] = np;
+    for (int j = 0; j < np; j++) sh_out[1 + j] = p[j];
+  }
+  __syncthreads();
+  if constexpr (kSphere) {
+    if (lm) {   // batch_cluster_kernel's loop, with a streaming pass per evaluation
+      constexpr int NPL = Mom<M>::NPLM;
+      __shared__ double sh_bcast[1 + NPL];
+      if (tid == 0) {
+        for (int i = 0; i < LM_SIZE; i++) sh_state[i] = 0.0;
+        const int np = (int)sh_out[0];
+        if (np == 0) sh_state[LM_STATUS] = 2.0;
+        for (int j = 0; j < np; j++) sh_state[LM_X + j] = sh_out[1 + j];
+      }
+      for (;;) {
+        __syncthreads();
+        if (tid == 0) {
+          sh_bcast[0] = sh_state[LM_STATUS];
+          const int o = (sh_state[LM_PHASE] != 0.0) ? LM_TRIAL : LM_X;
+          for (int j = 0; j < NPL; j++) sh_bcast[1 + j] = sh_state[o + j];
+        }
+        __syncthreads();
+        double lmx[NPL];
+        const double status = sh_bcast[0];
+        for (int j = 0; j < NPL; j++) lmx[j] = sh_bcast[1 + j];
+        if (status != 0.0) break;
+        ring.restart();
+        ls_pass<M, W, true, NL>(ring, sl, sh_ctr, lmx, sh_part, sh_mom[pass & 1]);
+        cluster_sum(cluster, sh_mom[pass++ & 1], NL, sh_tot);
+        if (tid == 0) lm_update_model(M, sh_tot, sh_state);
+      }
+      if (tid == 0) {
+        if (sh_state[LM_STATUS] != 1.0) sh_out[0] = 0.0;
+        else {
+          for (int j = 0; j < Model<M>::DIM; j++) sh_out[1 + j] = sh_state[LM_X + j] + sh_ctr[j];
+          sh_out[1 + Model<M>::DIM] = sh_state[LM_X + Model<M>::DIM];
+        }
+      }
+      __syncthreads();
+    }
+  }
+  if (rank == 0) {
+    const int np = (int)sh_out[0];
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    for (uint32_t i = tid; i < (uint32_t)P; i += kLsThreads) a.out_params[(size_t)b * P + i] = np ? sh_out[1 + i] : nan;
+  }
+  cluster.sync();   // no CTA leaves while another may still read its moments
+}
+
+namespace {
+const void* ls_kernel(int model, bool weighted) {
+  if (weighted) return model == ABSOR ? reinterpret_cast<const void*>(ls_batch_kernel<ABSOR, true>) : nullptr;
+#define CALL(MM) return reinterpret_cast<const void*>(ls_batch_kernel<MM, false>);
+#define LSQR_DEF_(ID, DIM) case ID: CALL(ID)
+  switch (model) {
+    case PLANE3: CALL(PLANE3)
+    case LINE2D: CALL(LINE2D)
+    LSQR_PLANE_ND_LIST(LSQR_DEF_)
+    LSQR_LINE_ND_LIST(LSQR_DEF_)
+    LSQR_SPHERE_ALL_LIST(LSQR_DEF_)
+    LSQR_DENSE_N_LIST(LSQR_DEF_)
+    case ABSOR: CALL(ABSOR)
+    case RAY: CALL(RAY)
+    case PIVOT: CALL(PIVOT)
+    default: return nullptr;
+  }
+#undef LSQR_DEF_
+#undef CALL
+}
+}  // namespace
+
+int ls_batch_max_cluster(int model, bool weighted) {
+  const void* kern = ls_kernel(model, weighted);
+  return kern ? cluster_max(kern, ls_smem(model_info(model).D)) : 0;
+}
+
+int launch_ls_batch(const LsBatchArgs& a, const uint32_t* problems, uint32_t count, uint32_t cluster, int ls_type, cudaStream_t s) {
+  const void* kern = ls_kernel(a.model, a.weights != nullptr);
+  if (!kern) return -1;
+  if (count == 0) return 0;
+  const size_t smem = ls_smem(model_info(a.model).D);
+  allow_dynamic_smem(kern, smem);
+  cudaLaunchConfig_t lc{};
+  lc.gridDim = dim3(count * cluster); lc.blockDim = dim3(kLsThreads); lc.dynamicSmemBytes = smem; lc.stream = s;
+  cudaLaunchAttribute at{};
+  at.id = cudaLaunchAttributeClusterDimension;
+  at.val.clusterDim.x = cluster; at.val.clusterDim.y = 1; at.val.clusterDim.z = 1;
+  if (cluster > 1) { lc.attrs = &at; lc.numAttrs = 1; }   // one CTA per problem: a plain launch
+  LsBatchArgs args = a;
+  void* params[] = {&args, &problems, &ls_type};
   return cudaLaunchKernelExC(&lc, kern, params) == cudaSuccess ? 1 : -1;
 }
 

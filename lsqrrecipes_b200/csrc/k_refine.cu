@@ -246,14 +246,7 @@ __global__ void __launch_bounds__(256) weighted_absor_moments_kernel(DataView dv
     double q[6];
 #pragma unroll
     for (int d = 0; d < 6; d++) q[d] = dv.soa64[(size_t)d * dv.ld + i] - dv.center[d];
-    const double wi = w[i];
-    acc[0] += wi;
-#pragma unroll
-    for (int j = 0; j < 6; j++) acc[1 + j] += q[j] * wi;
-#pragma unroll
-    for (int r = 0; r < 3; r++)
-#pragma unroll
-      for (int c = 0; c < 3; c++) acc[7 + r * 3 + c] += (q[r] * q[3 + c]) * wi;
+    acc_absor_weighted(q, w[i], acc);
   }
   __shared__ double sh[8][kMaxMoments];
   const uint32_t lane = threadIdx.x & 31;

@@ -101,6 +101,17 @@ template <> __device__ __forceinline__ void accumulate<ABSOR>(const double* q, d
 #pragma unroll
     for (int c = 0; c < 3; c++) acc[7 + r * 3 + c] = fma(q[r], q[3 + c], acc[7 + r * 3 + c]);
 }
+// Weighted Horn (AbsoluteOrientationParametersEstimator.cxx:217-261): pair q (centred) with weight w into sum w, sum w p1,
+// sum w p2 and sum w p1 p2^T (acc[0..15])
+__device__ __forceinline__ void acc_absor_weighted(const double* q, double w, double* acc) {
+  acc[0] += w;
+#pragma unroll
+  for (int j = 0; j < 6; j++) acc[1 + j] += q[j] * w;
+#pragma unroll
+  for (int r = 0; r < 3; r++)
+#pragma unroll
+    for (int c = 0; c < 3; c++) acc[7 + r * 3 + c] += (q[r] * q[3 + c]) * w;
+}
 // RayIntersectionParametersEstimator.cxx:108-123
 template <> __device__ __forceinline__ void accumulate<RAY>(const double* q, double* acc) {
   const double* n = q + 3;
