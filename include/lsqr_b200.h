@@ -76,7 +76,9 @@ typedef enum lsqr_precision {
                   * rounding band of the threshold.  The kD-line estimators are scored through the perpendicular (d = 2) / the Pluecker
                   * moment (d = 3) of the direction, which is taken as the unit vector estimate() returns (it is re-normalised; imported
                   * parameter vectors with a non-unit direction are scored as their normalised line, where LSQR_FP64 evaluates the
-                  * reference's expression literally, LineParametersEstimator.hxx:135-150). */
+                  * reference's expression literally, LineParametersEstimator.hxx:135-150).  Domain: a record whose fp32 copy is not
+                  * finite (|x - c| >= FLT_MAX, c the centre of the data) is an outlier of every hypothesis, as the reference treats
+                  * a record with an infinite or NaN component. */
 } lsqr_precision;
 
 typedef enum lsqr_sampler {

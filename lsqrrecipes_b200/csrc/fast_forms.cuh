@@ -77,14 +77,17 @@ LSQR_DEF_(LINE4, 4) LSQR_DEF_(LINE5, 5) LSQR_DEF_(LINE6, 6) LSQR_DEF_(LINE7, 7) 
 #undef LSQR_DEF_
 // |d - r| < delta  <=>  (r - delta)^2 <= d^2 < (r + delta)^2  <=>  0 <= t' < 4 r delta  with  t' = d^2 - (r - delta)^2: the chain
 // starts at -(r - delta)^2 and the datum is an inlier iff bits(t') < bits(4 r delta) as unsigned integers (count_carry; the
-// threshold is per hypothesis).  r < delta: no lower bound, t' = d^2 + 1 against (r + delta)^2 + 1.  A threshold that is not
-// positive (negative delta: SphereParametersEstimator.hxx:20 keeps its sign) is stored as 0: nothing agrees.
+// threshold is per hypothesis).  r < delta: no lower bound, t' = d^2 (>= +0) against (r + delta)^2 -- relative, like every other
+// form, so the decisions do not depend on the data's scale.  An empty interval (delta not positive -- SphereParametersEstimator.hxx:20
+// keeps its sign --, r + delta <= 0, NaN) is stored as window 0: nothing agrees.
 template <int DIM> __device__ __forceinline__ void hoist_sphere(const double* p, const double* c, const EstCfg& cfg, float* q) {
   for (int i = 0; i < DIM; i++) q[i] = (float)(p[i] - c[i]);
   const double r = p[DIM], dl = cfg.delta;
-  double start, width;
-  if (r >= dl) { start = -(r - dl) * (r - dl); width = 4.0 * r * dl; }
-  else { start = 1.0; width = (r + dl) * (r + dl) + 1.0; }
+  double start = 0.0, width = 0.0;
+  if (dl > 0) {
+    if (r >= dl) { start = -(r - dl) * (r - dl); width = 4.0 * r * dl; }
+    else if (r + dl > 0) width = (r + dl) * (r + dl);
+  }
   q[DIM] = (float)start;
   const float wf = (float)width;
   // stored ready for count_carry: 2^32 - bits(window); 0 = nothing agrees (window not positive, or NaN)
@@ -102,8 +105,14 @@ template <> __device__ __forceinline__ void hoist32<ABSOR>(const double* p, cons
 template <> __device__ __forceinline__ void hoist32<RAY>(const double* p, const double* c, const EstCfg&, float* q) {
   for (int i = 0; i < 3; i++) q[i] = (float)(p[i] - c[i]);
 }
-template <> __device__ __forceinline__ void hoist32<PIVOT>(const double* p, const double* c, const EstCfg&, float* q) {
-  for (int i = 0; i < 3; i++) { q[i] = (float)p[i]; q[3 + i] = (float)(-(p[3 + i] - c[9 + i])); }   // the chain starts at -(tW - c)
+// PivotCalibrationParametersEstimator.cxx:108-123 compares the unsquared distance with delta: a negative one admits nothing, which
+// the squared form cannot see -- NaN constants then (every residual NaN: an outlier)
+template <> __device__ __forceinline__ void hoist32<PIVOT>(const double* p, const double* c, const EstCfg& cfg, float* q) {
+  const bool none = cfg.delta < 0.0;
+  for (int i = 0; i < 3; i++) {   // the chain starts at -(tW - c)
+    q[i] = none ? __int_as_float(0x7fffffff) : (float)p[i];
+    q[3 + i] = none ? __int_as_float(0x7fffffff) : (float)(-(p[3 + i] - c[9 + i]));
+  }
 }
 
 template <int N> __device__ __forceinline__ void hoist_dense(const double* p, const EstCfg& cfg, float* q) {
@@ -130,6 +139,10 @@ template <int M> constexpr int thr_slot() { return model_family(M) == FAM_SPHERE
 
 // ---- per-model residual forms on point pairs ----------------------------------------------
 struct Thr2 { f2 delta, neg_delta2; float fdelta; };
+// The threshold the fp32 kernels compare with |s| and count the shifted forms against (window 2 delta): a delta that is not
+// positive admits nothing.  (EstCfg.delta is |delta| where the reference squares it; the dense systems compare |a.x - b| with
+// delta itself, and a negative window would have admitted every s' >= 0.)
+__host__ __device__ __forceinline__ float fp32_delta(const EstCfg& cfg) { return cfg.delta > 0.0 ? (float)cfg.delta : 0.0f; }
 
 // signed(): g with inlier <=> g < 0.   For PLANE3 / LINE2D, dist(): s with inlier <=> |s| < delta.
 template <int M> struct Eval;
@@ -255,10 +268,11 @@ template <> struct Eval<RAY> {
     const f2 ntt = sub2(splat(0.f), tt);
     const f2 dx = fma2(ntt, x[3], vx), dy = fma2(ntt, x[4], vy), dz = fma2(ntt, x[5], vz);
     const f2 g = fma2(dx, dx, fma2(dy, dy, fma2(dz, dz, t.neg_delta2)));
-    // t >= 0 && dist^2 < delta^2  <=>  max(g, -t) < 0; with NaN padding the compare fails and the (positive) NaN -t is kept
-    float g0, g1, n0, n1;
-    halves(g, g0, g1); halves(ntt, n0, n1);
-    return join(g0 > n0 ? g0 : n0, g1 > n1 ? g1 : n1);
+    // t >= 0 && dist^2 < delta^2  <=>  g < 0 && -t < 0: the sign bit of g AND -t.  A NaN on either side (canonical, positive)
+    // is an outlier: an infinite record coordinate makes -t infinite and g NaN, and a select of the larger would keep -inf.
+    f2 r;
+    asm("and.b64 %0, %1, %2;" : "=l"(r.v) : "l"(g.v), "l"(ntt.v));
+    return r;
   }
 };
 template <> struct Eval<PIVOT> {

@@ -74,8 +74,9 @@ __device__ __forceinline__ uint32_t count32(const double* prm, const double* sh_
 #pragma unroll
     for (int j = 0; j < Q; j++) q[j] = splat(qf[j]);
     Thr2 thr;
-    thr.delta = splat((float)cfg.delta); thr.neg_delta2 = splat(-(float)cfg.delta2); thr.fdelta = (float)cfg.delta;
-    const uint32_t negk = hyp_negk<M>(qf, 0u - __float_as_uint(2.0f * (float)cfg.delta));   // 2^32 - bits(window)
+    const float fdelta = fp32_delta(cfg);
+    thr.delta = splat(fdelta); thr.neg_delta2 = splat(-(float)cfg.delta2); thr.fdelta = fdelta;
+    const uint32_t negk = hyp_negk<M>(qf, 0u - __float_as_uint(2.0f * fdelta));   // 2^32 - bits(window)
     unsigned long long out = 0ull;
     uint32_t pairs = 0;
     for (uint32_t i = first; i < n; i += step) {

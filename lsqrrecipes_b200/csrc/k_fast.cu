@@ -163,7 +163,7 @@ static int run_consensus32(const DataView& dv, const float* hyp, size_t hld, uin
   const size_t smem = 2 * (size_t)Model<M>::D * TILE * sizeof(float);
   auto kern = consensus32_kernel<M, R, THREADS, TILE, PPI>;
   allow_dynamic_smem(kern, smem);
-  kern<<<dim3(hyp_blocks, plan.chunks), THREADS, smem, s>>>(dv.soa32, dv.ld, tiles_total, plan.tiles_per_chunk, hyp, hld, H, (float)cfg.delta, (float)cfg.delta2,
+  kern<<<dim3(hyp_blocks, plan.chunks), THREADS, smem, s>>>(dv.soa32, dv.ld, tiles_total, plan.tiles_per_chunk, hyp, hld, H, fp32_delta(cfg), (float)cfg.delta2,
                                                              counts);
   return 1;
 }
@@ -480,7 +480,7 @@ static int run_consensus_cb(const DataView& dv, const float* hyp, size_t hld, ui
     hyp_blocks = (live + THREADS * R - 1) / (THREADS * R);
     if (cudaMemcpy2DAsync(bank, sizeof(float) * cp, dv.soa32 + base, sizeof(float) * dv.ld, sizeof(float) * npts, D, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return -1;
     const uint32_t sub = pick_sub(npts);
-    kern<<<dim3(hyp_blocks, (npts + sub - 1) / sub), THREADS, 0, s>>>(npts, sub, live_hyp, hld, live, (float)cfg.delta, (float)cfg.delta2, live_cnt);
+    kern<<<dim3(hyp_blocks, (npts + sub - 1) / sub), THREADS, 0, s>>>(npts, sub, live_hyp, hld, live, fp32_delta(cfg), (float)cfg.delta2, live_cnt);
     launches += 2;
     evals += (uint64_t)live * std::min(npts, rem);
   }

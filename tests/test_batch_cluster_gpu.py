@@ -2,13 +2,12 @@
 cluster each (batch_cluster_kernel).  The limits come from Engine.batch_capacity; fp64 results are pinned against an
 independent path (the same Philox hypotheses scored by lsqr_score, the round loop and stop rule replayed here, the consensus
 set from lsqr_consensus, the refit from the CPU oracle); a problem's outputs must not depend on the other problems of the call."""
-import math
-
 import numpy as np
 import pytest
 
 from conftest import SIGN_IDX, same_up_to_sign
 from lsqrrecipes_b200 import FP32, FP64, MODELS, SAMPLE_PHILOX, Engine, LsqrError, synth
+from oracle.fast32 import replay as _replay
 from oracle.pyoracle import INFO
 from oracle.pyoracle import MODELS as ORACLE_MODELS
 
@@ -41,32 +40,6 @@ def _sizes(one_block, max_records):
     b = max_records // 2 - 5
     b = b if b % 2 else b - 1
     return [a, b]
-
-
-def _replay(counts, valid, n, k, prob, max_tries):
-    """batch_kernel's round loop (rounds of 32, strict > on the key, the stop rule after a raise).  Returns (winner, count,
-    conclusive): conclusive is False when a stop-rule value t + 0.5 lies within a few ulps of an integer, where the device's
-    log / pow may round to the other side."""
-    tries = min(math.comb(n, k), 0xFFFFFFFF) if n >= k else 0
-    tries = min(tries, max_tries)
-    best, done, conclusive = 0, 0, True
-    log1mp = math.log(1.0 - prob)
-    while done < tries:
-        keys = [(int(counts[h]) << 32) | (0xFFFFFFFF - h) if valid[h] else 0 for h in range(done, min(done + 32, tries))]
-        rb = max(keys, default=0)
-        if rb > best:
-            best = rb
-            c = best >> 32
-            if c == n:
-                tries = 0
-            elif 0.0 < prob < 1.0 and c > 0:
-                t = log1mp / math.log(1.0 - (c / n) ** k) + 0.5
-                if abs(t - round(t)) <= 8 * math.ulp(t):
-                    conclusive = False
-                nt = 0xFFFFFFFF if t >= 4294967295.0 else int(t)
-                tries = min(nt, tries)
-        done += 32
-    return 0xFFFFFFFF - (best & 0xFFFFFFFF), best >> 32, conclusive
 
 
 @pytest.mark.parametrize("precision", [FP64, FP32])

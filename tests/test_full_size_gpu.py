@@ -15,7 +15,7 @@ import pytest
 from conftest import SIGN_IDX, same_up_to_sign
 from lsqrrecipes_b200 import FP32, FP64, SAMPLE_LIST, SAMPLE_PARAMS, Engine, synth
 from oracle.pyoracle import MODELS
-from test_parity_gpu import _fp32_band
+from oracle.fast32 import fp32_band as _fp32_band
 
 pytestmark = pytest.mark.gpu
 

@@ -13,6 +13,8 @@ import pytest
 
 from conftest import SIGN_IDX, golden, is_sphere, lm_case_is_clear, ls_types, model_family, pinv_tol, same_up_to_sign
 from lsqrrecipes_b200 import FP32, FP64, SAMPLE_EXHAUSTIVE, SAMPLE_LIST, SAMPLE_PARAMS, Engine, synth
+from oracle.fast32 import fp32_band as _fp32_band
+from oracle.fast32 import residual64 as _residual64
 from oracle.pyoracle import INFO, MODELS
 
 pytestmark = pytest.mark.gpu
@@ -366,72 +368,6 @@ def test_consensus_mask_and_refine_vs_oracle(port, name, m):
         direct = eng.least_squares(data[mask_ref.astype(bool)])
         assert same_up_to_sign(direct, want, SIGN_IDX[name], REFINE_TOL)
         eng.close()
-
-
-def _fp32_band(name, data, prm, delta):
-    """Half-width (in residual units) of the band around the threshold inside which an fp32 decision may legitimately differ
-    from the fp64 one: relative to the magnitude of the terms that are summed to form the residual (data in fp32 after
-    centring, fused multiply-adds in fp32).  The constants are MEASURED: tools/measure_fp32_band.py finds, for the 256
-    hypotheses with the largest fp32/fp64 count difference among 20 000 per estimator on 200 000 data, the distance to the
-    threshold of the farthest datum that was decided differently (profiles/r02_fp32_band.jsonl); the widest needs 0.29 of this
-    band, the 3-D plane 0.06 (2.8e-5 absolute for coordinates of +-1000, i.e. 1.6e-8 of the coordinate scale)."""
-    if name == "usxw":                 # the summed terms: pixel * scaled rotation column, t3, t2, t1
-        scale = np.abs(data[:, 12:]).max() * np.abs(prm[11:17]).max() * 2 + np.abs(prm[:6]).max() * 2 + np.abs(data[:, 9:12]).max() + 1.0
-        return 4e-7 * scale
-    if name == "uscp":
-        scale = np.abs(data[:, 12:14]).max() * np.abs(prm[8:14]).max() * 2 + np.abs(prm[:3]).max() + np.abs(data[:, 9:12]).max() + np.abs(data[:, 14:]).max() + 1.0
-        return 4e-7 * scale
-    fam, dim = model_family(name)
-    if fam == "dense":   # the summed terms are the products a_i x_i and b
-        nc = data.shape[1] - 1
-        scale = np.abs(data[:, :nc]).max() * np.abs(prm).max() * nc + np.abs(data[:, nc]).max() + 1.0
-        return 1e-7 * scale
-    scale = np.abs(data).max() + np.abs(prm).max() + 1.0
-    # (the constants were measured in up to four dimensions; a residual of d terms accumulates ~sqrt(d) as much rounding)
-    return 1e-7 * scale * (4.0 if (name in ("absor", "pivot", "ray") or fam == "line") else 2.0) * max(1.0, (dim / 4.0) ** 0.5)
-
-
-def _residual64(name, prm, data, delta):
-    """|residual| in float64 numpy, and the threshold it is compared with (distance units)."""
-    p = np.asarray(prm)
-    fam, _ = model_family(name)
-    if fam == "plane":
-        d = data.shape[1]
-        return np.abs((data - p[d:]) @ p[:d]), delta
-    if name == "line2d":
-        return np.abs((data - p[2:4]) @ p[0:2]), delta
-    if fam == "line":
-        d = data.shape[1]
-        v = data - p[d:]
-        w = v - (v @ p[:d])[:, None] * p[:d]
-        return np.linalg.norm(w, axis=1), delta
-    if is_sphere(name):
-        d = data.shape[1]
-        return np.abs(np.linalg.norm(data - p[:d], axis=1) - p[d]), delta
-    if name == "absor":
-        R = synth.quat_to_matrix(*p[:4])
-        return np.linalg.norm(data[:, :3] @ R.T + p[4:7] - data[:, 3:], axis=1), delta
-    if name == "ray":
-        v = p[:3] - data[:, :3]
-        t = np.sum(v * data[:, 3:], axis=1)
-        r = np.linalg.norm(v - t[:, None] * data[:, 3:], axis=1)
-        r[t < 0] = np.inf
-        return r, delta
-    if name == "pivot":
-        R = data[:, :9].reshape(-1, 3, 3)
-        return np.linalg.norm(np.einsum("nij,j->ni", R, p[:3]) + data[:, 9:] - p[3:6], axis=1), delta
-    if fam == "dense":
-        nc = data.shape[1] - 1
-        return np.abs(data[:, :nc] @ p[:nc] - data[:, nc]), delta
-    if name == "usxw":
-        R2 = data[:, :9].reshape(-1, 3, 3)
-        w = np.outer(data[:, 12], p[11:14]) + np.outer(data[:, 13], p[14:17]) + p[3:6]
-        return np.linalg.norm(np.einsum("nij,nj->ni", R2, w) + data[:, 9:12] - p[0:3], axis=1), delta
-    if name == "uscp":
-        R2 = data[:, :9].reshape(-1, 3, 3)
-        w = np.outer(data[:, 12], p[8:11]) + np.outer(data[:, 13], p[11:14]) + p[0:3]
-        return np.linalg.norm(np.einsum("nij,nj->ni", R2, w) + data[:, 9:12] - data[:, 14:17], axis=1), delta
-    raise AssertionError(name)
 
 
 @pytest.mark.parametrize("name,m", ALL)

@@ -4,7 +4,7 @@
     bit-exact, the arg-max the oracle's;
   * fp32 fast mode against the fp64 mode over 131 072 hypotheses x 10 M points (1.3 * 10^12 evaluations each): every count
     difference of every hypothesis is explained by data whose fp64 residual lies inside the fp32 rounding band of the
-    threshold (the band of tests/test_parity_gpu.py::_fp32_band, whose constants are twice what tools/measure_fp32_band.py
+    threshold (the band of oracle/fast32.py::fp32_band, whose constants are twice what tools/measure_fp32_band.py
     measured); the band is counted on the GPU by scoring the same hypotheses in fp64 at delta + band and delta - band.
 """
 import numpy as np
@@ -12,7 +12,7 @@ import pytest
 
 from lsqrrecipes_b200 import FP32, FP64, SAMPLE_LIST, SAMPLE_PARAMS, Engine, synth
 from oracle.pyoracle import MODELS
-from test_parity_gpu import _fp32_band
+from oracle.fast32 import fp32_band as _fp32_band
 
 pytestmark = pytest.mark.gpu
 

@@ -5,7 +5,7 @@ differently by the fp32 fast mode?
 For every estimator H Philox hypotheses are scored in fp32 and in fp64 (same parameter vectors).  For the hypotheses with the
 largest count differences the residuals are recomputed in float64 numpy; a difference of k decisions needs the k data closest to
 the threshold, so the k-th smallest | |residual| - delta | is the band that hypothesis needs.  Reported per model: the largest
-needed band, absolute and as a fraction of the band the test allows (_fp32_band); the test's constants are set so that this
+needed band, absolute and as a fraction of the band the test allows (oracle/fast32.py fp32_band); the test's constants are set so that this
 fraction stays below one half.   python tools/measure_fp32_band.py [n] [H] [model ...]"""
 import json
 import os
@@ -15,9 +15,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
 from lsqrrecipes_b200 import FP32, FP64, MODELS, SAMPLE_PARAMS, Engine, synth  # noqa: E402
-from test_parity_gpu import _fp32_band, _residual64  # noqa: E402
+from oracle.fast32 import fp32_band as _fp32_band  # noqa: E402
+from oracle.fast32 import residual64 as _residual64  # noqa: E402
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 200_000
 H = int(sys.argv[2]) if len(sys.argv) > 2 else 20_000
